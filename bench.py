@@ -4,8 +4,12 @@
 (the sfu_amazon_100k reproduction shape) on N B200s, plus roofline / CPU-baseline / end-to-end legs.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload cfg1|cfg2|cfg3|cfg4|cfg5]
+                    [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU, NCCL); rank 0 prints ONE JSON line.
+--dump-outputs DIR: rank 0 also writes what the last timed step computed as DIR/<name>.npy (see dump_outputs), so that
+two builds run with the same arguments (hence the same seeded inputs) can be compared output for output.  Two runs of one
+build are not bit-identical: on one B200 (1000 W) cfg2 dumps agreed within 2e-5 of each array's largest magnitude.
 Synthetic data of the reference's shape (SURVEY.md 8d), reference initialisation under seed 10.
 Workloads: cfg2 = headline; cfg1 (config_example shape), cfg3 (per-GPU shard of the 8 x 64 data-parallel run),
 cfg4 (scaled decoder: H 1024, V 50k, T 64), cfg5 (inference: encode + resample decoding, batch 1024) are recorded under
@@ -19,6 +23,7 @@ import os
 import sys
 import threading
 import time
+import zlib
 
 import numpy as np
 import torch
@@ -445,7 +450,7 @@ def run_inference_workload(args):
     inf = importlib.import_module("disentanglement-vae_b200.inference")
     dev = torch.device("cuda", 0)
     torch.cuda.set_device(0)
-    B, T, R = BATCH, SEQ_T, 30
+    B, T = BATCH, SEQ_T
     dvae.set_seed(10)
     vae = dvae.build_vae(CFG2, VOCAB, None, LABELS, dev, SOS, EOS)
     vae.train()
@@ -455,7 +460,7 @@ def run_inference_workload(args):
     clocks = ClockSampler(0)
     ev_ = inf.ConsistencyEvaluator(vae, B, T, keep_tokens=True)
     warm = max(args.warmup, 3)
-    steps = args.steps if args.steps != 50 else R
+    steps = args.steps
     n0 = dvae.launch_count()
     ev_.use_graph = False
     ev_.encode_once(Xh, Lh)
@@ -478,6 +483,8 @@ def run_inference_workload(args):
     torch.cuda.synchronize()
     ms = a.elapsed_time(b)
     clk = clocks.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: v[-1] for k, v in out.items()})          # the last resample
     toks = float(L.sum()) * 2 * steps
     # e2e: host tokens in -> encode once -> R resamples -> predictions of both passes back on the host (wall clock)
     t0 = time.perf_counter()
@@ -527,6 +534,48 @@ def run_inference_workload(args):
 
 
 # ------------------------------------------------------------------------------------------------
+DUMP_BYTES = 60 * 10 ** 6       # array data of one --dump-outputs directory: with the .npy headers it stays under 64 MB
+
+
+def _dump_cap(sizes, budget):
+    """The largest per-array size c with sum(min(s, c)) <= budget, or None when every array fits whole."""
+    if sum(sizes) <= budget:
+        return None
+    left, rest = budget, sorted(sizes)
+    for i, s in enumerate(rest):
+        c = left // (len(rest) - i)
+        if s > c:
+            return c
+        left -= s
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes {name: tensor or array} as out_dir/<name>.npy: floating point as float32, integers as float64 (exact).
+    Over DUMP_BYTES in all, the largest arrays are cut to an equal share each, a sorted sample of their flattened elements
+    drawn by a generator seeded with the array's name, so the same run always writes the same elements."""
+    os.makedirs(out_dir, exist_ok=True)
+    host = {}
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy() if torch.is_tensor(t) else np.asarray(t)
+        host[name] = a.astype(np.float32 if a.dtype.kind == "f" else np.float64)
+    cap = _dump_cap([a.nbytes for a in host.values()], DUMP_BYTES)
+    for name, a in host.items():
+        if cap is not None and a.nbytes > cap:
+            idx = np.random.default_rng(zlib.crc32(name.encode())).choice(a.size, cap // a.itemsize, replace=False)
+            a = a.reshape(-1)[np.sort(idx)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def train_step_outputs(vae, eng, out):
+    """What a caller of TrainEngine.step_resident holds after a step: the returned loss block, the updated parameters and
+    Adam's first moments (an average of the gradients, which the parameter update alone shows only scaled by lr)."""
+    m = vae.grad_views(eng.m)
+    arrays = {"losses": out}
+    arrays.update({f"param.{n}": p for n, p in vae.named_parameters()})
+    arrays.update({f"adam_exp_avg.{n}": m[n] for n in vae._layout})
+    return arrays
+
+
 def _events(n):
     return [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(n)]
 
@@ -610,7 +659,7 @@ def gemm_class_trace(eng, batch, steps=3):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 50; cfg5: 30 resamples)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-graph", action="store_true")
@@ -621,7 +670,13 @@ def main():
     ap.add_argument("--tf", type=float, default=None, help="teacher_forcing_prob (default 1.0 = headline; 0.5 = the shipped configs' value)")
     ap.add_argument("--workload", default="cfg2", choices=["cfg1", "cfg2", "cfg3", "cfg4", "cfg5"],
                     help="cfg2 = headline (BASELINE.json configs[1]); the others are secondary configs, recorded under profiles/")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32 / float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 30 if args.workload == "cfg5" else 50
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     uniform_lengths = select_workload(args.workload)
     global BATCH, CFG2
     if args.batch is not None:
@@ -711,6 +766,8 @@ def main():
     step_ms = {"min": srt[0], "median": srt[len(srt) // 2], "p90": srt[min(len(srt) - 1, int(0.9 * len(srt)))], "max": srt[-1],
                "note": "per-step CUDA-event times of this rank's timed region (ms_per_step is their mean, max over ranks)"}
     loss_last = eng.losses_from(out.cpu())["total_loss"]
+    if args.dump_outputs and rank == 0:          # before the legs below train the same engine further
+        dump_outputs(args.dump_outputs, train_step_outputs(vae, eng, out))
 
     if args.only_steps:
         if world > 1:

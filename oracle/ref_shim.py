@@ -17,9 +17,9 @@ The reference imports two packages at module top that are not installed here
 * `torchtext.data.metrics.bleu_score` -- logging only (`/root/reference/vae/losses.py:133`);
   stubbed to 0.0.
 
-`/root/reference` exists only in the build container, never on the GPU box.  The only callers
-of `load_reference()` are `tests/golden/make_golden.py` (fixture generator) and CPU tests that
-skip when the directory is absent.
+The reference is not part of this repository (point DVAE_REFERENCE_ROOT at a checkout of it).  The
+only caller of `load_reference()` is `tests/golden/make_golden.py`, which stores what the reference
+computes under `tests/golden/`; the tests compare against those files and never import the reference.
 """
 import os
 import sys

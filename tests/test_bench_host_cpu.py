@@ -6,7 +6,9 @@ import os
 import sys
 import time
 
+import numpy as np
 import pytest
+import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -59,6 +61,26 @@ def test_every_baseline_config_is_a_selectable_workload(bench, name):
     assert cfg["workload"].startswith(name) and cfg["global_batch"] == bench.BATCH and cfg["seq_len"] == bench.SEQ_T
     assert bench.workload_config(8)["global_batch"] == 8 * bench.BATCH and bench.workload_config(8)["parallelism"] == "dp8"
     assert "model" not in cfg            # the tier's contract: config names the workload, no model keys
+
+
+def test_dump_outputs_stays_under_64_mb_and_samples_the_same_elements_every_time(bench, tmp_path):
+    rng = np.random.default_rng(0)
+    arrays = {"losses": torch.arange(32, dtype=torch.float32), "lengths": torch.arange(7, dtype=torch.int64) * 3,
+              "param.w": torch.from_numpy(rng.standard_normal((6000, 5000)).astype(np.float32)),       # 120 MB alone
+              "param.b": np.linspace(-1, 1, 999)}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["lengths.npy", "losses.npy", "param.b.npy", "param.w.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 64 * 10 ** 6
+    got = {f[:-4]: np.load(tmp_path / "a" / f) for f in files}
+    assert got["losses"].dtype == np.float32 and np.array_equal(got["losses"], np.arange(32))      # small arrays whole
+    assert got["lengths"].dtype == np.float64 and np.array_equal(got["lengths"], np.arange(7) * 3)
+    assert got["param.b"].dtype == np.float32 and got["param.b"].shape == (999,)
+    w = got["param.w"]
+    assert w.dtype == np.float32 and w.ndim == 1 and 10 ** 7 < w.size < arrays["param.w"].numel()
+    assert np.isin(w, arrays["param.w"].numpy()).all()                                             # elements, not noise
+    assert np.array_equal(w, np.load(tmp_path / "b" / "param.w.npy"))                              # the same sample
 
 
 def test_algorithmic_flops_match_the_survey_accounting(bench):

@@ -9,7 +9,6 @@ import pytest
 import torch
 
 from conftest import ROOT, load_golden, golden_state_dict
-from oracle import ref_shim
 
 HEADER = os.path.join(ROOT, "include", "dvae_b200.h")
 
@@ -121,44 +120,56 @@ def test_cpu_model_refuses_to_run(dvae):
     assert bow.context2params["content"].in_features == bow.encoder.emb_dim
 
 
-@pytest.mark.skipif(not ref_shim.reference_available(), reason="reference checkout not present (GPU box)")
+# Model settings of the golden cases (tests/golden/make_golden.py): each file's `sd.*` arrays are the reference's
+# state_dict right after its set_seed(10) and build_vae(), before any step.
+_GOLDEN_INIT = {
+    "tiny_uni": ({}, {"polarity": 1}),
+    "tiny_bi": ({"bidirectional_encoder": True, "embedding_dim": 10, "hidden_dim": 8,
+                 "latent_dims": {"total": 7, "polarity": 1, "uncertainty": 2}}, {"uncertainty": 1, "polarity": 1}),
+    "tiny_eval_mc": ({"num_rnn_layers": 1, "embedding_dim": 6, "hidden_dim": 8, "latent_dims": {"total": 5, "modality": 2}},
+                     {"modality": 3}),
+    "tiny_bow": ({"bow_encoder": True, "embedding_dim": 10, "hidden_dim": 8, "latent_dims": {"total": 5, "polarity": 1}},
+                 {"polarity": 1}),
+    "tiny_adv_mi": ({"bidirectional_encoder": True, "embedding_dim": 10, "hidden_dim": 8, "adversarial_loss": True,
+                     "mi_loss": True, "latent_dims": {"total": 9, "polarity": 1, "uncertainty": 2}},
+                    {"uncertainty": 3, "polarity": 1}),
+}
+
+
+def _seeded_model_of_golden_case(dvae, case):
+    over, label_dims = _GOLDEN_INIT[case]
+    g = load_golden(case)
+    p = _params(**{"embedding_dim": 12, "hidden_dim": 16, "bidirectional_encoder": False, "encoder_dropout": 0.0,
+                   "decoder_dropout": 0.0, "latent_dims": {"total": 6, "polarity": 1}, **over})
+    dvae.set_seed(10)
+    return g, dvae.build_vae(p, int(g["V"]), None, label_dims, torch.device("cpu"), int(g["sos"]), int(g["eos"]))
+
+
 def test_adversarial_and_mi_modules_match_reference_structure_and_seeded_init(dvae):
     """adversarial_loss / mi_loss: same adversary and estimator names, same state_dict keys, and -- because the
     construction order is the reference's -- bit-identical seeded initial weights (incl. the CLUB estimators, which the
-    reference keeps in a plain dict outside the state_dict)."""
-    ref_model, _, ref_utils = ref_shim.load_reference()
-    p = _params(adversarial_loss=True, mi_loss=True, latent_dims={"total": 9, "polarity": 1, "uncertainty": 2})
-    label_dims = {"uncertainty": 3, "polarity": 1}
-    ref_utils.set_seed(10)
-    ref = ref_model.build_vae(p, 41, None, label_dims, torch.device("cpu"), 2, 3)
-    dvae.set_seed(10)
-    mine = dvae.build_vae(p, 41, None, label_dims, torch.device("cpu"), 2, 3)
-    assert list(ref.adversaries.keys()) == list(mine.adversaries.keys())
-    assert list(ref.mi_estimators.keys()) == list(mine.mi_estimators.keys())
-    rs, ms = ref.state_dict(), mine.state_dict()
+    reference keeps in a plain dict outside the state_dict; stored as `mi0.*` in the golden file)."""
+    g, mine = _seeded_model_of_golden_case(dvae, "tiny_adv_mi")
+    assert list(mine.adversaries.keys()) == [str(n) for n in g["adv_names"]]
+    assert list(mine.mi_estimators.keys()) == [str(n) for n in g["mi_names"]]
+    rs, ms = golden_state_dict(g), mine.state_dict()
     assert list(rs.keys()) == list(ms.keys())
     for k in rs:
-        assert torch.equal(rs[k], ms[k]), k
-    for n in ref.mi_estimators:
-        a, b = ref.mi_estimators[n].state_dict(), mine.mi_estimators[n].state_dict()
+        assert np.array_equal(rs[k], ms[k].numpy()), k
+    for n, est in mine.mi_estimators.items():
+        a, b = golden_state_dict(g, f"mi0.{n}."), est.state_dict()
         assert list(a.keys()) == list(b.keys())
         for k in a:
-            assert torch.equal(a[k], b[k]), (n, k)
+            assert np.array_equal(a[k], b[k].numpy()), (n, k)
     assert [n for n, _ in mine.named_parameters() if n.startswith("adversaries")]
     assert not [q for q in mine.trainable_parameters() if any(q is w for w in mine.adversaries.parameters())]
     assert not any(n.startswith("adversaries") for n in mine._layout)      # adversaries own their optimizers
 
 
-@pytest.mark.skipif(not ref_shim.reference_available(), reason="reference checkout not present (GPU box)")
 def test_same_seed_gives_reference_initialisation(dvae):
-    ref_model, _, ref_utils = ref_shim.load_reference()
-    p = _params()
-    label_dims = {"uncertainty": 1, "polarity": 1}
-    ref_utils.set_seed(10)
-    ref = ref_model.build_vae(p, 41, None, label_dims, torch.device("cpu"), 2, 3)
-    dvae.set_seed(10)
-    mine = dvae.build_vae(p, 41, None, label_dims, torch.device("cpu"), 2, 3)
-    rs, ms = ref.state_dict(), mine.state_dict()
-    assert list(rs.keys()) == list(ms.keys())
-    for k in rs:
-        assert torch.equal(rs[k], ms[k]), k
+    for case in ("tiny_uni", "tiny_bi", "tiny_eval_mc", "tiny_bow"):
+        g, mine = _seeded_model_of_golden_case(dvae, case)
+        rs, ms = golden_state_dict(g), mine.state_dict()
+        assert list(rs.keys()) == list(ms.keys()), case
+        for k in rs:
+            assert np.array_equal(rs[k], ms[k].numpy()), (case, k)
