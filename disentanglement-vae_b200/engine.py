@@ -16,6 +16,8 @@ Variants of the step (all with the reference's semantics):
     plan as above; the small objectives on the latent spaces (adversaries, CLUB estimators) run eagerly through their
     autograd Functions (`functions.py`, C-ABI kernels) and hand d(loss)/dz to the fused heads' backward.  Single GPU,
     no graph.
+  * evaluation (eval_step / eval_steps, run.py:347-423): the same forward with train=False, the losses and corpus BLEU of
+    the predictions, one graph per decode regime; no backward, no optimizer, training state untouched.
 """
 import os
 import random
@@ -126,6 +128,10 @@ class TrainEngine:
             base += 7919 * self.rank          # every data-parallel shard draws its own eps / dropout / coin streams
         self._gen = torch.Generator().manual_seed(base)
         self._pyrand = random.Random(base)
+        # evaluation draws its eps / coins from streams of its own, so that eval_step never shifts the training streams
+        self._eval_gen = torch.Generator().manual_seed(base + 0x5EED)
+        self._eval_pyrand = random.Random(base + 0x5EED)
+        self._eval = None      # evaluation buffers and graphs, allocated on the first eval_step
         self.use_graph = use_graph and not self.aux
         self._graphs = None
         self._buckets = None
@@ -167,8 +173,12 @@ class TrainEngine:
         _lib.planes_owner = self._plane_token
 
     # ---- the kernel sequences ------------------------------------------------------------------
-    def _forward(self, fork_ok=True):
+    def _forward(self, fork_ok=True, train=True, sampled=None, preds=None):
+        """Forward pass of one step up to the reconstruction loss.  The defaults are the training step; eval_step passes
+        train=False (no dropout) and its own decode regime / prediction buffer."""
         pl, P, m = self.plan, self.model._P, self.model
+        sampled = self.sampled if sampled is None else sampled
+        preds = self.preds if preds is None else preds
         n_pl = len(self._wplanes)
         n_ih = sum(1 for w, a, b in self._wplanes if a is not None)      # LSTM input weights come first, W_out^T last
         if n_pl:               # operand planes of the weights the encoder reads first: one launch, first thing in the step
@@ -183,7 +193,9 @@ class TrainEngine:
         # the decoder's input embeddings, its layer-0 input projection and the W_out operand planes do not depend on
         # the encoder (teacher forcing): they run on a side stream under the encoder's recurrences (64 of 148 SMs)
         cur = torch.cuda.current_stream()
-        hoist = fork_ok and os.environ.get("DVAE_HOIST", "1") != "0" and not d_bow(pl) and not self.sampled
+        hoist = fork_ok and os.environ.get("DVAE_HOIST", "1") != "0" and not d_bow(pl) and not sampled
+        # W_out^T planes (10 MB at cfg 2) are read by the vocabulary backward only: not refreshed for an evaluation
+        refresh_wt = n_pl > n_ih and train
         fork_prep = None
         if hoist:
             if self._side is None:
@@ -192,23 +204,23 @@ class TrainEngine:
             def fork_prep():      # forked behind the encoder's layer-0 projection GEMMs, which fill the machine themselves
                 self._side.wait_stream(cur)
                 with torch.cuda.stream(self._side):
-                    pl.decode_prepare(P, self.inputs, m.sos_token_idx, True)
-                    if n_pl > n_ih:      # W_out^T planes (10 MB at cfg 2) are read by the vocabulary backward only
+                    pl.decode_prepare(P, self.inputs, m.sos_token_idx, train)
+                    if refresh_wt:
                         check(self.lib.dvae_weight_planes_refresh_ex(n_ih, n_pl - n_ih, _lib.stream_ptr()), "dvae_weight_planes_refresh")
-        if n_pl > n_ih and not hoist:
+        if refresh_wt and not hoist:
             check(self.lib.dvae_weight_planes_refresh_ex(n_ih, n_pl - n_ih, _lib.stream_ptr()), "dvae_weight_planes_refresh")
-        pl.encode(P, self.inputs, self.lengths, True, after_l0_proj=fork_prep)
+        pl.encode(P, self.inputs, self.lengths, train, after_l0_proj=fork_prep)
         pl.heads(P, pl.ctx, pl.eps, self.labels, self.kl_w)
         if hoist:
             cur.wait_stream(self._side)
-        if self.sampled:
+        if sampled:
             # vae/model.py:457-472: position i's input is inputs[:, i] when its coin is heads, else the token sampled from
             # position i's logits; preds doubles as decoder-input buffer and as `token_predictions`
-            self.preds.copy_(self.inputs)
-            self.preds[:, 0].fill_(m.sos_token_idx)
-            h_top = pl.decode_sampled(P, self.preds, self.coins, True)
+            preds.copy_(self.inputs)
+            preds[:, 0].fill_(m.sos_token_idx)
+            h_top = pl.decode_sampled(P, preds, self.coins, train)
         else:
-            h_top = pl.decode_forced(P, self.inputs, m.sos_token_idx, True)
+            h_top = pl.decode_forced(P, self.inputs, m.sos_token_idx, train)
         pl.vocab_ce(P, h_top, self.inputs, self.lengths)
         return h_top, hoist
 
@@ -488,13 +500,13 @@ class TrainEngine:
                     check(self.lib.dvae_weight_planes_enable(0), "dvae_weight_planes_enable")
         return cm()
 
-    def _run(self):
+    def _run(self, body=None):
         # the registry is consulted while kernels are ENQUEUED (eager steps, graph capture): on around this engine's launches only
         self._register_weight_planes()
         if self._wplanes:
             check(self.lib.dvae_weight_planes_enable(1), "dvae_weight_planes_enable")
         try:
-            return self._run_inner()
+            return (body or self._run_inner)()
         finally:
             if self._wplanes:
                 check(self.lib.dvae_weight_planes_enable(0), "dvae_weight_planes_enable")
@@ -614,21 +626,24 @@ class TrainEngine:
             ev.synchronize()
         return self._slot
 
-    def _fill_scalars(self, hv):
+    def _fill_scalars(self, hv, eval_tf=None):
         """Adam hyper-parameters and step count, KL weights (cyclic value of this global step), dropout / noise seed and the
-        teacher-forcing coins of this step, written into a pinned host block."""
+        teacher-forcing coins of this step, written into a pinned host block.  eval_tf (an evaluation's teacher-forcing
+        probability): "cyclic" KL weights are 1.0 (run.py:374-375), seed and coins come from the evaluation streams."""
+        train = eval_tf is None
         sc = hv["scal"]
         sc[0], sc[1], sc[2], sc[3], sc[4] = self.lr, 0.9, 0.999, 1e-8, float(self.adam_step + 1)
         for i, n in enumerate(self.d.space_names):
             w = self.lambdas[n] if n in self.lambdas else self.lambdas["default"]
             if w == "cyclic":
-                w = get_cyclic_kl_weight(self.step_idx, self.total_steps)
+                w = get_cyclic_kl_weight(self.step_idx, self.total_steps) if train else 1.0
             sc[8 + i] = float(w)
-        hv["seed"][0] = int(torch.randint(0, 2 ** 62, (1,), generator=self._gen))
-        if self.sampled:      # one coin per decoding step, shared by the batch (vae/model.py:463)
+        hv["seed"][0] = int(torch.randint(0, 2 ** 62, (1,), generator=self._gen if train else self._eval_gen))
+        tf, rnd = (self.tf_prob, self._pyrand) if train else (eval_tf, self._eval_pyrand)
+        if tf < 1.0:          # one coin per decoding step, shared by the batch (vae/model.py:463)
             c = hv["coins"]
             for i in range(c.shape[0]):
-                c[i] = 1 if self._pyrand.random() < self.tf_prob else 0
+                c[i] = 1 if rnd.random() < tf else 0
 
     def _upload(self, slot, names=None):
         """H2D of a pinned block: the whole block (one copy), or only the named fields (device-resident batches)."""
@@ -661,9 +676,10 @@ class TrainEngine:
         self.adam_step += 1
         return self.plan.out
 
-    def _enqueue_host_step(self, inputs, lengths, labels):
+    def _enqueue_host_step(self, inputs, lengths, labels, eval_tf=None):
         """Stage one HOST batch into the next pinned block, enqueue its single H2D copy, the step and the D2H copy of the
-        result block; returns the slot (its event completes when the losses are in h_outs[slot])."""
+        result block; returns the slot (its event completes when the losses are in h_outs[slot]).  eval_tf: an
+        evaluation step at that teacher-forcing probability instead (result block in the evaluation ring)."""
         slot = self._acquire_slot()
         hv = self._hv[slot]
         hv["inputs"][...] = inputs.numpy() if torch.is_tensor(inputs) else inputs
@@ -671,8 +687,15 @@ class TrainEngine:
         for i, n in enumerate(self.label_names):
             y = labels[n]
             hv["labels"][i] = (y.numpy() if torch.is_tensor(y) else y).reshape(-1)
-        self._fill_scalars(hv)
+        self._fill_scalars(hv, eval_tf)
         self._upload(slot)
+        if eval_tf is not None:
+            ev = self._eval
+            self._run(lambda: self._eval_run(eval_tf < 1.0))
+            ev["h_out"][slot].copy_(ev["out"], non_blocking=True)
+            ev["aux"][slot] = self._eval_aux() if self.aux else None
+            self._release_slot(slot)
+            return slot
         self._run()
         self.h_outs[slot].copy_(self.plan.out, non_blocking=True)
         self._release_slot(slot)
@@ -705,21 +728,147 @@ class TrainEngine:
             self._slot_ev[slot].synchronize()
             yield self.losses_from(self.h_outs[slot])
 
-    def losses_from(self, out):
+    def losses_from(self, out, aux=None):
+        """The loss dict of `compute_all_losses` from a result block; `aux`: the adversarial / MI values to add (default:
+        those of the last training step)."""
         S, NS = self.d.S, _lib.HEADS_NSCALARS
+        aux = self.last_aux if aux is None else aux
         o = out.tolist()
         L = {"reconstruction_loss": o[NS], "total_weighted_kl": o[0], "total_kl": o[1], "total_dsc_loss": o[2],
              "idv_kls": {n: o[3 + i] for i, n in enumerate(self.d.space_names)},
              "idv_dsc_losses": {n: o[3 + S + i] for i, n in enumerate(self.d.space_names) if self.d.dsc_out[i] > 0},
              "idv_dsc_accs": {n: o[3 + 2 * S + i] for i, n in enumerate(self.d.space_names) if self.d.dsc_out[i] > 0}}
         L["total_loss"] = o[NS] + o[0] + o[2]
-        if self.aux and self.last_aux:
-            L["total_adv_loss"] = float(self.last_aux["total_adv_loss"].detach())
-            L["total_mi"] = float(self.last_aux["total_mi"].detach())
+        if self.aux and aux:
+            L["total_adv_loss"] = float(aux["total_adv_loss"].detach())
+            L["total_mi"] = float(aux["total_mi"].detach())
             for k in ("idv_adv_losses", "idv_adv_dsc_accs", "idv_mi_estimates"):
-                L[k] = self.last_aux[k]
+                L[k] = aux[k]
             L["total_loss"] += L["total_adv_loss"] + L["total_mi"]
         return L
+
+    # ---- evaluation: the body of run.py:evalstep (run.py:347-423) --------------------------------------------------
+    # Result block (float32): [0, NS + 5) the training block's layout (heads scalars, [NS] reconstruction loss),
+    # [NS + 1] corpus BLEU, then the 10 int64 BLEU counts of dvae_bleu_counts (clipped 1-4, total 1-4, cand / ref length).
+    def _eval_setup(self):
+        if self._eval is not None:
+            return self._eval
+        NB = self.plan.out.numel()
+        out = torch.zeros(NB + 20, device=self.device, dtype=torch.float32)
+        self._eval = ev = {"out": out, "counts": out[NB:].view(torch.int64), "nb": NB, "graphs": {},
+                           "preds": torch.zeros(self.B, self.T, device=self.device, dtype=torch.int64),
+                           "h_out": torch.zeros(self.NSLOT, out.numel(), dtype=torch.float32).pin_memory(),
+                           "aux": [None] * self.NSLOT}
+        return ev
+
+    def _eval_body(self, sampled):
+        """Eval-mode forward (no dropout, one eps draw), every loss of compute_all_losses and corpus BLEU of the
+        predictions against the inputs, into the evaluation result block.  No backward pass, no optimizer."""
+        from .losses import bleu_counts_, bleu_score_
+        ev, pl, m = self._eval, self.plan, self.model
+        preds = ev["preds"]
+        self._forward(train=False, sampled=sampled, preds=preds)
+        if not sampled:      # teacher forcing: the predictions are the decoder inputs (vae/model.py:455)
+            preds.copy_(self.inputs)
+            preds[:, 0].fill_(m.sos_token_idx)
+        NS, NB = _lib.HEADS_NSCALARS, ev["nb"]
+        ev["out"][:NB].copy_(pl.out)
+        ev["counts"].zero_()
+        bleu_counts_(ev["counts"], self.inputs, preds, m.eos_token_idx)
+        bleu_score_(ev["out"][NS + 1:NS + 2], ev["counts"])
+
+    def _eval_run(self, sampled):
+        ev = self._eval
+        if not self.use_graph:
+            self._eval_body(sampled)
+        else:
+            g = ev["graphs"].get(sampled)
+            if g is None:      # warm up eagerly (lazy module loading, workspaces), then capture; nothing to undo
+                s = torch.cuda.Stream(device=self.device)
+                s.wait_stream(torch.cuda.current_stream())
+                with torch.cuda.stream(s):
+                    self._eval_body(sampled)
+                torch.cuda.current_stream().wait_stream(s)
+                torch.cuda.synchronize()
+                g = torch.cuda.CUDAGraph()
+                with torch.cuda.graph(g, stream=s):
+                    self._eval_body(sampled)
+                torch.cuda.synchronize()
+                ev["graphs"][sampled] = g
+            g.replay()
+        if self.world > 1:
+            self._eval_all_reduce()
+
+    def _eval_all_reduce(self):
+        """Every loss term is a batch mean and the BLEU statistics are counts: scale the means by this shard's B, sum the
+        block over the ranks (one all-reduce, float64 -- exact for the counts) and divide by the global batch."""
+        from .losses import bleu_score_
+        ev, NB, NS = self._eval, self._eval["nb"], _lib.HEADS_NSCALARS
+        red = torch.cat([ev["out"][:NB].double() * self.B, ev["counts"].double(),
+                         torch.full((1,), float(self.B), device=self.device, dtype=torch.float64)])
+        dist.all_reduce(red, op=dist.ReduceOp.SUM, group=self.pg)
+        ev["out"][:NB].copy_(red[:NB] / red[-1])
+        ev["counts"].copy_(red[NB:NB + 10].round().long())
+        bleu_score_(ev["out"][NS + 1:NS + 2], ev["counts"])
+
+    def _eval_aux(self):
+        """run.py:evalstep's adversarial / MI terms (compute_adversarial_losses / compute_mi_losses, forward only) on the
+        evaluation latents in plan.z / mu / logvar."""
+        from . import losses
+        from .functions import adversary_logits
+        m = self.model
+        with torch.no_grad():
+            lat = self._latents(self.plan.z)
+            Y = {n: self.labels[i].reshape(-1, 1) for i, n in enumerate(self.label_names)}
+            A = losses.compute_adversarial_losses(m, adversary_logits(m, lat), Y)
+            M = losses.compute_mi_losses(m, lat, beta=0.01)          # compute_all_losses: mi_loss_weight = 0.01
+        return {"total_adv_loss": A["total_adv_loss"], "total_mi": M["total_mi"], "idv_adv_losses": A["idv_adv_losses"],
+                "idv_adv_dsc_accs": A["idv_adv_dsc_accs"], "idv_mi_estimates": M["idv_mi_estimates"]}
+
+    def _eval_losses(self, slot):
+        ev, NS, NB = self._eval, _lib.HEADS_NSCALARS, self._eval["nb"]
+        h = ev["h_out"][slot]
+        L = self.losses_from(h[:NB], aux=ev["aux"][slot])
+        L["bleu"] = float(h[NS + 1])
+        L["bleu_counts"] = h[NB:].view(torch.int64).tolist()
+        return L
+
+    def eval_step(self, inputs, lengths, labels, teacher_forcing_prob):
+        """Validation step (run.py:evalstep, run.py:347-423) on HOST tensors (inputs [B,T] int64, lengths [B], labels
+        {name: [B,1]}): eval-mode forward (no dropout, one eps draw), the loss dict of compute_all_losses with "cyclic" KL
+        weights at 1.0 (run.py:374-375), plus "bleu" (compute_bleu of the predictions against the inputs) and
+        "bleu_counts" (its 10 corpus statistics, which add over batches).  One captured graph per decode regime
+        (teacher_forcing_prob == 1: forced decode; < 1: sampled decode, coins drawn per call), one H2D and one D2H copy.
+        Parameters, optimizer state, step counters and the training random streams are not touched; plan.z / mu / logvar
+        hold this batch afterwards (utils.LatentLog.append(engine.plan, ids) logs dev latents); eval_predictions holds
+        the predicted tokens.  Data parallel: every rank passes its shard and gets the losses of the global batch."""
+        self._eval_setup()
+        slot = self._enqueue_host_step(inputs, lengths, labels, eval_tf=float(teacher_forcing_prob))
+        self._slot_ev[slot].synchronize()
+        return self._eval_losses(slot)
+
+    def eval_steps(self, batches, teacher_forcing_prob, lag=2):
+        """eval_step over an iterable of HOST batches (inputs, lengths, labels), pipelined as train_steps: yields each
+        batch's loss dict `lag` batches behind the one being enqueued.  Sum "bleu_counts" over the batches and pass them
+        to losses.bleu_from_counts() for the BLEU of the whole dev set."""
+        assert 0 <= lag < self.NSLOT
+        self._eval_setup()
+        tf = float(teacher_forcing_prob)
+        pending = []
+        for inputs, lengths, labels in batches:
+            pending.append(self._enqueue_host_step(inputs, lengths, labels, eval_tf=tf))
+            if len(pending) > lag:
+                slot = pending.pop(0)
+                self._slot_ev[slot].synchronize()
+                yield self._eval_losses(slot)
+        for slot in pending:
+            self._slot_ev[slot].synchronize()
+            yield self._eval_losses(slot)
+
+    @property
+    def eval_predictions(self):
+        """[B,T] token predictions of the last eval_step (device tensor; overwritten by the next one)."""
+        return self._eval["preds"] if self._eval is not None else None
 
     @property
     def token_predictions(self):

@@ -161,6 +161,22 @@ class ConsistencyEvaluator:
         if self.keep_tokens:
             out["token_predictions"][r].copy_(self.preds)
 
+    def bleu(self, out):
+        """[R] float32 device tensor: corpus BLEU (losses.compute_bleu) of every resample's token_predictions against the
+        inputs given to encode_once().  Needs keep_tokens=True.  Runs after resample(), outside its graph: two kernels per
+        resample into one [R,10] block of counters, no host read."""
+        from .losses import bleu_counts_, bleu_score_
+        if "token_predictions" not in out:
+            raise _lib.DvaeError("bleu() needs the token_predictions of resample(): build the evaluator with keep_tokens=True")
+        tok = out["token_predictions"]
+        R = tok.size(0)
+        counts = torch.zeros(R, 10, device=self.device, dtype=torch.int64)
+        scores = torch.empty(R, device=self.device, dtype=torch.float32)
+        for r in range(R):
+            bleu_counts_(counts[r], self.inputs, tok[r], self.model.eos_token_idx)
+            bleu_score_(scores[r:r + 1], counts[r])
+        return scores
+
     def predictions(self, packed_logits):
         """{label: [..., B] int64} = Discriminator.predict (vae/model.py:204-210) on packed logits [..., B, OD]."""
         d, preds, off = self.d, {}, 0

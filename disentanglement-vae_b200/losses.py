@@ -162,6 +162,53 @@ def compute_mi_losses(model, latent_params, beta=1.0):
     return {"total_mi": total_mi, "idv_mi_estimates": idv_mi_estimates}
 
 
+def bleu_counts_(counts, refs, cands, eos_token_idx):
+    """Adds the corpus-BLEU statistics of (refs [B,T_ref], cands [B,T_cand]), int64 device tensors, into `counts`
+    (int64 [10] device tensor, see dvae_bleu_counts) on the current stream."""
+    _lib.check(_lib.load().dvae_bleu_counts(refs.data_ptr(), refs.stride(0), refs.size(1), cands.data_ptr(), cands.stride(0),
+                                            cands.size(1), refs.size(0), int(eos_token_idx), counts.data_ptr(),
+                                            _lib.stream_ptr()), "dvae_bleu_counts")
+    return counts
+
+
+def bleu_score_(score, counts):
+    """score[0] (float32 device tensor) = corpus BLEU of the statistics in `counts`, on the current stream."""
+    _lib.check(_lib.load().dvae_bleu_score(counts.data_ptr(), score.data_ptr(), _lib.stream_ptr()), "dvae_bleu_score")
+    return score
+
+
+def bleu_from_counts(counts, device=None):
+    """Corpus BLEU (float) of accumulated statistics: e.g. the sum of TrainEngine.eval_steps' "bleu_counts" over a dev
+    set, which is the BLEU of the whole set, not the mean of the batches' BLEU."""
+    dev = torch.device("cuda") if device is None else torch.device(device)
+    with torch.cuda.device(dev):
+        c = torch.as_tensor(counts, dtype=torch.int64).to(dev)
+        score = torch.empty(1, device=dev, dtype=torch.float32)
+        return bleu_score_(score, c).item()
+
+
+def compute_bleu(Xbatch, pred_batch, idx2word, eos_token_idx):
+    """vae/losses.py:128-134: corpus BLEU (torchtext 0.6 `bleu_score`, 4-grams, uniform weights) of the predicted sentences
+    against the inputs, each row cut after its first EOS and stripped of its first and last token.
+
+    Computed on the device by `dvae_bleu_counts` + `dvae_bleu_score` over token ids, with one host read.  `idx2word` is
+    accepted and not used: the reference's vocabulary maps ids to distinct words (it is built from sorted unique tokens,
+    run.py:491-504), so comparing ids gives the same matches as comparing the words.  Host or device int64 tensors [B,T]
+    are accepted; the two may have different T."""
+    if Xbatch.dim() != 2 or pred_batch.dim() != 2 or Xbatch.size(0) != pred_batch.size(0):
+        raise ValueError(f"compute_bleu expects two [B,T] token tensors with the same B, got {tuple(Xbatch.shape)} "
+                         f"and {tuple(pred_batch.shape)}")
+    dev = pred_batch.device if pred_batch.is_cuda else (Xbatch.device if Xbatch.is_cuda else torch.device("cuda"))
+    refs = Xbatch.to(dev, torch.int64).contiguous()
+    cands = pred_batch.to(dev, torch.int64).contiguous()
+    with torch.cuda.device(dev):
+        counts = torch.zeros(10, device=dev, dtype=torch.int64)
+        score = torch.empty(1, device=dev, dtype=torch.float32)
+        bleu_counts_(counts, refs, cands, eos_token_idx)
+        bleu_score_(score, counts)
+        return score.item()
+
+
 def compute_all_losses(model, model_outputs, Xbatch, Ybatch, lengths, kl_weights_dict, mi_loss_weight=0.01):
     """run.py:128-163."""
     L = dict()

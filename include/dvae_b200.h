@@ -412,6 +412,23 @@ int dvae_vocab_sample_step_planes(const float* h, int64_t ldh, int B, int H, int
 int dvae_recount_lengths(const int64_t* tokens, int64_t tok_stride_b, int64_t tok_stride_t, int B, int T,
                          int64_t eos, int64_t pad, int64_t min_len, int64_t* lengths_out, void* stream);
 
+/* Corpus BLEU of predicted sentences against their inputs: `compute_bleu` (vae/losses.py:128-134), i.e. torchtext 0.6
+ * `bleu_score` (max_n = 4, weights 0.25, one reference per candidate) over rows cut by `tensor2text` (vae/utils.py:225).
+ * Each row of `ref` [B, T_ref] and `cand` [B, T_cand] (row strides in elements, tokens contiguous) is cut after its first
+ * `eos` (the whole row if it has none) and then loses its first and last token ([1:-1]: SOS and EOS, or SOS and the last
+ * token of a row without EOS).  Token ids are compared, not words: the same result as the reference's strings because
+ * its idx2word is injective (the vocabulary is built from sorted unique tokens, run.py:491-504).
+ *   dvae_bleu_counts: ADDS this batch's statistics into counts[10] = {clipped n-gram matches n = 1..4, candidate n-grams
+ *                     n = 1..4, candidate length, reference length}, so a corpus accumulates over calls and ranks (zero the
+ *                     counters first).  T_ref and T_cand may differ; each must be <= DVAE_BLEU_MAX_T (else DVAE_EINVAL).
+ *   dvae_bleu_score : score_out[0] = 0 if any clipped count is 0, else
+ *                     exp(min(1 - ref_len / cand_len, 0)) * exp(sum_n 0.25 log(clipped_n / total_n)), in float64,
+ *                     stored as float32 in device memory (one thread; capturable in a CUDA graph). */
+#define DVAE_BLEU_MAX_T 256
+int dvae_bleu_counts(const int64_t* ref, int64_t ref_stride, int T_ref, const int64_t* cand, int64_t cand_stride,
+                     int T_cand, int B, int64_t eos, int64_t* counts, void* stream);
+int dvae_bleu_score(const int64_t* counts, float* score_out, void* stream);
+
 /* Backward: d_h [N,H], d_w [V,H], d_bias [V] (all overwritten) for d(loss) = grad_scale_dev[0]
  * (NULL = 1).  Softmax tiles are recomputed from h, w and the saved lse.
  *   ws: dvae_vocab_ce_bwd_ws_floats(N, V, H) floats.
