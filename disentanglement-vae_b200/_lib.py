@@ -73,10 +73,6 @@ SIGNATURES = {
     "dvae_nvls_barrier_words": (_l, []),
     "dvae_nvls_all_reduce": (_i, [_p, _l, _pp, _i, _i, _p, C.c_uint32, C.c_uint32, _i, C.c_uint64, _p, _p]),
     "dvae_p2p_all_reduce": (_i, [_pp, _l, _pp, _i, _i, _p, C.c_uint32, C.c_uint32, _i, C.c_uint64, _p, _p]),
-    "dvae_flag_signal": (_i, [_p, _p, _i, _p, _p]),
-    "dvae_flag_wait": (_i, [_p, _p, _p]),
-    "dvae_flag_signal_value": (_i, [_p, C.c_uint32, _p]),
-    "dvae_flag_wait_value": (_i, [_p, C.c_uint32, _p]),
     "dvae_heads_ws_floats": (_l, [_i, _i]),
     "dvae_latent_heads_fwd": (_i, [_p, _i, _i, _i, _ip, _ip, _p, _p, _p, _p, _p, _p, _p, _p, _p, _i, _p, _p, _p,
                                    _p, _p, _p, _p, _p]),

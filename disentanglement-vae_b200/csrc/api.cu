@@ -32,7 +32,7 @@ void set_defer_joins(bool on);
 namespace {
 struct SideStreams {
   cudaStream_t s[3];
-  cudaStream_t sig = nullptr;                   // carries the bucket-ready flag writes (dvae_flag_signal)
+  cudaStream_t sig = nullptr;                   // carries the gradient-exchange kernels forked by dvae_fork_after
   cudaEvent_t fork_ev, join_ev[3], mark_ev, chain_ev, sig_ev[5], sig_join;
   bool ok = false;
   bool pending[3] = {false, false, false};     // detached work (deferred joins)
@@ -143,34 +143,10 @@ int join_side_streams(cudaStream_t main) {
   return DVAE_OK;
 }
 
-// ---- device flags: ordering between a captured step and work enqueued outside it ---------------------------------
-// A data-parallel step is ONE CUDA graph; the gradient exchanges are NCCL calls enqueued outside it on a communication
-// stream.  Events cannot order the two (an event recorded by a graph node is not seen by a cudaStreamWaitEvent issued
-// before the node runs), so the graph writes "bucket k final" flags in device memory and the communication stream runs
-// a one-thread kernel that polls the flag before each exchange; the other way round for "all exchanges done" before
-// the optimizer kernels.  Values are step counters (monotonic), so nothing is ever reset.
+// ---- scheduling of the gradient exchange inside a captured data-parallel step ---------------------------------------
+// The step counter lives in device memory and is advanced by the graph's first node, so the exchange kernels derive a
+// fresh barrier epoch on every replay without anything being reset.
 namespace {
-__device__ __forceinline__ uint32_t ld_acquire_u32(const uint32_t* p) {
-  uint32_t v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-__global__ void flag_set_kernel(uint32_t* flag, const uint32_t* counter, uint32_t value) {
-  const uint32_t v = counter ? *counter : value;
-  __threadfence();
-  asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(flag), "r"(v) : "memory");
-}
-__global__ void flag_wait_kernel(const uint32_t* flag, const uint32_t* counter, uint32_t value) {
-  const uint32_t want = counter ? *counter : value;
-  uint64_t t0, t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t0));
-  while ((int32_t)(ld_acquire_u32(flag) - want) < 0) {
-    __nanosleep(128);
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    if (t - t0 > 60ull * 1000000000ull) __trap();      // a peer never arrived: fail the context instead of spinning forever
-  }
-  __threadfence();
-}
 __global__ void counter_increment_kernel(uint32_t* counter) { *counter += 1; }
 }  // namespace
 
@@ -196,30 +172,6 @@ int fork_after(bool include_sides, cudaStream_t extra, cudaStream_t main, cudaSt
   return DVAE_OK;
 }
 
-int flag_signal(uint32_t* flag, const uint32_t* counter, bool include_sides, cudaStream_t extra, cudaStream_t main) {
-  SideStreams* ss = side_streams();
-  if (!ss) {      // no side streams: in-stream write
-    flag_set_kernel<<<1, 1, 0, main>>>(flag, counter, 0);
-    DVAE_LAUNCH_CHECK();
-    return DVAE_OK;
-  }
-  DVAE_CUDA(cudaEventRecord(ss->sig_ev[3], main));
-  DVAE_CUDA(cudaStreamWaitEvent(ss->sig, ss->sig_ev[3], 0));
-  if (include_sides)
-    for (int i = 0; i < 3; ++i)
-      if (ss->pending[i]) {
-        DVAE_CUDA(cudaEventRecord(ss->sig_ev[i], ss->s[i]));
-        DVAE_CUDA(cudaStreamWaitEvent(ss->sig, ss->sig_ev[i], 0));
-      }
-  if (extra) {
-    DVAE_CUDA(cudaEventRecord(ss->sig_ev[4], extra));
-    DVAE_CUDA(cudaStreamWaitEvent(ss->sig, ss->sig_ev[4], 0));
-  }
-  flag_set_kernel<<<1, 1, 0, ss->sig>>>(flag, counter, 0);
-  DVAE_LAUNCH_CHECK();
-  ss->sig_pending = true;
-  return DVAE_OK;
-}
 void set_defer_joins(bool on) { g_defer_joins = on; }
 bool defer_joins_enabled() { return g_defer_joins; }
 }  // namespace dvae
@@ -314,34 +266,12 @@ extern "C" int dvae_join_side_streams(void* stream) {
   dvae::set_defer_joins(false);
   return dvae::join_side_streams((cudaStream_t)stream);
 }
-extern "C" int dvae_flag_signal(uint32_t* flag, const uint32_t* counter, int include_sides, void* extra_stream, void* stream) {
-  DVAE_REQUIRE(flag && counter, "dvae_flag_signal: null pointer");
-  return dvae::flag_signal(flag, counter, include_sides != 0, (cudaStream_t)extra_stream, (cudaStream_t)stream);
-}
 extern "C" int dvae_fork_after(int include_sides, void* extra_stream, void* stream, void** forked_stream_out) {
   DVAE_REQUIRE(forked_stream_out, "dvae_fork_after: null pointer");
   cudaStream_t out = nullptr;
   const int rc = dvae::fork_after(include_sides != 0, (cudaStream_t)extra_stream, (cudaStream_t)stream, &out);
   *forked_stream_out = (void*)out;
   return rc;
-}
-extern "C" int dvae_flag_signal_value(uint32_t* flag, uint32_t value, void* stream) {
-  DVAE_REQUIRE(flag, "dvae_flag_signal_value: null pointer");
-  dvae::flag_set_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(flag, nullptr, value);
-  DVAE_LAUNCH_CHECK();
-  return DVAE_OK;
-}
-extern "C" int dvae_flag_wait(const uint32_t* flag, const uint32_t* counter, void* stream) {
-  DVAE_REQUIRE(flag && counter, "dvae_flag_wait: null pointer");
-  dvae::flag_wait_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(flag, counter, 0);
-  DVAE_LAUNCH_CHECK();
-  return DVAE_OK;
-}
-extern "C" int dvae_flag_wait_value(const uint32_t* flag, uint32_t value, void* stream) {
-  DVAE_REQUIRE(flag, "dvae_flag_wait_value: null pointer");
-  dvae::flag_wait_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(flag, nullptr, value);
-  DVAE_LAUNCH_CHECK();
-  return DVAE_OK;
 }
 extern "C" int dvae_counter_increment(uint32_t* counter, void* stream) {
   DVAE_REQUIRE(counter, "dvae_counter_increment: null pointer");

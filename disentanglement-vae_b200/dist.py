@@ -106,32 +106,3 @@ def grad_buckets4(model, flat_grad):
     if hi != base + dec.numel() or lo <= base:          # decoder.linear.* must be the tail of the decoder range
         return [[], b[0], b[1], b[2]]
     return [[flat_grad[lo:hi]], [flat_grad[base:lo]], b[1], b[2]]
-
-
-def grad_buckets5(model, flat_grad):
-    """grad_buckets4 with the last bucket split in two: [3] the encoder embedding's gradient (final when the scatter of
-    layer 0's input gradient has run) and [4] encoder layer 0's weights (final when its weight-gradient GEMMs, which run
-    on side streams in the tail of the step, have drained).  The 10 MB embedding exchange then runs under those GEMMs.
-    For the in-graph exchange kernels only: with NCCL the extra launch (~20 us of fixed latency) costs more than it hides."""
-    b = grad_buckets4(model, flat_grad)
-    lay, named = model._layout, dict(model.named_parameters())
-    emb = "encoder.embedding.weight"
-    if len(b[3]) != 1 or emb not in lay or lay[emb] != 0:
-        return [b[0], b[1], b[2], [], b[3]]          # everything waits for the drained side streams
-    low = b[3][0]
-    cut = (named[emb].numel() + 3) // 4 * 4
-    if (low.data_ptr() - flat_grad.data_ptr()) != 0 or cut >= low.numel() or any(0 < off < cut for off in lay.values()):
-        return [b[0], b[1], b[2], [], b[3]]
-    return [b[0], b[1], b[2], [low[:cut]], [low[cut:]]]
-
-
-def all_reduce_views_(views, group=None):
-    """SUM all-reduce of several views as ONE NCCL launch where the backend coalesces (each launch costs ~20 us of fixed
-    latency at these sizes: 1 MB 24 us, 10 MB 51 us, 36 MB 91 us on 2 B200s); one call per view otherwise."""
-    if len(views) > 1 and views[0].is_cuda and hasattr(dist, "_coalescing_manager"):
-        with dist._coalescing_manager(group=group, device=views[0].device, async_ops=False):
-            for v in views:
-                dist.all_reduce(v, op=dist.ReduceOp.SUM, group=group)
-        return
-    for v in views:
-        dist.all_reduce(v, op=dist.ReduceOp.SUM, group=group)

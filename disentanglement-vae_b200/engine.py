@@ -1,8 +1,9 @@
 """Graph-captured data-parallel training engine: the reference's train-step body
 (`run.py:217-276`: forward -> compute_all_losses -> backward -> clip_grad_norm_(5.0) -> [adversary steps] ->
 Adam.step -> zero_grad -> [MI-estimator steps]) as one fixed sequence of C-ABI kernel launches over pre-allocated
-buffers, replayed as CUDA graphs, with the NCCL all-reduce of the flat gradient buffer between backward and the
-optimiser tail when world_size > 1.
+buffers, replayed as CUDA graphs.  When world_size > 1 the flat gradient buffer is summed over the ranks in four buckets
+by the repo's all-reduce kernel inside the one step graph (peer-to-peer at two ranks, NVSwitch multicast beyond), or,
+when its start-up self-test fails on any rank, by NCCL between stage graphs.
 
 Same kernels and the same `StepPlan` as the drop-in autograd path (`functions.py`); what the engine removes is
 per-op host work (autograd bookkeeping, ctypes marshalling, allocator traffic).
@@ -29,7 +30,6 @@ from . import _lib
 from ._lib import ptr, check
 from .plan import StepPlan
 from .losses import get_cyclic_kl_weight
-from .dist import all_reduce_views_
 
 
 def d_bow(plan):
@@ -68,6 +68,7 @@ class TrainEngine:
         self.flat = model._flat[:self.n]
         self.use_graph = use_graph
         self._nvls = None
+        # DVAE_DP_NVLS=0 skips the exchange kernel: the one way to run the NCCL fallback where the kernel works (tests)
         if self.world > 1 and use_graph and not self.aux and os.environ.get("DVAE_DP_NVLS", "1") != "0":
             self._setup_nvls()          # gradient buffer in multicast memory (self.grad), or None: NCCL exchanges
         if self._nvls is None:
@@ -136,11 +137,9 @@ class TrainEngine:
         self._graphs = None
         self._buckets = None
         self._comm = None
-        # one-graph data parallel (dvae_flag_*): step counter, "bucket k final" flags [0..3] and "exchanges done" flag [7]
-        self._flag_mode = False
-        self._dp_step = 0
+        self._xchg_in_capture = False      # one-graph data parallel: the step being captured exchanges inside the graph
+        # step counter in device memory, from which the exchange kernels derive their barrier epochs
         self._dp_ctr = torch.zeros(1, dtype=torch.int32, device=self.device)
-        self._dp_flags = torch.zeros(8, dtype=torch.int32, device=self.device)
         self._side = None
         self.label_names = [n for n, o in zip(d.space_names, d.dsc_out) if o > 0]
         self.last_aux = {}
@@ -233,8 +232,8 @@ class TrainEngine:
         st = _lib.stream_ptr()
         cur = torch.cuda.current_stream()
         # part 0 (data parallel only): forward + vocabulary backward on their own, so that W_out's gradient is exchanged first
-        flags = self._flag_mode and part is None      # one-graph data parallel: exchanges / "bucket final" flags inside the graph
-        if flags:
+        xchg = self._xchg_in_capture and part is None      # one-graph data parallel: the exchanges inside the graph
+        if xchg:
             check(self.lib.dvae_counter_increment(ptr(self._dp_ctr), st), "dvae_counter_increment")
         if part == 0 or part is None or (part == 1 and not self._three_buckets()):
             h_top, hoist = self._forward()
@@ -246,7 +245,7 @@ class TrainEngine:
             if part == 0:
                 check(self.lib.dvae_join_side_streams(st), "dvae_join_side_streams")      # d_w runs on a side stream
                 return
-            if flags:
+            if xchg:
                 self._signal(0, True)
         if part in (None, 1):
             g_top, hoist = self._g_top, self._hoist
@@ -261,7 +260,7 @@ class TrainEngine:
                     if hoist:
                         cur.wait_stream(self._side)
             self._aux_pending = hoist and part is None
-            if flags:
+            if xchg:
                 self._signal(1, True, self._side if hoist else None)
         emb_enc = "encoder.embedding.weight" in m._layout
         if part in (None, 2):
@@ -274,21 +273,15 @@ class TrainEngine:
                 self._g_ctx = g_ctx
                 # data parallel with a multi-layer encoder: stop after the upper layers (their gradients go out under layer 0)
                 split = part == 2 and self._three_buckets()
-                if flags:
+                if xchg:
                     pl.encode_bwd(P, G, self.inputs, self.lengths, g_ctx, emb_grad=emb_enc, layers=(pl.d.Le - 1, 1))
                     self._signal(2, True)
                     pl.encode_bwd(P, G, self.inputs, self.lengths, g_ctx, emb_grad=emb_enc, layers=(0, 0))
-                    if len(self._buckets) == 5:      # exchange kernels: the encoder embedding's 10 MB go out as soon as the scatter
-                        self._signal(3, False)       # (on this stream) has run, under layer 0's weight-gradient GEMMs ...
-                        self._signal(4, True)        # ... whose 4 MB follow when the side streams have drained
-                    else:                            # NCCL: one launch (each costs ~20 us of fixed latency)
-                        self._signal(3, True)
+                    self._signal(3, True)
                 else:
                     pl.encode_bwd(P, G, self.inputs, self.lengths, g_ctx, emb_grad=emb_enc, layers=(pl.d.Le - 1, 1) if split else None)
             finally:
                 check(self.lib.dvae_join_side_streams(st), "dvae_join_side_streams")
-            if flags and self._nvls is None:      # every exchange of this step has finished (the communication stream says so)
-                check(self.lib.dvae_flag_wait(ptr(self._dp_flags[7:]), ptr(self._dp_ctr), st), "dvae_flag_wait")
         if part == 3:
             check(self.lib.dvae_defer_joins(1), "dvae_defer_joins")
             try:
@@ -316,8 +309,8 @@ class TrainEngine:
             return False
 
         # two GPUs: plain peer-to-peer loads / stores move a third of the bytes of the switch detour (measured 1.35 ms per cfg2
-        # step with multimem against 1.25 peer-to-peer at N = 2; multimem 1.25 against NCCL's 1.51 at N = 4); DVAE_DP_XCHG forces
-        mode = os.environ.get("DVAE_DP_XCHG", "p2p" if self.world == 2 else "nvls")
+        # step with multimem against 1.25 peer-to-peer at N = 2; multimem 1.25 against NCCL's 1.51 at N = 4)
+        mode = "p2p" if self.world == 2 else "nvls"
         n_pad = (self.n + 3) // 4 * 4
         ok, why, st = True, "", {}
         try:
@@ -362,62 +355,49 @@ class TrainEngine:
         self.grad = st["buf"][:self.n]
         self._nvls = st
 
+    # CTAs of the exchange kernel per bucket: early buckets finish under hundreds of us of backward pass, the last one is
+    # (nearly) exposed
+    XCHG_CTAS = (16, 16, 32, 64)
+
     def _signal(self, k, include_sides, extra=None):
         """Bucket k's gradients are final once everything enqueued so far (and, include_sides, the detached side-stream
-        work and `extra`) has run: start its exchange there, beside the rest of the backward pass."""
-        if self._nvls is not None:
-            # the exchange itself, as graph nodes on the library's signal stream: one multicast all-reduce kernel per view
-            import ctypes as C
-            out = C.c_void_p()
-            check(self.lib.dvae_fork_after(1 if include_sides else 0, extra.cuda_stream if extra is not None else None,
-                                           _lib.stream_ptr(), C.byref(out)), "dvae_fork_after")
-            nv = self._nvls
-            # early buckets finish under hundreds of us of backward pass: few CTAs; the late ones are (nearly) exposed
-            ctas = [int(c) for c in os.environ.get("DVAE_XCHG_CTAS", "16,16,32,64,64").split(",")][min(k, 4)]
-            if len(self._buckets) == 4 and k == 3:
-                ctas = max(ctas, 64)
-            for j, v in enumerate(self._buckets[k]):
-                off = v.data_ptr() - nv["buf"].data_ptr()
-                n = (v.numel() + 3) // 4 * 4
-                if nv["mode"] == "p2p":
-                    peers = (C.c_void_p * self.world)(*[bp + off for bp in nv["buf_ptrs"]])
-                    check(self.lib.dvae_p2p_all_reduce(peers, n, nv["bar_ptrs"], self.rank, self.world, ptr(self._dp_ctr),
-                                                       16, 2 * k + j + 1, ctas, 0, None, out.value), "dvae_p2p_all_reduce")
-                else:
-                    check(self.lib.dvae_nvls_all_reduce(nv["mc"] + off, n, nv["bar_ptrs"], self.rank, self.world, ptr(self._dp_ctr),
-                                                        16, 2 * k + j + 1, ctas, 0, None, out.value), "dvae_nvls_all_reduce")
-            return
-        check(self.lib.dvae_flag_signal(ptr(self._dp_flags[k:]), ptr(self._dp_ctr), 1 if include_sides else 0,
-                                        extra.cuda_stream if extra is not None else None, _lib.stream_ptr()), "dvae_flag_signal")
+        work and `extra`) has run: start its exchange there, beside the rest of the backward pass -- as graph nodes on the
+        library's signal stream, one all-reduce kernel per view."""
+        import ctypes as C
+        out = C.c_void_p()
+        check(self.lib.dvae_fork_after(1 if include_sides else 0, extra.cuda_stream if extra is not None else None,
+                                       _lib.stream_ptr(), C.byref(out)), "dvae_fork_after")
+        nv = self._nvls
+        ctas = self.XCHG_CTAS[k]
+        for j, v in enumerate(self._buckets[k]):
+            off = v.data_ptr() - nv["buf"].data_ptr()
+            n = (v.numel() + 3) // 4 * 4
+            if nv["mode"] == "p2p":
+                peers = (C.c_void_p * self.world)(*[bp + off for bp in nv["buf_ptrs"]])
+                check(self.lib.dvae_p2p_all_reduce(peers, n, nv["bar_ptrs"], self.rank, self.world, ptr(self._dp_ctr),
+                                                   16, 2 * k + j + 1, ctas, 0, None, out.value), "dvae_p2p_all_reduce")
+            else:
+                check(self.lib.dvae_nvls_all_reduce(nv["mc"] + off, n, nv["bar_ptrs"], self.rank, self.world, ptr(self._dp_ctr),
+                                                    16, 2 * k + j + 1, ctas, 0, None, out.value), "dvae_nvls_all_reduce")
 
     def _one_graph_dp(self):
-        """Data parallel as ONE graph per step: the exchanges are the repo's all-reduce kernels inside it (csrc/nvls.cu), or
-        (DVAE_DP_FLAGS=1) NCCL calls outside it ordered by device flags.  Otherwise: four stage graphs with NCCL between
-        them, whose ends also end the overlap of the weight-gradient GEMMs with the next recurrence."""
-        if not (self._three_buckets() and self.use_graph and not self.aux):
-            return False
-        # NCCL behind device flags is opt-in: it measured 1.26 (N=2) / 1.32 ms (N=4) per cfg2 step against 1.37 / 1.51 for the
-        # stage graphs, but two of seven runs sat at ~5 ms per step (a polling kernel ahead of NCCL's own stream ordering)
-        return self._nvls is not None or os.environ.get("DVAE_DP_FLAGS", "0") == "1"
+        """Data parallel as ONE graph per step, the exchanges being the repo's all-reduce kernels inside it (csrc/nvls.cu):
+        needs the kernel set up, graphs on and the four-bucket split.  Otherwise: stage graphs (or eager stages) with NCCL
+        between them, whose ends also end the overlap of the weight-gradient GEMMs with the next recurrence."""
+        return self._nvls is not None and self.use_graph and self._three_buckets()
 
     @property
     def exchange_mode(self):
-        """How this engine exchanges gradients: none | p2p | nvls (repo kernel inside the one-graph step) | nccl+flags |
-        nccl+stages."""
+        """How this engine exchanges gradients: none (one rank) | p2p | nvls (the repo's kernel inside the one-graph step,
+        peer-to-peer at two ranks, NVSwitch multicast beyond) | nccl+stages (NCCL between stage graphs: the fallback)."""
         if self.world == 1:
             return "none"
-        if self._nvls is not None and self._one_graph_dp():
-            return self._nvls["mode"]
-        return "nccl+flags" if self._one_graph_dp() else "nccl+stages"
+        return self._nvls["mode"] if self._one_graph_dp() else "nccl+stages"
 
     def _ensure_buckets(self):
         if self._buckets is None:
-            from .dist import grad_buckets4, grad_buckets3, grad_buckets5
-            # DVAE_DP_BUCKETS=5: encoder embedding ahead of layer 0's weights.  Measured no gain at N = 2 (1.27 vs 1.25 ms): the
-            # signal stream is still busy with stage 2's exchange when the embedding's gradient becomes final
-            if self._three_buckets() and self._nvls is not None and os.environ.get("DVAE_DP_BUCKETS", "4") == "5":
-                self._buckets = grad_buckets5(self.model, self.grad)
-            elif self._three_buckets():
+            from .dist import grad_buckets4, grad_buckets3
+            if self._three_buckets():
                 self._buckets = grad_buckets4(self.model, self.grad)
             else:
                 b3 = grad_buckets3(self.model, self.grad)
@@ -425,7 +405,7 @@ class TrainEngine:
             self._comm = torch.cuda.Stream(device=self.device)
 
     def _three_buckets(self):
-        return (self.world > 1 and not self.plan.d.bow and self.plan.d.Le >= 2 and os.environ.get("DVAE_DP_BUCKETS", "4") != "2")
+        return self.world > 1 and not self.plan.d.bow and self.plan.d.Le >= 2
 
     def _optim(self):
         st = _lib.stream_ptr()
@@ -478,10 +458,6 @@ class TrainEngine:
                          "idv_adv_losses": A["idv_adv_losses"], "idv_adv_dsc_accs": A["idv_adv_dsc_accs"],
                          "idv_mi_estimates": M["idv_mi_estimates"], "mi_estimator_loss": est_losses}
 
-    def _grad_buckets(self):
-        from .dist import grad_buckets
-        return grad_buckets(self.model, self.grad)
-
     def weight_planes(self):
         """Context manager for callers that drive the plan's kernel sequences themselves (bench.py's per-kernel timings):
         current planes, registry on inside the block."""
@@ -525,46 +501,27 @@ class TrainEngine:
             return
         # data parallel: gradients are all-reduced in the order the backward pass finishes them, on a communication stream,
         # under the rest of the backward pass: W_out | decoder embedding + LSTM | upper encoder layers + heads | encoder
-        # embedding + layer 0 (four stages, four graphs); DVAE_DP_BUCKETS=2: decoder | everything else (round 1)
-        three = self._three_buckets()
+        # embedding + layer 0 (four stages); bag-of-words or one-layer encoders: decoder | everything else (two stages)
         self._ensure_buckets()
         cur = torch.cuda.current_stream()
         if self.use_graph and self._graphs is None:
             self._capture()
-        if self._one_graph_dp():
-            self._dp_step += 1
+        if self._one_graph_dp():      # the exchanges are nodes of the graph
             self._graphs[0].replay()
-            if self._nvls is not None:      # the exchanges are nodes of the graph
-                return
-            # each NCCL exchange waits (on the device) for its bucket's flag of THIS step, and the graph's optimizer kernels
-            # wait for the flag written after the last exchange
-            cs = self._comm.cuda_stream
-            with torch.cuda.stream(self._comm):
-                for k, bucket in enumerate(self._buckets):
-                    if not bucket:
-                        continue
-                    check(self.lib.dvae_flag_wait_value(ptr(self._dp_flags[k:]), self._dp_step, cs), "dvae_flag_wait_value")
-                    all_reduce_views_(bucket, self.pg)
-                check(self.lib.dvae_flag_signal_value(ptr(self._dp_flags[7:]), self._dp_step, cs), "dvae_flag_signal_value")
             return
-        overlap = os.environ.get("DVAE_DP_OVERLAP", "1") != "0"
-        stages = (0, 1, 2, 3) if three else (1, 2)
+        # NCCL on the communication stream between stage graphs (or eager stages); stage gi finishes bucket gi
+        stages = (0, 1, 2, 3) if self._three_buckets() else (1, 2)
         for gi, part in enumerate(stages):
             if self.use_graph:
                 self._graphs[gi].replay()
             else:
                 self._fwd_bwd(part)
-            # the last stage takes every remaining bucket (five of them when the exchange kernels' finer split is in use)
-            views = [v for b in (self._buckets[gi:] if gi == len(stages) - 1 else self._buckets[gi:gi + 1]) for v in b]
-            if overlap and views:
+            if self._buckets[gi]:
                 self._comm.wait_stream(cur)
                 with torch.cuda.stream(self._comm):
-                    for v in views:
+                    for v in self._buckets[gi]:
                         dist.all_reduce(v, op=dist.ReduceOp.SUM, group=self.pg)
-        if overlap:
-            cur.wait_stream(self._comm)
-        else:
-            dist.all_reduce(self.grad, op=dist.ReduceOp.SUM, group=self.pg)
+        cur.wait_stream(self._comm)
         if self.use_graph:
             self._graphs[-1].replay()
         else:
@@ -589,18 +546,14 @@ class TrainEngine:
                 self._optim()
             graphs.append(g)
         elif self._one_graph_dp():
-            for bucket in self._buckets:      # communicator set-up (seconds) must not happen under a polling kernel
-                if bucket and self._nvls is None:
-                    all_reduce_views_(bucket, self.pg)
-            torch.cuda.synchronize()
             g = torch.cuda.CUDAGraph()
-            self._flag_mode = True
+            self._xchg_in_capture = True
             try:
                 with torch.cuda.graph(g, stream=s):
                     self._fwd_bwd(None)
                     self._optim()
             finally:
-                self._flag_mode = False
+                self._xchg_in_capture = False
             graphs.append(g)
         else:                 # the all-reduces sit between the graphs (NCCL on its own stream)
             for part in ((0, 1, 2, 3) if self._three_buckets() else (1, 2)):

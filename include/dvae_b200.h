@@ -125,25 +125,16 @@ int dvae_weight_planes_clear(void);
 int dvae_defer_joins(int on);
 int dvae_join_side_streams(void* stream);
 
-/* Device flags: ordering between a step captured as ONE CUDA graph and the gradient exchanges (NCCL) enqueued outside it.
- * An event recorded by a graph node cannot be waited on by a stream call issued before the node has run, so the order is
- * carried by step counters in device memory instead:
- *   dvae_counter_increment   *counter += 1                                  (first node of the captured step)
- *   dvae_flag_signal         *flag = *counter once everything enqueued so far on `stream` -- and, include_sides != 0, the
- *                            detached side-stream work (dvae_defer_joins) and `extra_stream` (or NULL) -- has finished;
- *                            runs on a library stream, does not block `stream`; joined by dvae_join_side_streams
- *   dvae_flag_wait           in-stream: a one-thread kernel polls until *flag >= *counter (wrap-safe), traps after 60 s
- *   dvae_flag_signal_value / dvae_flag_wait_value: the same with the value passed from the host (the eager side).
+/* Scheduling of the gradient exchange inside a data-parallel step captured as ONE CUDA graph:
+ *   dvae_counter_increment   *counter += 1 (first node of the captured step): the step counter from which the exchange
+ *                            kernels derive their barrier epochs, so that nothing is reset between replays
+ *   dvae_fork_after          the library's signal stream, made to wait for everything enqueued so far on `stream` -- and,
+ *                            include_sides != 0, the detached side-stream work (dvae_defer_joins) and `extra_stream` (or
+ *                            NULL); what the caller enqueues on *forked_stream_out afterwards runs beside `stream` until
+ *                            dvae_join_side_streams(stream)
  * Replaces nothing in the reference: it is the scheduling of DistributedDataParallel's bucketed gradient exchange. */
 int dvae_counter_increment(uint32_t* counter, void* stream);
-/* The library's signal stream, made to wait for everything enqueued so far on `stream` (+ detached side work / extra_stream
- * as for dvae_flag_signal); what the caller enqueues on *forked_stream_out afterwards runs beside `stream` until
- * dvae_join_side_streams(stream).  Used for the gradient-exchange kernels of a data-parallel step. */
 int dvae_fork_after(int include_sides, void* extra_stream, void* stream, void** forked_stream_out);
-int dvae_flag_signal(uint32_t* flag, const uint32_t* counter, int include_sides, void* extra_stream, void* stream);
-int dvae_flag_wait(const uint32_t* flag, const uint32_t* counter, void* stream);
-int dvae_flag_signal_value(uint32_t* flag, uint32_t value, void* stream);
-int dvae_flag_wait_value(const uint32_t* flag, uint32_t value, void* stream);
 
 /* All-reduce (SUM, in place) of one gradient bucket over NVSwitch multicast memory, one kernel per rank (nvls.cu):
  * cross-rank barrier, multimem.ld_reduce of this rank's 1/world slice, multimem.st of the sums into every rank's buffer,

@@ -1,9 +1,9 @@
 """Worker of tests/test_gpu_dp.py, launched by `python -m torch.distributed.run` with one rank per GPU.
 
 Every rank builds the same model, takes its strided shard of a seeded GLOBAL batch and runs K steps of the
-data-parallel TrainEngine (CUDA graphs + bucketed NCCL all-reduce on a communication stream, exactly what bench.py
-times at N > 1) with dropout off and the reparameterisation noise given, so that the run is comparable with a
-single-process engine on the whole batch.  Rank 0 writes the final weights and per-step losses."""
+data-parallel TrainEngine (CUDA graphs + bucketed gradient exchange, exactly what bench.py times at N > 1) with
+dropout off and the reparameterisation noise given, so that the run is comparable with a single-process engine on the
+whole batch.  Rank 0 writes the final weights and per-step losses."""
 import importlib
 import os
 import sys

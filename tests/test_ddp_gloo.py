@@ -160,30 +160,3 @@ def test_four_stage_split_puts_the_output_layer_first(dvae):
     assert sum(v.numel() for v in b[0]) >= n_lin and sum(v.numel() for v in b[0]) <= n_lin + 8
     off = vae._layout["decoder.linear.weight"]
     assert b[0][0].data_ptr() == flat.data_ptr() + 4 * off
-
-
-
-def test_five_stage_split_sends_the_encoder_embedding_before_layer_zero(dvae):
-    """In-graph exchange kernels (engine._signal): bucket [3] is exactly the encoder embedding's gradient, bucket [4] the rest
-    of the old last bucket (encoder layer 0), and the five buckets still cover the flat buffer exactly once."""
-    import importlib
-    dvae_dist = importlib.import_module("disentanglement-vae_b200.dist")
-    p = dict(bow_encoder=False, embedding_dim=12, hidden_dim=16, num_rnn_layers=2, encoder_dropout=0.0, decoder_dropout=0.0,
-             bidirectional_encoder=True, latent_dims={"total": 7, "polarity": 1, "uncertainty": 2}, adversarial_loss=False, mi_loss=False)
-    vae = dvae.build_vae(p, 29, None, {"uncertainty": 3, "polarity": 1}, torch.device("cpu"), 2, 3)
-    flat = torch.zeros(vae._flat_numel)
-    b = dvae_dist.grad_buckets5(vae, flat)
-    b4 = dvae_dist.grad_buckets4(vae, flat)
-    assert len(b) == 5
-    for views in b:
-        for v in views:
-            v += 1.0
-    assert torch.equal(flat, torch.ones_like(flat))
-    named = dict(vae.named_parameters())
-    n_emb = named["encoder.embedding.weight"].numel()
-    assert len(b[3]) == 1 and b[3][0].data_ptr() == flat.data_ptr() and n_emb <= b[3][0].numel() <= n_emb + 3
-    assert sum(v.numel() for v in b[3]) + sum(v.numel() for v in b[4]) == sum(v.numel() for v in b4[3])
-    for name, off in vae._layout.items():
-        if "_l0" in name and name.startswith("encoder.recurrent."):
-            lo = (b[4][0].data_ptr() - flat.data_ptr()) // 4
-            assert lo <= off and off + named[name].numel() <= lo + b[4][0].numel()

@@ -1,8 +1,8 @@
 """Hardware data-parallel parity (SURVEY.md 4(iv), VERDICT r1 "next 1b"): N ranks x (B/N) rows through the data-parallel
 TrainEngine must take the same optimisation steps as ONE engine on the concatenated batch, for every gradient exchange
-the engine has: the repo's all-reduce kernel inside a one-graph step (peer-to-peer loads / stores, NVSwitch multicast),
-NCCL outside a one-graph step ordered by device flags, and NCCL between four stage graphs.  Also the exchange kernel on
-its own against exact sums.  Spawns `torch.distributed.run`; skipped with < 2 GPUs."""
+the engine has: the repo's all-reduce kernel inside a one-graph step (peer-to-peer loads / stores at N = 2, NVSwitch
+multicast at N = 4) and the NCCL fallback between four stage graphs.  Also the exchange kernel on its own, both
+variants, against exact sums.  Spawns `torch.distributed.run`; skipped with < 2 GPUs."""
 import os
 import socket
 import subprocess
@@ -29,9 +29,6 @@ def _free_port():
 
 EXCHANGES = {                      # environment of the worker -> which exchange the engine uses
     "default": {},
-    "p2p": {"DVAE_DP_XCHG": "p2p"},
-    "multicast": {"DVAE_DP_XCHG": "nvls"},
-    "nccl_flags": {"DVAE_DP_NVLS": "0", "DVAE_DP_FLAGS": "1"},
     "nccl_stages": {"DVAE_DP_NVLS": "0"},
 }
 
@@ -55,8 +52,7 @@ def test_all_reduce_kernel_gives_exact_sums_on_every_rank(world):
     assert "XCHG_OK" in r.stdout, r.stdout[-2000:]
 
 
-@pytest.mark.parametrize("world,exchange", [(2, "default"), (2, "multicast"), (2, "nccl_flags"), (2, "nccl_stages"),
-                                            (4, "default")])
+@pytest.mark.parametrize("world,exchange", [(2, "default"), (2, "nccl_stages"), (4, "default")])
 def test_n_rank_engine_equals_single_rank_on_the_global_batch(tmp_path, world, exchange):
     if not torch.cuda.is_available() or torch.cuda.device_count() < world:
         pytest.skip(f"needs {world} GPUs")
@@ -64,8 +60,7 @@ def test_n_rank_engine_equals_single_rank_on_the_global_batch(tmp_path, world, e
     r = _torchrun(world, "dp_worker.py", out, env=EXCHANGES[exchange])
     assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-3000:]
     got = np.load(out)
-    want_mode = {"default": "p2p" if world == 2 else "nvls", "p2p": "p2p", "multicast": "nvls", "nccl_flags": "nccl+flags",
-                 "nccl_stages": "nccl+stages"}[exchange]
+    want_mode = {"default": "p2p" if world == 2 else "nvls", "nccl_stages": "nccl+stages"}[exchange]
     assert str(got["exchange"]) == want_mode, (str(got["exchange"]), want_mode)
     assert got["replicas_identical"][0] == 1.0, "ranks diverged: parameters differ after the all-reduced steps"
     import dp_worker
