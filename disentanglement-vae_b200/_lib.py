@@ -85,8 +85,11 @@ SIGNATURES = {
     "dvae_vocab_split_w": (_i, [_p, _i, _i, _i, _p, _p]),
     "dvae_vocab_ce_fwd_ex": (_i, [_p, _l, _i, _i, _i, _i, _p, _p, _p, _l, _p, _i, _p, _p, _p, _p, _p, _i, _p]),
     "dvae_vocab_ce_partials": (_i, [_p, _l, _i, _i, _i, _i, _p, _p, _p, _l, _p, _i, _p, _p]),
+    "dvae_vocab_ce_fwd_live": (_i, [_p, _l, _i, _i, _i, _i, _p, _p, _p, _l, _p, _i, _p, _p, _p, _p, _p, _i, _p]),
+    "dvae_vocab_live_rows_at": (_l, [_i, _i, _i]),
     "dvae_vocab_ce_bwd_ws_floats": (_l, [_i, _i, _i]),
     "dvae_vocab_ce_bwd": (_i, [_p, _l, _i, _i, _i, _i, _p, _p, _p, _l, _p, _p, _p, _p, _l, _p, _p, _p, _p, _p]),
+    "dvae_vocab_ce_bwd_live": (_i, [_p, _l, _i, _i, _i, _i, _p, _p, _p, _l, _p, _p, _p, _p, _l, _p, _p, _p, _p, _p]),
     "dvae_entropy_loss": (_i, [_p, _i, _i, _p, _p, _p, _p]),
     "dvae_club_mi": (_i, [_p, _p, _p, _i, _i, _p, _p, _p, _p, _p, _p, _p]),
     "dvae_club_nll": (_i, [_p, _p, _p, _i, _i, _p, _p, _p, _p, _p]),

@@ -68,7 +68,6 @@ constexpr int EPI_SCRATCH_BYTES = 8 * 32 * 32 * 4;               // per epilogue
 constexpr int AS_MAX_KB = 8, AS_KB_PER_STAGE = DVAE_AS_KB, AS_STAGE_BYTES = AS_KB_PER_STAGE * PS_TILE;
 constexpr int AS_STAGES = 12 / AS_KB_PER_STAGE, AS_STAGES_NOSCRATCH = 14 / AS_KB_PER_STAGE;
 constexpr uint32_t AS_T_AHI = 256, AS_T_ALO = 384;       // TMEM columns of the stationary A planes
-constexpr float kSingleScale = 256.f;                    // operand scale of the single-accumulator planes
 // [operand ring 192 KB][epilogue transpose scratch 32 KB][bias tiles 2 KB][barriers]
 constexpr int OFF_SCRATCH = STAGES * STAGE_BYTES;
 constexpr int OFF_BIAS = OFF_SCRATCH + EPI_SCRATCH_BYTES;          // per epilogue warp: the bias values of its tile columns
@@ -291,13 +290,47 @@ tc16_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
       for (int64_t i = blk * NUM_THREADS + tid; i < p.zero2_n4; i += nblk * NUM_THREADS) y4[i] = make_float4(0.f, 0.f, 0.f, 0.f);
     }
   }
-  const int m0 = blockIdx.x * BM;
-  const int nt0 = blockIdx.y * p.tiles_per_cta;
   const int n_tiles = (p.N + BN - 1) / BN;
-  const int nt1 = min(n_tiles, nt0 + p.tiles_per_cta);
-  const int nkb_total = (p.K + BK - 1) / BK;
-  const int kb0 = blockIdx.z * p.kb_per_split;
-  const int nkb = max(0, min(nkb_total, kb0 + p.kb_per_split) - kb0);
+  const int nkb_total = (p.K + BK - 1) / BK;   // k-blocks per row block of the operand planes (addressing)
+  // this CTA's (row tile, column-tile group, k split): the launch grid, or -- live rows -- the launched CTAs re-partitioned
+  // over the work the device-side live count leaves.  A CTA without work has cleared its share of zero_buf above and
+  // returns here, before barrier init, TMEM allocation or any wait: every CTA decides from the same *m_live, and M = 0
+  // (no live row) leaves every CTA idle, i.e. the launch is a no-op apart from the clearing.
+  int bx = blockIdx.x, by = blockIdx.y, bz = blockIdx.z, M = p.M, tpc = p.tiles_per_cta, kbps = p.kb_per_split;
+  int kb_end = nkb_total;
+  int64_t mstride = p.M;                       // mode 1: row stride of the partials
+  if (p.m_live) {
+    const int live = *p.m_live;
+    if (p.live_k) {                            // d_w = P^T . h: K runs over the live positions, split over the launched z
+      kb_end = (live + BK - 1) / BK;
+      kbps = (kb_end + (int)gridDim.z - 1) / (int)gridDim.z;
+      if (bz * kbps >= kb_end) return;
+    } else {
+      M = live;
+      const int rt = (M + BM - 1) / BM;
+      const int ctas = gridDim.x * gridDim.y * gridDim.z, c = (blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x;
+      if (rt == 0) return;
+      if (p.mode != 0) {                       // vocabulary groups x tiles per CTA: one wave over the live row tiles
+        int groups;
+        live_split(rt, ctas, n_tiles, &tpc, &groups);
+        if (c >= rt * groups) return;
+        bx = c % rt; by = c / rt; bz = 0;
+        mstride = (int64_t)rt * BM;
+      } else {                                 // d_h: the split-K factor grows as the live row tiles shrink
+        const int tiles = rt * gridDim.y;
+        int splits = max(1, min(nkb_total, ctas / tiles));
+        kbps = (nkb_total + splits - 1) / splits;
+        splits = (nkb_total + kbps - 1) / kbps;
+        if (c >= tiles * splits) return;
+        bx = c % rt; by = (c / rt) % gridDim.y; bz = c / tiles;
+      }
+    }
+  }
+  const int m0 = bx * BM;
+  const int nt0 = by * tpc;
+  const int nt1 = min(n_tiles, nt0 + tpc);
+  const int kb0 = bz * kbps;
+  const int nkb = max(0, min(kb_end, kb0 + kbps) - kb0);
   const int b_tile0 = p.b_row0 / BN;          // pre-split B planes: first row block of this launch's vocabulary chunk
 
   if (tid == 0) {
@@ -326,7 +359,7 @@ tc16_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   const int nstages = a_stat ? (p.mode == 1 ? AS_STAGES_NOSCRATCH : AS_STAGES) : STAGES;
   const uint32_t stage_bytes = a_stat ? AS_STAGE_BYTES : STAGE_BYTES;
   // (a padding CTA of an odd row-block count in CTA-pair mode re-reads the last real block: it only keeps the protocol going)
-  const int a_blk = min((int)blockIdx.x, (p.M + BM - 1) / BM - 1);
+  const int a_blk = min(bx, (M + BM - 1) / BM - 1);
   if (warp == MMA_WARP) tmem_alloc(tmem_slot, TMEM_COLS);
   tc_fence_before();
   __syncthreads();
@@ -367,7 +400,7 @@ tc16_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     } else if (lane == 0 && p.presplit) {
       // operand planes straight into the operand ring: one 16 KB tile k-block [hi, lo] per operand
       const uint8_t* a_tiles = reinterpret_cast<const uint8_t*>(p.a_planes) +
-                               ((int64_t)blockIdx.x * (p.a_kbtot ? p.a_kbtot : nkb_total) + p.a_kb0) * PS_TILE;
+                               ((int64_t)bx * (p.a_kbtot ? p.a_kbtot : nkb_total) + p.a_kb0) * PS_TILE;
       const uint8_t* b_planes = reinterpret_cast<const uint8_t*>(p.b_planes);
       int stage = 0, phase = 0;
       for (int nt = nt0; nt < nt1; ++nt) {
@@ -539,7 +572,7 @@ tc16_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     const int c_hi = wide_epi ? c_lo + 1 : c_lo + 2;
     const int ew = wide_epi ? c_lo * 4 + quarter : ehalf * 4 + quarter;      // 0..15 | 0..7
     const int row = m0 + quarter * 32 + lane;      // output row owned by this thread (TMEM lane)
-    const bool row_ok = row < p.M;
+    const bool row_ok = row < M;
     // c_row_scale: per-output-row factor (the A planes of that row were scaled by its inverse, e.g. per-row power-of-two
     // scaling of LSTM gate gradients); applied here, before the transpose, where a thread still owns one row
     const float oscale = p.alpha * (p.alpha_dev ? *p.alpha_dev : 1.f) * ((p.c_row_scale && row_ok) ? __ldg(p.c_row_scale + row) : 1.f) /
@@ -548,10 +581,11 @@ tc16_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     float rm = -INFINITY, rs = 0.f, rt = 0.f, rav = -INFINITY, row_lse = 0.f, row_nlse2 = 0.f, row_scale = 0.f;
     int rai = 0x7fffffff, tgt = -1;
     if (p.mode != 0 && row_ok) {
-      const int b = row % p.B, tpos = row / p.B + 1;
+      const int n = p.row_map ? __ldg(p.row_map + row) : row;      // decoder position of this row
+      const int b = n % p.B, tpos = n / p.B + 1;
       if (p.targets) tgt = (int)p.targets[(int64_t)b * p.tgt_stride_b + tpos];
       if (p.mode == 2) {
-        row_lse = p.lse[row];
+        row_lse = p.lse[n];
         row_nlse2 = -row_lse * kLog2e;
         row_scale = (tpos < p.lengths[b]) ? (p.grad_scale ? p.grad_scale[0] : 1.f) / (float)p.B : 0.f;
         tgt -= p.v0;
@@ -630,7 +664,7 @@ tc16_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
           // instruction k writes rows 2k, 2k+1 (lanes 0-15 / 16-31): two full 64-byte segments, no bank conflicts either way
           const uint32_t sc = smem_u + OFF_SCRATCH + ew * (32 * 16 * 4);
           const int r0 = m0 + quarter * 32;
-          const int nr = min(32, p.M - r0);
+          const int nr = min(32, M - r0);
           const bool dead = row_scale == 0.f;
           DVAE_TC16_MARK(tid == 0 && tile == 2, 104);
 #pragma unroll
@@ -660,7 +694,7 @@ tc16_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
               // operand of d_h = P . W); padding rows / columns carry zeros
               // (a tile reaches past the planes' last k-block when N is not a multiple of 128: those chunks do not exist)
               // (nor do the rows of a CTA pair's padding row block)
-              if (p.p_planes_a && col0 + hh * 16 + h8 * 8 < p.p_kb_a * BK && m0 < (p.M + BM - 1) / BM * BM)
+              if (p.p_planes_a && col0 + hh * 16 + h8 * 8 < p.p_kb_a * BK && m0 < (M + BM - 1) / BM * BM)
                 store_plane_chunk(p.p_planes_a, row, col0 + hh * 16 + h8 * 8, p.p_kb_a, v, p.p_scale);
 #pragma unroll
               for (int j = 0; j < 8; ++j) sts32(sc + (lane * 16 + ((h8 * 8 + j) ^ ((lane >> 1) & 15))) * 4, v[j]);
@@ -741,11 +775,11 @@ tc16_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
           __syncwarp();
           const int col = col0 + lane;
           const int r0 = m0 + quarter * 32;
-          const int nr = min(32, p.M - r0);              // valid rows of this warp's 32-row band
+          const int nr = min(32, M - r0);                // valid rows of this warp's 32-row band
           if (col < p.N && nr > 0) {
             const bool split = gridDim.z > 1 || p.atomic_out;
             float badd = 0.f;
-            if (p.mode == 0 && (!split || blockIdx.z == 0)) {
+            if (p.mode == 0 && (!split || bz == 0)) {
               if (p.bias) badd += __ldg(p.bias + col);
               if (p.bias2) badd += __ldg(p.bias2 + col);
             }
@@ -759,6 +793,8 @@ tc16_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
               } else {
                 for (int rr = 0; rr < nr; ++rr) cp[rr * ldc] = chunk_at(rr) + badd;
               }
+            } else if (split && p.row_map) {    // live rows: row k of this GEMM is row row_map[k] of C
+              for (int rr = 0; rr < nr; ++rr) atomicAdd(p.C + (int64_t)__ldg(p.row_map + r0 + rr) * ldc + col, chunk_at(rr) + badd);
             } else if (split) {
               for (int rr = 0; rr < nr; ++rr) atomicAdd(cp + rr * ldc, chunk_at(rr) + badd);   // C pre-scaled by beta
             } else {
@@ -884,9 +920,9 @@ tc16_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
       if (tid == 0 && tile < 4) DBG16(15 + 2 * tile);
     }
     if (p.mode == 1 && row_ok) {      // every epilogue warp set is a separate vocabulary split for the finalize kernel
-      const int64_t sp = wide_epi ? (int64_t)blockIdx.y * 4 + c_lo : (int64_t)blockIdx.y * 2 + ehalf;
-      *reinterpret_cast<float4*>(p.part + (sp * p.M + row) * 4) = make_float4(rm, rs, rt, rav);
-      p.part_idx[sp * p.M + row] = rai;
+      const int64_t sp = wide_epi ? (int64_t)by * 4 + c_lo : (int64_t)by * 2 + ehalf;
+      *reinterpret_cast<float4*>(p.part + (sp * mstride + row) * 4) = make_float4(rm, rs, rt, rav);
+      p.part_idx[sp * mstride + row] = rai;
     }
   }
   tc_fence_before();
@@ -995,7 +1031,7 @@ static int launch(const Params& p_in, dim3 grid, cudaStream_t st) {
   // ~1.3 us latency of a 16 KB fetch against 6 stages, not by L2 -> SM bytes, and the pair runs at the pace of its slower CTA.
   const char* mc_env = getenv("DVAE_TC16_MCAST");
   const bool mcast_on = mc_env && mc_env[0] == '1';
-  if (mcast_on && p.presplit && ceil_div(p.K, BK) <= AS_MAX_KB && grid.z == 1 && grid.x >= 2) {
+  if (mcast_on && p.presplit && ceil_div(p.K, BK) <= AS_MAX_KB && grid.z == 1 && grid.x >= 2 && !p.m_live) {
     p.mcast = 1;
     grid.x = (grid.x + 1) / 2 * 2;
     cudaLaunchConfig_t cfg = {};
@@ -1091,8 +1127,13 @@ int linear(const float* A, int64_t lda, int trans_a, const float* B, int64_t ldb
 // is split once per call (its weights).  c_row_scale: optional per-row output factor (device, [M]).
 int linear_planes(const void* a_planes, const void* b_planes, float* C, int64_t ldc, int M, int N, int K, const float* bias,
                   float beta, int act, float a_scale, float b_scale, const float* c_row_scale, bool c_zeroed, int max_splits,
-                  cudaStream_t st, int b_kb0, int b_kbtot, int max_ctas, int a_kb0, int a_kbtot, const uint32_t* a_amax, int a_amax_n) {
+                  cudaStream_t st, int b_kb0, int b_kbtot, int max_ctas, int a_kb0, int a_kbtot, const uint32_t* a_amax, int a_amax_n,
+                  const int* m_live, const int* row_map, int live_k) {
   DVAE_REQUIRE(a_planes && b_planes && C && M > 0 && N > 0 && K > 0, "tc16 linear_planes: bad argument");
+  // live rows: M (live_k = 0) or K (live_k = 1) is the capacity, the device count is read by the kernel; partial tiles are
+  // accumulated atomically into C, which the caller has cleared (or holds the sum to add to: beta = 1)
+  DVAE_REQUIRE(!m_live || ((beta == 1.f || (beta == 0.f && c_zeroed)) && act == 0 && !bias && !c_row_scale && (live_k || row_map)),
+               "tc16 linear_planes: live rows need a cleared (or accumulated) C, no bias / activation, and a row map for live M");
   Params p = {};
   p.presplit = 1; p.no_astat = 1; p.a_planes = a_planes; p.b_planes = b_planes; p.a_rows = M; p.b_rows = N;
   p.M = M; p.N = N; p.K = K; p.tiles_per_cta = 1; p.C = C; p.ldc = ldc; p.bias = bias; p.beta = beta; p.act = act; p.mode = 0;
@@ -1101,6 +1142,7 @@ int linear_planes(const void* a_planes, const void* b_planes, float* C, int64_t 
   p.b_kb0 = b_kb0; p.b_kbtot = b_kbtot;          // B planes wider than this GEMM's K range (a vocabulary chunk of W_out^T)
   p.a_kb0 = a_kb0; p.a_kbtot = a_kbtot;
   if (a_amax) { p.a_amax = a_amax; p.a_amax_n = a_amax_n; }      // A planes were scaled by 2^(13 - floor(log2 amax)) (weight_planes_kernel)
+  if (m_live) { p.m_live = m_live; p.row_map = row_map; p.live_k = live_k; p.atomic_out = 1; }
   const int tiles = ceil_div(M, BM) * ceil_div(N, BN), nkb = ceil_div(K, BK);
   int splits = 1;
   if (act == 0 && nkb >= 8) {      // same cost model as linear(), with the bulk-copy-fed k-block time
@@ -1138,9 +1180,11 @@ int linear_planes(const void* a_planes, const void* b_planes, float* C, int64_t 
 int ce_partials(const float* h, int64_t ldh, int N, int B, int H, int V, const float* w, const float* bias,
                 const int64_t* targets, int64_t tgt_stride_b, const int64_t* lengths, int tiles_per_split, int nsplit,
                 float* part, int* part_idx, const uint64_t* gumbel_seed, uint32_t gumbel_salt, const void* h_planes,
-                const void* w_planes, const int* skip_flag, cudaStream_t st) {
+                const void* w_planes, const int* skip_flag, cudaStream_t st, const int* m_live, const int* row_map) {
   Params p = {};
   p.skip_flag = skip_flag;
+  DVAE_REQUIRE(!m_live || (h_planes && w_planes && !gumbel_seed), "tc16 ce_partials: live rows need pre-split operands");
+  p.m_live = m_live; p.row_map = row_map;
   if (h_planes && w_planes) { p.presplit = 1; p.a_planes = h_planes; p.b_planes = w_planes; p.a_rows = N; p.b_rows = V; }
   p.A = h; p.lda = ldh; p.Bm = w; p.ldb = H;
   p.M = N; p.N = V; p.K = H; p.tiles_per_cta = tiles_per_split; p.bias = bias; p.mode = 1;
@@ -1156,8 +1200,10 @@ int softmax_grad(const float* h, int64_t ldh, int N, int B, int H, int V, int v0
                  const int64_t* targets, int64_t tgt_stride_b, const int64_t* lengths, const float* lse,
                  const float* grad_scale, float* P, int64_t ldp, const void* h_planes, const void* w_planes, float* zero_buf,
                  int64_t zero_n4, float* zero_buf2, int64_t zero2_n4, cudaStream_t st, void* p_planes_a, void* p_planes_t,
-                 float* p_colsum, float p_scale) {
+                 float* p_colsum, float p_scale, const int* m_live, const int* row_map) {
   Params p = {};
+  DVAE_REQUIRE(!m_live || (p_planes_a && p_planes_t && h_planes && w_planes), "tc16 softmax_grad: live rows need the planes output");
+  p.m_live = m_live; p.row_map = row_map;
   if (p_planes_a && p_planes_t && h_planes && w_planes) {
     p.p_planes_a = reinterpret_cast<uint8_t*>(p_planes_a); p.p_planes_t = reinterpret_cast<uint8_t*>(p_planes_t);
     p.p_colsum = p_colsum; p.p_scale = p_scale; p.p_kb_a = ceil_div(vc, BK); p.p_kb_t = ceil_div(N, BK);

@@ -42,9 +42,24 @@ struct Params {
   uint8_t* p_planes_a; uint8_t* p_planes_t; float* p_colsum; float p_scale; int p_kb_a, p_kb_t;
   const int* skip_flag;      // optional device flag: non-zero = the whole launch is a no-op (sampled decoding: a step whose
                              // input is teacher-forced needs no vocabulary sample; decided on the device so one CUDA graph serves every step)
+  // live rows (decoder positions the loss keeps; see dvae_vocab_ce_fwd_live): with m_live set, the extent that runs over
+  // decoder positions comes from device memory -- M (modes 1 / 2, and mode 0 with live_k = 0) or K (mode 0, live_k = 1) --
+  // and the launched CTAs are re-partitioned over the live work (live_split); row_map[k] = position of live row k (modes 1 / 2:
+  // targets / lse lookups; mode 0 with live_k = 0: output row k is accumulated into C row row_map[k])
+  const int* m_live; const int* row_map; int live_k;
   int dbg_skip_epilogue;     // probes only (DVAE_TC_SKIP_EPILOGUE=1): accumulators are released unread
   unsigned long long* dbg;   // optional: pipeline milestone timestamps (ns) of CTA (0,0,0), profiles/probes/tc16_timeline.py
 };
+
+// Vocabulary kernels over live rows: `ctas` launched CTAs, `row_tiles` live 128-row tiles, `col_tiles` vocabulary tiles ->
+// vocabulary groups (CTAs per row tile) and tiles per CTA, by the one-wave rule of the full-N launches (ce_nsplit)
+__host__ __device__ inline void live_split(int row_tiles, int ctas, int col_tiles, int* tiles_per_cta, int* groups) {
+  int g = row_tiles > 0 ? ctas / row_tiles : 1;
+  g = g < 1 ? 1 : (g > col_tiles ? col_tiles : g);
+  const int tpc = (col_tiles + g - 1) / g;
+  *tiles_per_cta = tpc;
+  *groups = (col_tiles + tpc - 1) / tpc;
+}
 
 bool enabled();     // DVAE_GEMM_IMPL=f16
 bool shape_ok(const float* A, int64_t lda, int trans_a, const float* B, int64_t ldb, int trans_b, int M, int N, int K);
@@ -55,11 +70,13 @@ int linear(const float* A, int64_t lda, int trans_a, const float* B, int64_t ldb
 // plane_floats: size of BOTH planes in floats.  Operands that many tiles re-read (the decoder states and the vocabulary
 // matrix in the vocab-CE kernels) are split once; the GEMM then runs without landing ring and converter warps.
 int64_t plane_floats(int R, int K);
+bool single_acc_planes(int K);      // planes of K-deep operands use the single-accumulator convention (tc_planes.cuh)
 int split_planes(const float* X, int64_t ld, int R, int K, float scale, void* planes, cudaStream_t st, bool force_dual = false);
 int linear_planes(const void* a_planes, const void* b_planes, float* C, int64_t ldc, int M, int N, int K, const float* bias,
                   float beta, int act, float a_scale, float b_scale, const float* c_row_scale, bool c_zeroed, int max_splits,
                   cudaStream_t st, int b_kb0 = 0, int b_kbtot = 0, int max_ctas = 0, int a_kb0 = 0, int a_kbtot = 0,
-                  const uint32_t* a_amax = nullptr, int a_amax_n = 1);
+                  const uint32_t* a_amax = nullptr, int a_amax_n = 1, const int* m_live = nullptr, const int* row_map = nullptr,
+                  int live_k = 0);
 // Weight-plane registry (api.cu): GEMMs whose B operand is a registered weight matrix (or a 128-row / 32-column aligned
 // block of it) fetch B as pre-split planes by bulk copy; only A goes through the converter warps.
 constexpr int kMaxPlaneEntries = 24;
@@ -77,12 +94,14 @@ bool presplit_enabled();      // DVAE_VOCAB_PRESPLIT=0 disables
 int ce_partials(const float* h, int64_t ldh, int N, int B, int H, int V, const float* w, const float* bias,
                 const int64_t* targets, int64_t tgt_stride_b, const int64_t* lengths, int tiles_per_split, int nsplit,
                 float* part, int* part_idx, const uint64_t* gumbel_seed, uint32_t gumbel_salt, const void* h_planes,
-                const void* w_planes, const int* skip_flag, cudaStream_t st);
+                const void* w_planes, const int* skip_flag, cudaStream_t st, const int* m_live = nullptr,
+                const int* row_map = nullptr);
 int softmax_grad(const float* h, int64_t ldh, int N, int B, int H, int V, int v0, int vc, const float* w, const float* bias,
                  const int64_t* targets, int64_t tgt_stride_b, const int64_t* lengths, const float* lse,
                  const float* grad_scale, float* P, int64_t ldp, const void* h_planes, const void* w_planes, float* zero_buf,
                  int64_t zero_n4, float* zero_buf2, int64_t zero2_n4, cudaStream_t st, void* p_planes_a = nullptr,
-                 void* p_planes_t = nullptr, float* p_colsum = nullptr, float p_scale = 1.f);
+                 void* p_planes_t = nullptr, float* p_colsum = nullptr, float p_scale = 1.f, const int* m_live = nullptr,
+                 const int* row_map = nullptr);
 
 }  // namespace tc16
 }  // namespace dvae

@@ -16,6 +16,7 @@ namespace tc16 {
 constexpr int kPlaneRows = 128, kPlaneK = 32;
 constexpr int kPlaneBytes = kPlaneRows * kPlaneK * 2, kPlaneTileBytes = 2 * kPlaneBytes;      // 8 KB per plane, 16 KB per [hi | lo] tile
 constexpr float kPlaneLoScale = 2048.f;
+constexpr float kSingleScale = 256.f;                    // operand scale of the single-accumulator planes
 
 // (x0, x1) * s -> packed fp16 hi pair (returned) and lo pair; packed fp32 arithmetic (FMUL2 / FFMA2)
 __device__ __forceinline__ uint32_t pack_hi_lo(float x0, float x1, float s, uint32_t& lo, float ls = kPlaneLoScale) {

@@ -11,6 +11,7 @@
 
 #include "gemm_simt.cuh"
 #include "tc_gemm16.cuh"
+#include "tc_planes.cuh"
 
 namespace dvae {
 
@@ -35,11 +36,15 @@ struct CeArgs {
   const int64_t* lengths;
   int N, B, H, V, sos;
   int tiles_per_split, nsplit;
-  float* part;      // [nsplit][N][4]: max, sumexp, target logit, argmax value
-  int* part_idx;    // [nsplit][N]
+  float* part;      // [nsplit][R][4]: max, sumexp, target logit, argmax value; R = N, or (live rows) rt * 128 for rt live
+                    // row tiles, inside a capacity of N rounded up to whole row tiles (part_rows)
+  int* part_idx;    // [nsplit][R]
   const uint64_t* gumbel_seed; uint32_t gumbel_salt;   // sampling: arg-max over logits + Gumbel noise
   const void* h_planes; const void* w_planes;          // optional pre-split fp16 operand planes (tc16::split_planes)
   const int* skip_flag;                                // optional device flag: non-zero = no-op (see tc16::Params::skip_flag)
+  // live rows (dvae_vocab_ce_fwd_live): the partials cover the *m_live rows of the row list `rows` only, in the layout
+  // tc16_gemm_kernel chose on the device for `live_ctas` launched CTAs (tc16::live_split)
+  const int* m_live; const int* rows; int live_ctas;
 };
 
 __device__ __forceinline__ void merge_ms(float& m, float& s, float m2, float s2) {
@@ -143,15 +148,27 @@ __global__ void __launch_bounds__(kFinThreads) vocab_ce_finalize_kernel(CeArgs p
   __shared__ float red[kFinThreads / 32];
   const int sub = threadIdx.x % kFinLanes, slot = threadIdx.x / kFinLanes;
   constexpr int kRows = kFinThreads / kFinLanes;
+  // rows of the partials: every decoder position, or (live rows) the *m_live entries of the row list, in the split count and
+  // row stride the partials kernel derived from the same count
+  int rows = p.N, nsplit = p.nsplit;
+  int64_t stride = p.N;
+  if (p.m_live) {
+    rows = *p.m_live;
+    const int rt = (rows + GCE::BM - 1) / GCE::BM;
+    int tpc, groups;
+    tc16::live_split(rt, p.live_ctas, (p.V + GCE::BN - 1) / GCE::BN, &tpc, &groups);
+    nsplit = 4 * groups;      // pre-split operands: four epilogue warp sets per CTA, each a split of its own
+    stride = (int64_t)rt * GCE::BM;
+  }
   float local = 0.f;
-  for (int n0 = blockIdx.x * kRows; n0 < p.N; n0 += gridDim.x * kRows) {      // block-uniform trip count (shuffles below)
-    const int n = n0 + slot;
+  for (int k0 = blockIdx.x * kRows; k0 < rows; k0 += gridDim.x * kRows) {      // block-uniform trip count (shuffles below)
+    const int k = k0 + slot;
     float m = -INFINITY, s = 0.f, t = 0.f, av = -INFINITY;
     int ai = 0x7fffffff;
-    if (n < p.N) {
-      for (int sp = sub; sp < p.nsplit; sp += kFinLanes) {
-        float4 q = *reinterpret_cast<const float4*>(p.part + ((int64_t)sp * p.N + n) * 4);
-        int qi = p.part_idx[(int64_t)sp * p.N + n];
+    if (k < rows) {
+      for (int sp = sub; sp < nsplit; sp += kFinLanes) {
+        float4 q = *reinterpret_cast<const float4*>(p.part + ((int64_t)sp * stride + k) * 4);
+        int qi = p.part_idx[(int64_t)sp * stride + k];
         merge_ms(m, s, q.x, q.y);
         t += q.z;
         if (q.w > av || (q.w == av && qi < ai)) { av = q.w; ai = qi; }
@@ -166,7 +183,8 @@ __global__ void __launch_bounds__(kFinThreads) vocab_ce_finalize_kernel(CeArgs p
       t += t2;
       if (av2 > av || (av2 == av && ai2 < ai)) { av = av2; ai = ai2; }
     }
-    if (sub == 0 && n < p.N) {
+    if (sub == 0 && k < rows) {
+      const int n = p.rows ? p.rows[k] : k;      // decoder position
       float l = m + logf(s), e = l - t;
       if (lse) lse[n] = l;
       if (nll) nll[n] = e;
@@ -260,6 +278,10 @@ __global__ void __launch_bounds__(GCE::NT) vocab_p_kernel(PArgs p) {
   }
 }
 
+// row capacity of each split's partials: N, or -- live rows, where the kernel re-partitions its CTAs on the device -- whole row
+// tiles (groups x live row tiles <= launched CTAs, so [4 x launched splits][row tiles x 128] holds every layout it can pick)
+static int64_t part_rows(const CeArgs& p) { return p.m_live ? (int64_t)ceil_div(p.N, GCE::BM) * GCE::BM : p.N; }
+
 // per-(row, vocabulary split) partials: tensor-core kernel when the shape allows, fp32 SIMT otherwise
 // On return p.nsplit / p.part_idx describe the partials that were actually written (the fp16-split kernel's two
 // -- four with pre-split operands -- epilogue warp sets each emit their own split).
@@ -267,10 +289,11 @@ static int ce_partials(CeArgs& p, cudaStream_t st) {
   if (!force_simt_gemm() && p.N >= 64 && p.V >= 128 && p.H >= 32 && tc16::supported(p.h, p.ldh, 0, p.w, p.H, 0, p.N, p.V, p.H)) {
     const int launched = p.nsplit;
     p.nsplit = (p.h_planes && p.w_planes ? 4 : 2) * launched;      // pre-split operands: 16 epilogue warps, 4 column chunks
-    p.part_idx = reinterpret_cast<int*>(p.part + (int64_t)p.nsplit * p.N * 4);
+    p.part_idx = reinterpret_cast<int*>(p.part + (int64_t)p.nsplit * part_rows(p) * 4);
+    if (p.m_live) p.live_ctas = ceil_div(p.N, GCE::BM) * launched;
     return tc16::ce_partials(p.h, p.ldh, p.N, p.B, p.H, p.V, p.w, p.bias, p.targets, p.tgt_stride_b, p.lengths,
                              p.tiles_per_split, launched, p.part, p.part_idx, p.gumbel_seed, p.gumbel_salt, p.h_planes,
-                             p.w_planes, p.skip_flag, st);
+                             p.w_planes, p.skip_flag, st, p.m_live, p.rows);
   }
   if (!force_simt_gemm() && p.N >= 64 && p.V >= 128 && p.H >= 32 && tc::tc_linear_supported(p.h, p.ldh, p.w, p.H, p.N, p.V, p.H))
     return tc::tc_ce_partials(p.h, p.ldh, p.N, p.B, p.H, p.V, p.w, p.bias, p.targets, p.tgt_stride_b, p.lengths,
@@ -324,24 +347,112 @@ static int p_chunk_planes(int N, int V) {
   const int64_t nc = (vr + vmax - 1) / vmax;
   return (int)(((V + nc - 1) / nc + 127) / 128 * 128);
 }
+static bool tplanes_enabled() {      // DVAE_VOCAB_TPLANES=0: the gradient GEMMs convert W_out^T / h^T in every CTA
+  const char* e = getenv("DVAE_VOCAB_TPLANES");
+  return !(e && e[0] == '0');
+}
 static bool p_planes_enabled() {
   const char* e = getenv("DVAE_VOCAB_PPLANES");
   return !(e && e[0] == '0');
+}
+
+
+// ---- live rows: the decoder positions the loss keeps ----------------------------------------------------------------
+// Position n = t * B + b (row t + 1 of the targets) enters the loss only when t + 1 < len_b: its loss weight is zero and its
+// softmax gradient exactly zero otherwise.  The live-row path runs the vocabulary GEMMs over the live rows only, in
+// ascending n (so the loss sums in a fixed order), with the count M known on the device only: launch grids stay sized for
+// every position and tc16_gemm_kernel re-partitions its CTAs from *m_live, so one captured graph serves every length mix.
+
+// rows[k] = position of live row k (ascending), *m_live = M.  One CTA of up to 1024 threads: per position t, a ballot over
+// the batch ranks each live b among those before it.
+__global__ void __launch_bounds__(1024) vocab_live_rows_kernel(const int64_t* __restrict__ lengths, int T1, int B, int* __restrict__ rows,
+                                                               int* __restrict__ m_live) {
+  __shared__ int wcnt[32];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = blockDim.x >> 5;
+  int base = 0;
+  for (int t = 0; t < T1; ++t) {
+    for (int b0 = 0; b0 < B; b0 += blockDim.x) {
+      const int b = b0 + threadIdx.x;
+      const bool live = b < B && t + 1 < lengths[b];
+      const unsigned bal = __ballot_sync(0xffffffffu, live);
+      if (lane == 0) wcnt[w] = __popc(bal);
+      __syncthreads();
+      int before = 0, total = 0;
+      for (int i = 0; i < nw; ++i) {
+        const int c = wcnt[i];
+        before += i < w ? c : 0;
+        total += c;
+      }
+      __syncthreads();      // wcnt is rewritten by the next round
+      if (live) rows[base + before + __popc(bal & ((1u << lane) - 1))] = t * B + b;
+      base += total;
+    }
+  }
+  if (threadIdx.x == 0) *m_live = base;
+}
+
+// The live rows of h [N, H] (row stride H) as operand planes, rows in row-list order:
+//   a_planes: the A operand of the forward / softmax-gradient GEMMs, [M rows, K = H] (scale / lo_scale: the convention of
+//             tc16::split_planes for K = H);
+//   t_planes: the B operand of d_w = P^T . h, [H rows, K = positions], dual-accumulator convention (weight_planes_kernel),
+//             k-blocks per row block for all N positions.
+// Rows M .. the next 128-row tile of a_planes and positions M .. the next 32-position k-block of t_planes are written as
+// zeros: the GEMMs read them (multiplied by zeros of P, which would not clear a stale NaN).
+__global__ void __launch_bounds__(256) vocab_live_gather_kernel(const float* __restrict__ h, int N, int H, const int* __restrict__ rows,
+                                                                const int* __restrict__ m_live, float a_scale, float a_lo_scale,
+                                                                uint8_t* __restrict__ a_planes, uint8_t* __restrict__ t_planes) {
+  const int M = *m_live;
+  const int KB = (H + 31) / 32, KC = KB * 4;
+  const int64_t na = (int64_t)((M + 127) / 128) * 128 * KC;
+  const int HP = (H + 127) / 128 * 128, KBt = (N + 31) / 32;
+  const int64_t nt = (int64_t)HP * ((M + 31) / 32 * 4);
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < na + nt; i += (int64_t)gridDim.x * blockDim.x) {
+    float v[8];
+    if (i < na) {
+      const int kc = (int)(i % KC), r = (int)(i / KC);
+      if (r < M && kc * 8 + 8 <= H) {
+        const float4* src = reinterpret_cast<const float4*>(h + (int64_t)__ldg(rows + r) * H + kc * 8);
+        const float4 x0 = __ldg(src), x1 = __ldg(src + 1);
+        v[0] = x0.x; v[1] = x0.y; v[2] = x0.z; v[3] = x0.w; v[4] = x1.x; v[5] = x1.y; v[6] = x1.z; v[7] = x1.w;
+      } else {
+#pragma unroll
+        for (int e = 0; e < 8; ++e) v[e] = 0.f;
+      }
+      uint4 hi, lo;
+      hi.x = tc16::pack_hi_lo(v[0], v[1], a_scale, lo.x, a_lo_scale); hi.y = tc16::pack_hi_lo(v[2], v[3], a_scale, lo.y, a_lo_scale);
+      hi.z = tc16::pack_hi_lo(v[4], v[5], a_scale, lo.z, a_lo_scale); hi.w = tc16::pack_hi_lo(v[6], v[7], a_scale, lo.w, a_lo_scale);
+      const int64_t off = tc16::plane_chunk_offset(r, kc * 8, KB);
+      *reinterpret_cast<uint4*>(a_planes + off) = hi;
+      *reinterpret_cast<uint4*>(a_planes + off + tc16::kPlaneBytes) = lo;
+    } else {
+      // consecutive threads: consecutive hidden units, so each of the 8 loads is a coalesced segment of one row of h
+      const int64_t j = i - na;
+      const int r = (int)(j % HP), k0 = (int)(j / HP) * 8;
+#pragma unroll
+      for (int e = 0; e < 8; ++e) v[e] = (r < H && k0 + e < M) ? __ldg(h + (int64_t)__ldg(rows + k0 + e) * H + r) : 0.f;
+      tc16::store_plane_chunk(t_planes, r, k0, KBt, v, 1.f);
+    }
+  }
 }
 
 }  // namespace dvae
 
 using namespace dvae;
 
-// workspace layout (floats): [partials 4*ns*N*5 + 8][block sums][pad to 4][operand planes of h and w]
+// workspace layout (floats): [partials 4*ns*N'*5 + 8][block sums][pad to 4][operand planes of h and w]
+//   [live rows: planes of h^T (B operand of d_w) | row list (N ints) | live count (1 int) | pad]      (N' = N in whole row tiles)
 static int64_t ce_part_floats(int N, int V) {
   int tps;
   int ns = ce_nsplit(N, V, &tps);
-  return (4LL * ns * N * 5 + 8 + kFinMaxBlocks + 3) / 4 * 4;    // x4: the fp16-split kernel writes up to four partials per (row, split)
+  const int64_t rows = (int64_t)ceil_div(N, GCE::BM) * GCE::BM;
+  return (4LL * ns * rows * 5 + 8 + kFinMaxBlocks + 3) / 4 * 4;    // x4: the fp16-split kernel writes up to four partials per (row, split)
 }
+static int64_t live_off(int N, int V, int H) { return ce_part_floats(N, V) + tc16::plane_floats(N, H) + tc16::plane_floats(V, H); }
 extern "C" int64_t dvae_vocab_ce_ws_floats(int N, int V, int H) {
-  return ce_part_floats(N, V) + tc16::plane_floats(N, H) + tc16::plane_floats(V, H);
+  return live_off(N, V, H) + tc16::plane_floats(H, N) + (N + 8 + 3) / 4 * 4;
 }
+// float offset of the row list in the forward workspace (the live count follows its N entries)
+extern "C" int64_t dvae_vocab_live_rows_at(int N, int V, int H) { return live_off(N, V, H) + tc16::plane_floats(H, N); }
 
 // (ws, w) of the last dvae_vocab_split_w call that actually wrote W planes on this host thread
 static thread_local const void* g_wsplit_ws = nullptr;
@@ -361,14 +472,20 @@ extern "C" int dvae_vocab_split_w(const float* w, int N, int V, int H, float* ws
   return DVAE_OK;
 }
 
+// the live-row path runs on the pre-split kernels with the softmax gradient as operand planes; other shapes run every row
+static bool live_ok(int N, int V, int H, const float* h, int64_t ldh, const float* w) {
+  return use_tc16(N, V, H, h, ldh, w) && use_presplit(N, V, H) && ldh == H && (reinterpret_cast<uintptr_t>(h) & 15) == 0 &&
+         (reinterpret_cast<uintptr_t>(w) & 15) == 0 && p_planes_enabled() && tplanes_enabled();
+}
+
 static int vocab_ce_fwd_impl(const float* h, int64_t ldh, int T1, int B, int H, int V, const float* w,
                              const float* bias, const int64_t* targets, int64_t tgt_stride_b,
                              const int64_t* lengths, int sos, float* lse, float* nll, int32_t* argmax,
-                             float* loss, float* ws, bool w_planes_ready, void* stream) {
+                             float* loss, float* ws, bool w_planes_ready, bool live, void* stream) {
   cudaStream_t st = (cudaStream_t)stream;
   DVAE_REQUIRE(h && w && bias && targets && lengths && loss && ws, "dvae_vocab_ce_fwd: null pointer");
   DVAE_REQUIRE(T1 > 0 && B > 0 && H > 0 && V > 0, "dvae_vocab_ce_fwd: bad shape T1=%d B=%d H=%d V=%d", T1, B, H, V);
-  CeArgs p;
+  CeArgs p = {};
   p.h = h; p.ldh = ldh; p.w = w; p.bias = bias; p.targets = targets; p.tgt_stride_b = tgt_stride_b;
   p.lengths = lengths; p.N = T1 * B; p.B = B; p.H = H; p.V = V; p.sos = sos;
   p.nsplit = ce_nsplit(p.N, V, &p.tiles_per_split);
@@ -381,7 +498,24 @@ static int vocab_ce_fwd_impl(const float* h, int64_t ldh, int T1, int B, int H, 
     float* hp = ws + ce_part_floats(p.N, V);
     float* wp = hp + tc16::plane_floats(p.N, H);
     int rc;
-    if ((rc = tc16::split_planes(h, ldh, p.N, H, 1.f, hp, st))) return rc;
+    if (live && live_ok(p.N, V, H, h, ldh, w)) {
+      // live rows: the row list, then the live rows of h as the A planes here and as the h^T planes of the backward's d_w
+      float* tp = ws + live_off(p.N, V, H);
+      int* rows = reinterpret_cast<int*>(tp + tc16::plane_floats(H, p.N));
+      const int nthr = min(1024, ceil_div(B, 32) * 32);
+      vocab_live_rows_kernel<<<1, nthr, 0, st>>>(lengths, T1, B, rows, rows + p.N);
+      DVAE_LAUNCH_CHECK();
+      const bool single = tc16::single_acc_planes(H);
+      const int64_t items = (tc16::plane_floats(p.N, H) + tc16::plane_floats(H, p.N)) / 16;
+      const int blocks = ceil_div(items, 256) < 148 * 4 ? ceil_div(items, 256) : 148 * 4;
+      vocab_live_gather_kernel<<<blocks, 256, 0, st>>>(h, p.N, H, rows, rows + p.N, single ? tc16::kSingleScale : 1.f,
+                                                       single ? 1.f : tc16::kPlaneLoScale, reinterpret_cast<uint8_t*>(hp),
+                                                       reinterpret_cast<uint8_t*>(tp));
+      DVAE_LAUNCH_CHECK();
+      p.rows = rows; p.m_live = rows + p.N;
+    } else if ((rc = tc16::split_planes(h, ldh, p.N, H, 1.f, hp, st))) {
+      return rc;
+    }
     // W planes: skipped when the caller vouches for an earlier dvae_vocab_split_w on the same (ws, w) since the last
     // weight update, and that call did write them
     if (!(w_planes_ready && g_wsplit_ws == ws && g_wsplit_w == w) && (rc = tc16::split_planes(w, H, V, H, 1.f, wp, st))) return rc;
@@ -389,7 +523,7 @@ static int vocab_ce_fwd_impl(const float* h, int64_t ldh, int T1, int B, int H, 
   }
   g_wsplit_ws = g_wsplit_w = nullptr;
   { int rc = ce_partials(p, st); if (rc) return rc; }
-  float* block_sums = ws + (int64_t)p.nsplit * p.N * 5 + 8;      // p.nsplit: as updated by ce_partials
+  float* block_sums = ws + (int64_t)p.nsplit * part_rows(p) * 5 + 8;      // p.nsplit: as updated by ce_partials
   const int nblk = min(kFinMaxBlocks, ceil_div(p.N, kFinThreads / kFinLanes));
   vocab_ce_finalize_kernel<<<nblk, kFinThreads, 0, st>>>(p, lse, nll, argmax, block_sums);
   DVAE_LAUNCH_CHECK();
@@ -403,7 +537,7 @@ extern "C" int dvae_vocab_ce_fwd(const float* h, int64_t ldh, int T1, int B, int
                                  const int64_t* lengths, int sos, float* lse, float* nll, int32_t* argmax,
                                  float* loss, float* ws, void* stream) {
   return vocab_ce_fwd_impl(h, ldh, T1, B, H, V, w, bias, targets, tgt_stride_b, lengths, sos, lse, nll, argmax, loss, ws,
-                           false, stream);
+                           false, false, stream);
 }
 
 // flags bit 0: the W planes in ws are current (dvae_vocab_split_w on the same ws / w since the last weight update)
@@ -412,7 +546,18 @@ extern "C" int dvae_vocab_ce_fwd_ex(const float* h, int64_t ldh, int T1, int B, 
                                     const int64_t* lengths, int sos, float* lse, float* nll, int32_t* argmax,
                                     float* loss, float* ws, int flags, void* stream) {
   return vocab_ce_fwd_impl(h, ldh, T1, B, H, V, w, bias, targets, tgt_stride_b, lengths, sos, lse, nll, argmax, loss, ws,
-                           (flags & 1) != 0, stream);
+                           (flags & 1) != 0, false, stream);
+}
+
+// dvae_vocab_ce_fwd_ex over the live rows only (positions t + 1 < len_b): lse / nll / argmax are written at live positions
+// only, the loss is the same masked average.  ws keeps the row list, the live count and the h^T planes for
+// dvae_vocab_ce_bwd_live.
+extern "C" int dvae_vocab_ce_fwd_live(const float* h, int64_t ldh, int T1, int B, int H, int V, const float* w,
+                                      const float* bias, const int64_t* targets, int64_t tgt_stride_b,
+                                      const int64_t* lengths, int sos, float* lse, float* nll, int32_t* argmax,
+                                      float* loss, float* ws, int flags, void* stream) {
+  return vocab_ce_fwd_impl(h, ldh, T1, B, H, V, w, bias, targets, tgt_stride_b, lengths, sos, lse, nll, argmax, loss, ws,
+                           (flags & 1) != 0, true, stream);
 }
 
 // softmax-gradient chunks alternate between two buffers when there is more than one chunk: the next chunk's P is then
@@ -432,6 +577,67 @@ static int64_t p_region_floats(int N, int V) {
 extern "C" int64_t dvae_vocab_ce_bwd_ws_floats(int N, int V, int H) {
   return p_region_floats(N, V) / 4 * 4 + tc16::plane_floats(N, H) + tc16::plane_floats(V, H) + tc16::plane_floats(H, V) +
          tc16::plane_floats(H, N);
+}
+
+// d_w GEMM CTA cap, A/B knob (measured: capping this one costs 17 us -- it outlasts the recurrence it runs beside)
+static int dw_max_ctas() {
+  static const int cap = [] { const char* e = getenv("DVAE_VOCAB_DW_MAX_CTAS"); return e ? atoi(e) : 0; }();
+  return cap;
+}
+
+// planes of W_out^T [H, V] (B operand of d_h = P . W): registered by the caller, or added to `tab` to be split into tp
+static const void* wT_planes_of(const float* w, int H, int V, float* tp, tc16::PlaneTable& tab, int* kbtot) {
+  tc16::PlaneHit hit;
+  if (tc16::find_weight_planes(w, H, 1, H, V, &hit) && hit.tile0 == 0 && hit.kb0 == 0) {
+    *kbtot = hit.kbtot;
+    return hit.planes;
+  }
+  tab.e[tab.n++] = tc16::PlaneTable::Entry{w, V, H, nullptr, tp};
+  *kbtot = ceil_div(V, 32);
+  return tp;
+}
+
+// The vocabulary backward with every operand as planes: per vocabulary chunk, the softmax-gradient kernel writes P as planes
+// in both orientations (and adds the bias gradient), then d_h (+)= P . W and d_w = P^T . h, both bulk-copy fed.
+// m_live / rows (live rows, see dvae_vocab_ce_bwd_live): P covers the live rows only, row k of d_h's GEMM is added into row
+// rows[k] and d_w's K runs over the live positions; both GEMMs then accumulate into outputs cleared beforehand.
+static int planes_bwd(const float* h, int64_t ldh, int N, int B, int H, int V, const float* w, const float* bias,
+                      const int64_t* targets, int64_t tgt_stride_b, const int64_t* lengths, const float* lse,
+                      const float* grad_scale_dev, float* d_h, int64_t lddh, float* d_w, float* d_bias, const void* h_planes,
+                      const void* w_planes, const void* wT_planes, int wT_kbtot, const void* hT_planes, float a_scale, float* ws,
+                      const int* m_live, const int* rows, cudaStream_t st) {
+  const int vc_max = p_chunk_planes(N, V), nbuf = p_buffers_planes(N, V);
+  const int64_t pa_fl = tc16::plane_floats(N, vc_max), pt_fl = tc16::plane_floats(vc_max, N);
+  DVAE_CUDA(cudaMemsetAsync(d_bias, 0, sizeof(float) * V, st));
+  int chunk = 0;
+  const int nchunks = ceil_div(V, vc_max);
+  for (int v0 = 0; v0 < V; v0 += vc_max, ++chunk) {
+    const int vc = min(vc_max, V - v0);
+    float* pa = ws + (int64_t)(chunk % nbuf) * (pa_fl + pt_fl);
+    float* pt = pa + pa_fl;
+    float* dw = d_w + (int64_t)v0 * H;
+    // the softmax-gradient kernel clears d_h (once, all N rows) and this chunk's rows of d_w when they are aligned; the live-row
+    // GEMMs accumulate in any case, so there a memset clears what the kernel cannot
+    const bool zh = chunk == 0 && lddh == H && (((uintptr_t)d_h) & 15) == 0 && ((int64_t)N * H) % 4 == 0;
+    const bool zw = (((uintptr_t)dw) & 15) == 0 && ((int64_t)vc * H) % 4 == 0;
+    if (m_live && chunk == 0 && !zh) DVAE_CUDA(cudaMemsetAsync(d_h, 0, sizeof(float) * (size_t)N * H, st));      // lddh == H
+    if (m_live && !zw) DVAE_CUDA(cudaMemsetAsync(dw, 0, sizeof(float) * (size_t)vc * H, st));
+    int rc;
+    if ((rc = tc16::softmax_grad(h, ldh, N, B, H, V, v0, vc, w, bias, targets, tgt_stride_b, lengths, lse, grad_scale_dev, nullptr,
+                                 vc_max, h_planes, w_planes, zh ? d_h : nullptr, (int64_t)N * H / 4, zw ? dw : nullptr,
+                                 (int64_t)vc * H / 4, st, pa, pt, d_bias + v0, a_scale, m_live, rows))) return rc;
+    Fork fork(st);
+    // d_h [N,H] (+)= P [N,vc] . W[v0:v0+vc, :]: A = P planes, B = planes of W_out^T, k-blocks v0/32 .. of its K = V axis
+    if ((rc = tc16::linear_planes(pa, wT_planes, d_h, lddh, N, H, vc, nullptr, chunk ? 1.f : 0.f, 0, a_scale, 1.f, nullptr,
+                                  m_live ? true : zh, 16, st, v0 / 32, wT_kbtot, 0, 0, 0, nullptr, 1, m_live, rows, 0))) return rc;
+    // d_w[v0:v0+vc, :] = P^T [vc,N] . h [N,H]: A = transposed P planes, B = planes of h^T
+    if ((rc = tc16::linear_planes(pt, hT_planes, dw, H, vc, H, N, nullptr, 0.f, 0, a_scale, 1.f, nullptr, m_live ? true : zw, 16,
+                                  fork.side(0), 0, 0, dw_max_ctas(), 0, 0, nullptr, 1, m_live, nullptr, 1))) return rc;
+    // main waits for the side branch only when the NEXT chunk reuses a buffer (or at the end)
+    if (chunk + 1 == nchunks || chunk + 1 >= nbuf)
+      if ((rc = fork.join())) return rc;
+  }
+  return DVAE_OK;
 }
 
 extern "C" int dvae_vocab_ce_bwd(const float* h, int64_t ldh, int T1, int B, int H, int V, const float* w,
@@ -472,18 +678,11 @@ extern "C" int dvae_vocab_ce_bwd(const float* h, int64_t ldh, int T1, int B, int
   // W_out^T [H, V] (registered by the caller, or split here) and h^T [H, N]
   const void *wT_planes = nullptr, *hT_planes = nullptr;
   int wT_kbtot = 0;
-  if (h_planes && H % 32 == 0 && N >= 128 && (reinterpret_cast<uintptr_t>(w) & 15) == 0 && ldh == H &&
-      !(getenv("DVAE_VOCAB_TPLANES") && getenv("DVAE_VOCAB_TPLANES")[0] == '0')) {
+  if (h_planes && H % 32 == 0 && N >= 128 && (reinterpret_cast<uintptr_t>(w) & 15) == 0 && ldh == H && tplanes_enabled()) {
     float* tp = ws + front + tc16::plane_floats(N, H) + tc16::plane_floats(V, H);
-    tc16::PlaneHit hit;
     tc16::PlaneTable tab;
     tab.n = 0;
-    if (tc16::find_weight_planes(w, H, 1, H, V, &hit) && hit.tile0 == 0 && hit.kb0 == 0) {
-      wT_planes = hit.planes; wT_kbtot = hit.kbtot;
-    } else {
-      tab.e[tab.n++] = tc16::PlaneTable::Entry{w, V, H, nullptr, tp};
-      wT_planes = tp; wT_kbtot = ceil_div(V, 32);
-    }
+    wT_planes = wT_planes_of(w, H, V, tp, tab, &wT_kbtot);
     float* hp_t = tp + tc16::plane_floats(H, V);
     tab.e[tab.n++] = tc16::PlaneTable::Entry{h, N, H, nullptr, hp_t};
     hT_planes = hp_t;
@@ -494,12 +693,9 @@ extern "C" int dvae_vocab_ce_bwd(const float* h, int64_t ldh, int T1, int B, int
   // gradient), and the two gradient GEMMs are bulk-copy fed on both operands
   const bool pp = wT_planes && hT_planes && h_planes && w_planes && p_planes_enabled() && lddh % 4 == 0 &&
                   tc16::supported(h, ldh, 0, w, H, 0, N, min(vc_max, V), H);
-  int64_t pa_fl = 0, pt_fl = 0;
-  if (pp) {
-    vc_max = p_chunk_planes(N, V); nbuf = p_buffers_planes(N, V);
-    pa_fl = tc16::plane_floats(N, vc_max); pt_fl = tc16::plane_floats(vc_max, N);
-    DVAE_CUDA(cudaMemsetAsync(d_bias, 0, sizeof(float) * V, st));
-  }
+  if (pp)
+    return planes_bwd(h, ldh, N, B, H, V, w, bias, targets, tgt_stride_b, lengths, lse, grad_scale_dev, d_h, lddh, d_w, d_bias,
+                      h_planes, w_planes, wT_planes, wT_kbtot, hT_planes, ph.a_scale, ws, nullptr, nullptr, st);
   int chunk = 0;
   const int nchunks = ceil_div(V, vc_max);
   for (int v0 = 0; v0 < V; v0 += vc_max, ++chunk) {
@@ -508,26 +704,6 @@ extern "C" int dvae_vocab_ce_bwd(const float* h, int64_t ldh, int T1, int B, int
     p.v0 = v0; p.vc = vc; p.P = Pc;
     int rc;
     bool dh_zeroed = false, dw_zeroed = false;
-    if (pp) {
-      float* pa = ws + (int64_t)(chunk % nbuf) * (pa_fl + pt_fl);
-      float* pt = pa + pa_fl;
-      const bool zh = chunk == 0 && lddh == H && (((uintptr_t)d_h) & 15) == 0 && ((int64_t)N * H) % 4 == 0;
-      const bool zw = (((uintptr_t)(d_w + (int64_t)v0 * H)) & 15) == 0 && ((int64_t)vc * H) % 4 == 0;
-      if ((rc = tc16::softmax_grad(h, ldh, N, B, H, V, v0, vc, w, bias, targets, tgt_stride_b, lengths, lse, grad_scale_dev, nullptr,
-                                   vc_max, h_planes, w_planes, zh ? d_h : nullptr, (int64_t)N * H / 4,
-                                   zw ? d_w + (int64_t)v0 * H : nullptr, (int64_t)vc * H / 4, st, pa, pt, d_bias + v0, ph.a_scale))) return rc;
-      Fork fork(st);
-      // d_h [N,H] (+)= P [N,vc] . W[v0:v0+vc, :]: A = P planes, B = planes of W_out^T, k-blocks v0/32 .. of its K = V axis
-      if ((rc = tc16::linear_planes(pa, wT_planes, d_h, lddh, N, H, vc, nullptr, chunk ? 1.f : 0.f, 0, ph.a_scale, 1.f, nullptr, zh, 16, st,
-                                    v0 / 32, wT_kbtot))) return rc;
-      // d_w[v0:v0+vc, :] = P^T [vc,N] . h [N,H]: A = transposed P planes, B = planes of h^T
-      static const int dw_cap = [] { const char* e = getenv("DVAE_VOCAB_DW_MAX_CTAS"); return e ? atoi(e) : 0; }();      // measured: capping this one costs 17 us (it outlasts the recurrence it runs beside)
-      if ((rc = tc16::linear_planes(pt, hT_planes, d_w + (int64_t)v0 * H, H, vc, H, N, nullptr, 0.f, 0, ph.a_scale, 1.f, nullptr, zw, 16,
-                                    fork.side(0), 0, 0, dw_cap))) return rc;
-      if (chunk + 1 == nchunks || chunk + 1 >= nbuf)
-        if ((rc = fork.join())) return rc;
-      continue;
-    }
     if (!force_simt_gemm() && N >= 64 && vc >= 128 && H >= 32 && tc16::supported(h, ldh, 0, w, H, 0, N, vc, H)) {
       // the kernel also clears the outputs of this chunk's split-K GEMMs (d_h once, this chunk's rows of d_w): no memset nodes
       const bool zh = chunk == 0 && lddh == H && (((uintptr_t)d_h) & 15) == 0 && ((int64_t)N * H) % 4 == 0;
@@ -563,6 +739,41 @@ extern "C" int dvae_vocab_ce_bwd(const float* h, int64_t ldh, int T1, int B, int
   return DVAE_OK;
 }
 
+// dvae_vocab_ce_bwd over the live rows of the dvae_vocab_ce_fwd_live call whose workspace is fwd_ws (same h, w, lengths,
+// untouched since): the softmax gradient of the live rows only, as operand planes in both orientations; d_h = P . W with its
+// row k accumulated into row rows[k] of d_h (every other row of d_h is zero) and d_w = P^T . h over the live positions.
+// Shapes the live-row forward does not take were run over every row there, and are here too.
+extern "C" int dvae_vocab_ce_bwd_live(const float* h, int64_t ldh, int T1, int B, int H, int V, const float* w,
+                                      const float* bias, const int64_t* targets, int64_t tgt_stride_b,
+                                      const int64_t* lengths, const float* lse, const float* grad_scale_dev,
+                                      float* d_h, int64_t lddh, float* d_w, float* d_bias, const float* fwd_ws, float* ws,
+                                      void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  DVAE_REQUIRE(h && w && bias && targets && lengths && lse && d_h && d_w && d_bias && ws && fwd_ws, "dvae_vocab_ce_bwd_live: null pointer");
+  DVAE_REQUIRE(T1 > 0 && B > 0 && H > 0 && V > 0, "dvae_vocab_ce_bwd_live: bad shape");
+  const int N = T1 * B;
+  const bool fwd_live = live_ok(N, V, H, h, ldh, w);
+  if (!fwd_live || lddh != H || (reinterpret_cast<uintptr_t>(d_h) & 15))
+    // the forward's h planes hold the live rows only: the every-row path splits h itself
+    return dvae_vocab_ce_bwd(h, ldh, T1, B, H, V, w, bias, targets, tgt_stride_b, lengths, lse, grad_scale_dev, d_h, lddh, d_w,
+                             d_bias, fwd_live ? nullptr : fwd_ws, ws, stream);
+  const float* hp = fwd_ws + ce_part_floats(N, V);
+  const float* wp = hp + tc16::plane_floats(N, H);
+  const float* hT_planes = fwd_ws + live_off(N, V, H);
+  const int* rows = reinterpret_cast<const int*>(hT_planes + tc16::plane_floats(H, N));
+  float a_scale = 1.f;      // power-of-two scale of P near B (see dvae_vocab_ce_bwd)
+  while (a_scale * 2.f <= (float)B) a_scale *= 2.f;
+  tc16::PlaneTable tab;
+  tab.n = 0;
+  int wT_kbtot;
+  const void* wT_planes = wT_planes_of(w, H, V, ws + p_region_floats(N, V) / 4 * 4 + tc16::plane_floats(N, H) + tc16::plane_floats(V, H),
+                                       tab, &wT_kbtot);
+  int rc = tc16::weight_planes_launch(tab, st);
+  if (rc) return rc;
+  return planes_bwd(h, ldh, N, B, H, V, w, bias, targets, tgt_stride_b, lengths, lse, grad_scale_dev, d_h, lddh, d_w, d_bias, hp, wp,
+                    wT_planes, wT_kbtot, hT_planes, a_scale, ws, rows + N, rows, st);
+}
+
 // Measurement entry (bench.py roofline, ncu): ONLY the projection + online-softmax partials kernel of dvae_vocab_ce_fwd.
 // `ws` must come from an earlier dvae_vocab_ce_fwd call with the same arguments (it holds the fp16 operand planes).
 extern "C" int dvae_vocab_ce_partials(const float* h, int64_t ldh, int T1, int B, int H, int V, const float* w,
@@ -570,7 +781,7 @@ extern "C" int dvae_vocab_ce_partials(const float* h, int64_t ldh, int T1, int B
                                       const int64_t* lengths, int sos, float* ws, void* stream) {
   DVAE_REQUIRE(h && w && bias && targets && lengths && ws, "dvae_vocab_ce_partials: null pointer");
   DVAE_REQUIRE(T1 > 0 && B > 0 && H > 0 && V > 0, "dvae_vocab_ce_partials: bad shape");
-  CeArgs p;
+  CeArgs p = {};
   p.h = h; p.ldh = ldh; p.w = w; p.bias = bias; p.targets = targets; p.tgt_stride_b = tgt_stride_b;
   p.lengths = lengths; p.N = T1 * B; p.B = B; p.H = H; p.V = V; p.sos = sos;
   p.nsplit = ce_nsplit(p.N, V, &p.tiles_per_split);
@@ -591,7 +802,7 @@ static int vocab_sample_step_impl(const float* h, int64_t ldh, int B, int H, int
   cudaStream_t st = (cudaStream_t)stream;
   DVAE_REQUIRE(h && w && bias && seed_dev && tokens_out && ws, "dvae_vocab_sample_step: null pointer");
   DVAE_REQUIRE(B > 0 && H > 0 && V > 0, "dvae_vocab_sample_step: bad shape");
-  CeArgs p;
+  CeArgs p = {};
   p.h = h; p.ldh = ldh; p.w = w; p.bias = bias; p.targets = nullptr; p.tgt_stride_b = 0; p.lengths = nullptr;
   p.N = B; p.B = B; p.H = H; p.V = V; p.sos = 0;
   p.nsplit = ce_nsplit(p.N, V, &p.tiles_per_split);

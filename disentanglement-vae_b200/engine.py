@@ -47,6 +47,10 @@ class TrainEngine:
         self.lib = _lib.load()
         self.device = model._flat.device
         self.plan = StepPlan(model, B, T, self.device)
+        # the vocabulary projection and its gradients run over the positions the loss keeps only (the row count is read
+        # on the device, so the captured step serves every length distribution); nothing the engine returns reads
+        # vocabulary outputs at masked positions
+        self.plan.live_rows = True
         self.d = d = self.plan.d
         self.world = dist.get_world_size(process_group) if (dist.is_available() and dist.is_initialized()) else 1
         self.rank = dist.get_rank(process_group) if self.world > 1 else 0

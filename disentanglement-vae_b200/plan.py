@@ -92,6 +92,9 @@ class StepPlan:
         self.recon = self.out[_lib.HEADS_NSCALARS:_lib.HEADS_NSCALARS + 1]
         self.ce_ws = buf(self.lib.dvae_vocab_ce_ws_floats(max(self.N, 1), d.V, d.Hd))
         self.sample_ws = None                      # allocated on first sampled decode
+        # vocabulary kernels over the live rows only (t < len_b): vocab_ce then leaves lse / nll / argmax at masked
+        # positions unwritten.  TrainEngine sets it; the drop-in path returns every position's argmax and keeps all rows.
+        self.live_rows = False
         self._bwd_ready = False
         self.seed_dev = torch.zeros(1, device=device, dtype=torch.int64)
         self.labels = buf(max(sum(1 for o in d.dsc_out if o > 0), 1), B)
@@ -301,12 +304,13 @@ class StepPlan:
         lib, d, st = self.lib, self.d, _lib.stream_ptr()
         w_ready = getattr(self, "_w_planes_ready", None) == P["decoder.linear.weight"].data_ptr()
         self._w_planes_ready = None
-        check(lib.dvae_vocab_ce_fwd_ex(ptr(h_top), d.Hd, self.T1, self.B, d.Hd, d.V, ptr(P["decoder.linear.weight"]),
-                                       ptr(P["decoder.linear.bias"]), ptr(targets), targets.stride(0), ptr(lengths),
-                                       d.sos, ptr(self.lse), ptr(self.nll), ptr(self.argmax), ptr(self.recon),
-                                       ptr(self.ce_ws), 1 if w_ready else 0, st), "dvae_vocab_ce_fwd")
-        # the backward of this same step may reuse the operand planes the call left in ce_ws
-        self._ce_planes_valid = (h_top.data_ptr(), P["decoder.linear.weight"].data_ptr())
+        fwd = lib.dvae_vocab_ce_fwd_live if self.live_rows else lib.dvae_vocab_ce_fwd_ex
+        check(fwd(ptr(h_top), d.Hd, self.T1, self.B, d.Hd, d.V, ptr(P["decoder.linear.weight"]),
+                  ptr(P["decoder.linear.bias"]), ptr(targets), targets.stride(0), ptr(lengths),
+                  d.sos, ptr(self.lse), ptr(self.nll), ptr(self.argmax), ptr(self.recon),
+                  ptr(self.ce_ws), 1 if w_ready else 0, st), "dvae_vocab_ce_fwd")
+        # the backward of this same step may reuse the operand planes (live rows: and the row list) the call left in ce_ws
+        self._ce_planes_valid = (h_top.data_ptr(), P["decoder.linear.weight"].data_ptr(), lengths.data_ptr(), self.live_rows)
         return self.recon
 
     # ------------------------------------------------------------------------------------------
@@ -316,13 +320,18 @@ class StepPlan:
         self._alloc_bwd()
         lib, d, st = self.lib, self.d, _lib.stream_ptr()
         # operand planes left by this step's forward call (same h_top, same weights): no need to split again
-        reuse = getattr(self, "_ce_planes_valid", None) == (h_top.data_ptr(), P["decoder.linear.weight"].data_ptr())
+        valid = getattr(self, "_ce_planes_valid", None)
+        reuse = valid is not None and valid[:3] == (h_top.data_ptr(), P["decoder.linear.weight"].data_ptr(), lengths.data_ptr())
+        live = reuse and valid[3]          # the live-row backward needs the forward's row list: same call, same lengths
         self._ce_planes_valid = None
-        check(lib.dvae_vocab_ce_bwd(ptr(h_top), d.Hd, self.T1, self.B, d.Hd, d.V, ptr(P["decoder.linear.weight"]),
-                                    ptr(P["decoder.linear.bias"]), ptr(targets), targets.stride(0), ptr(lengths),
-                                    ptr(self.lse), ptr(grad_scale_dev), ptr(self.g_top), d.Hd,
-                                    ptr(G["decoder.linear.weight"]), ptr(G["decoder.linear.bias"]),
-                                    ptr(self.ce_ws) if reuse else None, ptr(self.ce_bwd_ws), st),
+        # a live-row forward's lse exists at live positions only: the every-row backward reads it only where the loss
+        # weight is non-zero, so it still applies (without the forward's planes, which hold the live rows only)
+        bwd = lib.dvae_vocab_ce_bwd_live if live else lib.dvae_vocab_ce_bwd
+        check(bwd(ptr(h_top), d.Hd, self.T1, self.B, d.Hd, d.V, ptr(P["decoder.linear.weight"]),
+                  ptr(P["decoder.linear.bias"]), ptr(targets), targets.stride(0), ptr(lengths),
+                  ptr(self.lse), ptr(grad_scale_dev), ptr(self.g_top), d.Hd,
+                  ptr(G["decoder.linear.weight"]), ptr(G["decoder.linear.bias"]),
+                  ptr(self.ce_ws) if reuse else None, ptr(self.ce_bwd_ws), st),
               "dvae_vocab_ce_bwd")
         return self.g_top
 

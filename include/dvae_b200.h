@@ -361,6 +361,18 @@ int dvae_vocab_ce_fwd_ex(const float* h, int64_t ldh, int T1, int B, int H, int 
                          const int64_t* lengths, int sos, float* lse, float* nll, int32_t* argmax,
                          float* loss, float* ws, int flags, void* stream);
 
+/* The same over the LIVE rows only: positions with t < len_b (the ones the loss keeps), in ascending n.  Their count is
+ * known on the device only -- the call builds the row list from `lengths` and sizes the GEMMs' work from it, with launch
+ * grids for all N rows -- so one captured CUDA graph serves every length distribution.  lse / nll / argmax are written at
+ * live positions only; the loss is that of dvae_vocab_ce_fwd.  ws (dvae_vocab_ce_ws_floats) keeps the row list at float
+ * offset dvae_vocab_live_rows_at(N, V, H) (N int32 entries, then the live count) and the operand planes that
+ * dvae_vocab_ce_bwd_live reads.  Shapes the pre-split tensor-core kernels do not take run over every row. */
+int dvae_vocab_ce_fwd_live(const float* h, int64_t ldh, int T1, int B, int H, int V, const float* w,
+                           const float* bias, const int64_t* targets, int64_t tgt_stride_b,
+                           const int64_t* lengths, int sos, float* lse, float* nll, int32_t* argmax,
+                           float* loss, float* ws, int flags, void* stream);
+int64_t dvae_vocab_live_rows_at(int N, int V, int H);
+
 /* Measurement entry (bench.py roofline, ncu): only the projection + online-softmax partials kernel of
  * dvae_vocab_ce_fwd (no operand split, no finalize).  ws must come from an earlier dvae_vocab_ce_fwd call with the same
  * arguments.  Not part of the reference-facing surface. */
@@ -431,6 +443,15 @@ int dvae_vocab_ce_bwd(const float* h, int64_t ldh, int T1, int B, int H, int V, 
                       const int64_t* lengths, const float* lse, const float* grad_scale_dev,
                       float* d_h, int64_t lddh, float* d_w, float* d_bias, const float* fwd_ws, float* ws,
                       void* stream);
+
+/* Backward of dvae_vocab_ce_fwd_live: same arguments as dvae_vocab_ce_bwd, with fwd_ws (required) the workspace of the
+ * dvae_vocab_ce_fwd_live call on the same h, w and lengths, untouched since.  Only live rows enter the GEMMs; the other
+ * rows of d_h are zero, as they are in dvae_vocab_ce_bwd. */
+int dvae_vocab_ce_bwd_live(const float* h, int64_t ldh, int T1, int B, int H, int V, const float* w,
+                           const float* bias, const int64_t* targets, int64_t tgt_stride_b,
+                           const int64_t* lengths, const float* lse, const float* grad_scale_dev,
+                           float* d_h, int64_t lddh, float* d_w, float* d_bias, const float* fwd_ws, float* ws,
+                           void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Train-step tail: clip_grad_norm_(5.0) + Adam + zero_grad (run.py:255,261-262) over ONE flat
