@@ -56,6 +56,7 @@ SIGNATURES = {
     "dvae_vocab_sample_step_planes": (_i, [_p, _l, _i, _i, _i, _p, _p, _p, _p, _u32, _p, _l, _p, _p, _p]),
     "dvae_recount_lengths": (_i, [_p, _l, _l, _i, _i, _l, _l, _l, _p, _p]),
     "dvae_bleu_counts": (_i, [_p, _l, _i, _p, _l, _i, _i, _l, _p, _p]),
+    "dvae_bleu_counts_ex": (_i, [_p, _l, _i, _p, _l, _i, _i, _l, _p, _p, _p]),
     "dvae_bleu_score": (_i, [_p, _p, _p]),
     "dvae_lstm_state_ws_floats": (_l, [_i, _i, _i]),
     "dvae_lstm_seq_fwd": (_i, [_p, _l, _i, _i, _i, _i, _i, _pp, _pp, _pp, _pp, _p, _p, _l, _l, _p, _p, _l, _p, _p,

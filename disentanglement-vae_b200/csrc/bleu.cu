@@ -1,6 +1,8 @@
 // Corpus BLEU on token ids (see include/dvae_b200.h):
 //   dvae_bleu_counts -- the n-gram statistics of vae/losses.py:128-134 (torchtext 0.6 bleu_score, max_n = 4) of one batch,
 //                       ADDED into int64 counters so that a corpus can be accumulated over calls and ranks
+//   dvae_bleu_counts_ex -- the same with a row-length bound read from device memory (rows padded beyond their batch's
+//                       length, the engine's eval graph at every padded length)
 //   dvae_bleu_score  -- the score from those counters, in float64, written to device memory (graph-capturable)
 // One warp per row: both truncated rows are staged in shared memory, every lane takes candidate positions, and a position
 // contributes min(count_cand, count_ref) of its n-gram only where that n-gram first occurs in the candidate.  O(4 T^2) per
@@ -32,7 +34,13 @@ __device__ __forceinline__ bool ngram_eq(const int64_t* a, int i, const int64_t*
 __global__ void __launch_bounds__(kBleuWarps * 32) bleu_counts_kernel(const int64_t* __restrict__ ref, int64_t ref_stride,
                                                                         int T_ref, const int64_t* __restrict__ cand,
                                                                         int64_t cand_stride, int T_cand, int B, int64_t eos,
+                                                                        const int* __restrict__ t_max,
                                                                         unsigned long long* __restrict__ counts) {
+  if (t_max != nullptr) {      // rows end at the batch's own padded length: EOS-less rows are cut there, not at the buffer's end
+    const int t = max(*t_max, 0);
+    T_ref = min(T_ref, t);
+    T_cand = min(T_cand, t);
+  }
   __shared__ int64_t s_ref[kBleuWarps][DVAE_BLEU_MAX_T];
   __shared__ int64_t s_cand[kBleuWarps][DVAE_BLEU_MAX_T];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
@@ -93,17 +101,23 @@ __global__ void bleu_score_kernel(const int64_t* __restrict__ counts, float* __r
 }  // namespace
 }  // namespace dvae
 
-extern "C" int dvae_bleu_counts(const int64_t* ref, int64_t ref_stride, int T_ref, const int64_t* cand, int64_t cand_stride,
-                                int T_cand, int B, int64_t eos, int64_t* counts, void* stream) {
+extern "C" int dvae_bleu_counts_ex(const int64_t* ref, int64_t ref_stride, int T_ref, const int64_t* cand,
+                                   int64_t cand_stride, int T_cand, int B, int64_t eos, const int* t_max, int64_t* counts,
+                                   void* stream) {
   DVAE_REQUIRE(ref && cand && counts && B > 0 && T_ref > 0 && T_cand > 0 && ref_stride >= T_ref && cand_stride >= T_cand,
                "dvae_bleu_counts: bad argument");
   DVAE_REQUIRE(T_ref <= DVAE_BLEU_MAX_T && T_cand <= DVAE_BLEU_MAX_T,
                "dvae_bleu_counts: T_ref = %d, T_cand = %d; at most %d tokens per row", T_ref, T_cand, DVAE_BLEU_MAX_T);
   const int grid = dvae::ceil_div(B, dvae::kBleuWarps) < 148 * 4 ? dvae::ceil_div(B, dvae::kBleuWarps) : 148 * 4;
   dvae::bleu_counts_kernel<<<grid, dvae::kBleuWarps * 32, 0, (cudaStream_t)stream>>>(
-      ref, ref_stride, T_ref, cand, cand_stride, T_cand, B, eos, reinterpret_cast<unsigned long long*>(counts));
+      ref, ref_stride, T_ref, cand, cand_stride, T_cand, B, eos, t_max, reinterpret_cast<unsigned long long*>(counts));
   DVAE_LAUNCH_CHECK();
   return DVAE_OK;
+}
+
+extern "C" int dvae_bleu_counts(const int64_t* ref, int64_t ref_stride, int T_ref, const int64_t* cand, int64_t cand_stride,
+                                int T_cand, int B, int64_t eos, int64_t* counts, void* stream) {
+  return dvae_bleu_counts_ex(ref, ref_stride, T_ref, cand, cand_stride, T_cand, B, eos, nullptr, counts, stream);
 }
 
 extern "C" int dvae_bleu_score(const int64_t* counts, float* score_out, void* stream) {

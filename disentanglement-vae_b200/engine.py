@@ -19,16 +19,25 @@ Variants of the step (all with the reference's semantics):
     no graph.
   * evaluation (eval_step / eval_steps, run.py:347-423): the same forward with train=False, the losses and corpus BLEU of
     the predictions, one graph per decode regime; no backward, no optimizer, training state untouched.
+
+Batch shapes: the engine is built for (B, T) and takes any batch [B', T'] with B' <= B and 2 <= T' <= T.  A narrower batch
+is padded to T with PAD columns in the pinned staging block (exact: the encoder reads the lengths, the loss keeps position
+(t, b) only when t + 1 < len_b, and the vocabulary kernels run over those positions only).  A batch with fewer rows runs
+on a `_Shape` of its own at (B', T) -- plan, staging block, graphs -- built on its first batch and cached; parameters,
+gradients, Adam moments, weight planes, counters and random streams are shared.  A batch of the full shape (B, T) runs
+exactly the graph the engine had before any other shape was seen.
 """
 import os
 import random
+from collections import OrderedDict
 
+import numpy as np
 import torch
 import torch.distributed as dist
 
 from . import _lib
 from ._lib import ptr, check
-from .plan import StepPlan
+from .plan import StepPlan, Dims
 from .losses import get_cyclic_kl_weight
 
 
@@ -36,9 +45,66 @@ def d_bow(plan):
     return bool(plan.d.bow)
 
 
+class _Shape:
+    """The per-shape state of a TrainEngine at B rows (padded length: the engine's T): its StepPlan, the device block the
+    per-step host data lands in with its typed views, the pinned host blocks that fill it (one per ring slot), the
+    sampled-decode prediction buffer, the captured train graph(s) and the evaluation buffers / graphs."""
+
+    def __init__(self, eng, B):
+        T, d, dev = eng.T, eng.d, eng.device
+        self.B = B
+        self.plan = StepPlan(eng.model, B, T, dev)
+        # the vocabulary projection and its gradients run over the positions the loss keeps only (the row count is read
+        # on the device, so the captured step serves every length distribution); nothing the engine returns reads
+        # vocabulary outputs at masked positions
+        self.plan.live_rows = True
+        T1 = max(T - 1, 1)
+        # Everything the host sends per step lives in ONE device block (typed views below) filled by ONE H2D copy from a ring
+        # of pinned host blocks: token ids, lengths, Philox seed, labels, Adam / KL scalars, teacher-forcing coins.  An
+        # asynchronous H2D copy reads host memory when it executes, so a slot is rewritten only after the event recorded
+        # behind its last use has completed (ADVICE r1: un-synchronised step_resident calls saw a later step's scalars).
+        lay, off = {}, 0
+        for name, nbytes in (("inputs", B * T * 8), ("lengths", B * 8), ("seed", 8), ("labels", eng.n_dsc * B * 4),
+                             ("scal", (8 + max(d.S, 1)) * 4), ("coins", T1 * 4)):
+            lay[name] = (off, nbytes)
+            off = (off + nbytes + 15) // 16 * 16
+        # the batch's own padded length T' (int32; the BLEU kernel's row bound) in word 5 of the scalar block, which the
+        # step does not read: the block keeps its size
+        lay["tlen"] = (lay["scal"][0] + 5 * 4, 4)
+        self.bytes, self.lay = off, lay
+        self.d_stage = torch.zeros(off, device=dev, dtype=torch.uint8)
+
+        def view(buf, name, dtype, *shape):
+            o, n = lay[name]
+            return buf[o:o + n].view(dtype).view(*shape)
+        self.inputs = view(self.d_stage, "inputs", torch.int64, B, T)
+        self.lengths = view(self.d_stage, "lengths", torch.int64, B)
+        self.labels = view(self.d_stage, "labels", torch.float32, eng.n_dsc, B)
+        self.d_scal = view(self.d_stage, "scal", torch.float32, 8 + max(d.S, 1))
+        self.coins = view(self.d_stage, "coins", torch.int32, T1)          # 1 = teacher-forced step
+        self.coins.fill_(1)
+        self.tlen = view(self.d_stage, "tlen", torch.int32, 1)
+        self.plan.seed_dev = view(self.d_stage, "seed", torch.int64, 1)     # the plan's kernels read the seed from here
+        self.preds = torch.zeros(B, T, device=dev, dtype=torch.int64) if eng.sampled else None
+        self.h_stage = torch.zeros(eng.NSLOT, off, dtype=torch.uint8).pin_memory()
+        self.hv = [{k: view(self.h_stage[i], k, dt, *shp).numpy() for k, dt, shp in
+                    (("inputs", torch.int64, (B, T)), ("lengths", torch.int64, (B,)), ("seed", torch.int64, (1,)),
+                     ("labels", torch.float32, (eng.n_dsc, B)), ("scal", torch.float32, (8 + max(d.S, 1),)),
+                     ("coins", torch.int32, (T1,)), ("tlen", torch.int32, (1,)))} for i in range(eng.NSLOT)]
+        for hv in self.hv:
+            hv["coins"][:] = 1
+            hv["lengths"][:] = 1
+            hv["tlen"][:] = T
+        self.graphs = None     # captured train step: one graph, or the data-parallel stage graphs
+        self.eval = None       # evaluation buffers and graphs, allocated on this shape's first eval_step
+
+
 class TrainEngine:
     # pinned staging slots for the per-step scalar block (ring, guarded by CUDA events) = how many steps the host may run ahead
     NSLOT = max(3, int(os.environ.get("DVAE_ENGINE_SLOTS", "4")))
+    # batch sizes B' < B kept besides the full shape, least recently used evicted first.  A run through RatioSampler or a
+    # DataLoader with drop_last=False meets one (its last batch); evaluation over a dev set adds at most one more.
+    MAX_EXTRA_SHAPES = 2
 
     def __init__(self, model, params, B, T, lr=None, total_steps=None, use_graph=True, max_norm=5.0,
                  process_group=None, seed=None, teacher_forcing_prob=None):
@@ -46,12 +112,7 @@ class TrainEngine:
         self.model, self.params, self.B, self.T = model, params, B, T
         self.lib = _lib.load()
         self.device = model._flat.device
-        self.plan = StepPlan(model, B, T, self.device)
-        # the vocabulary projection and its gradients run over the positions the loss keeps only (the row count is read
-        # on the device, so the captured step serves every length distribution); nothing the engine returns reads
-        # vocabulary outputs at masked positions
-        self.plan.live_rows = True
-        self.d = d = self.plan.d
+        self.d = d = Dims(model)
         self.world = dist.get_world_size(process_group) if (dist.is_available() and dist.is_initialized()) else 1
         self.rank = dist.get_rank(process_group) if self.world > 1 else 0
         self.pg = process_group
@@ -89,40 +150,14 @@ class TrainEngine:
         self.kl_w = torch.zeros(max(d.S, 1), **f32)
         self.sumsq = torch.zeros(1, **f32)
         self.red_ws = torch.zeros(1032, **f32)
-        T1 = max(T - 1, 1)
-        # Everything the host sends per step lives in ONE device block (typed views below) filled by ONE H2D copy from a ring
-        # of pinned host blocks: token ids, lengths, Philox seed, labels, Adam / KL scalars, teacher-forcing coins.  An
-        # asynchronous H2D copy reads host memory when it executes, so a slot is rewritten only after the event recorded
-        # behind its last use has completed (ADVICE r1: un-synchronised step_resident calls saw a later step's scalars).
-        lay, off = {}, 0
-        for name, nbytes in (("inputs", B * T * 8), ("lengths", B * 8), ("seed", 8), ("labels", self.n_dsc * B * 4),
-                             ("scal", (8 + max(d.S, 1)) * 4), ("coins", T1 * 4)):
-            lay[name] = (off, nbytes)
-            off = (off + nbytes + 15) // 16 * 16
-        self._stage_bytes, self._stage_lay = off, lay
-        self.d_stage = torch.zeros(off, device=self.device, dtype=torch.uint8)
-
-        def view(buf, name, dtype, *shape):
-            o, n = lay[name]
-            return buf[o:o + n].view(dtype).view(*shape)
-        self.inputs = view(self.d_stage, "inputs", torch.int64, B, T)
-        self.lengths = view(self.d_stage, "lengths", torch.int64, B)
-        self.labels = view(self.d_stage, "labels", torch.float32, self.n_dsc, B)
-        self.d_scal = view(self.d_stage, "scal", torch.float32, 8 + max(d.S, 1))
-        self.coins = view(self.d_stage, "coins", torch.int32, T1)          # 1 = teacher-forced step
-        self.coins.fill_(1)
-        self.plan.seed_dev = view(self.d_stage, "seed", torch.int64, 1)     # the plan's kernels read the seed from here
-        self.preds = torch.zeros(B, T, device=self.device, dtype=torch.int64) if self.sampled else None
+        self._full = self._sh = _Shape(self, B)     # _sh: the shape of the most recent step
+        self._extra = OrderedDict()                   # B' -> _Shape, least recently used first
+        self._last_T = T                              # padded length of the most recent training step's batch
+        self._eval_last = None                        # (shape, T') of the most recent evaluation batch
         ns = self.NSLOT
-        self.h_stage = torch.zeros(ns, off, dtype=torch.uint8).pin_memory()
-        self.h_outs = torch.zeros(ns, self.plan.out.numel(), dtype=torch.float32).pin_memory()
-        self._hv = [{k: view(self.h_stage[i], k, dt, *shp).numpy() for k, dt, shp in
-                     (("inputs", torch.int64, (B, T)), ("lengths", torch.int64, (B,)), ("seed", torch.int64, (1,)),
-                      ("labels", torch.float32, (self.n_dsc, B)), ("scal", torch.float32, (8 + max(d.S, 1),)),
-                      ("coins", torch.int32, (T1,)))} for i in range(ns)]
-        for hv in self._hv:
-            hv["coins"][:] = 1
-            hv["lengths"][:] = 1
+        self.h_outs = torch.zeros(ns, self._full.plan.out.numel(), dtype=torch.float32).pin_memory()
+        # the evaluation result ring, shared by the shapes like h_outs (allocated on the first eval_step)
+        self._eval_ring = None
         self.h_out = self.h_outs[0]
         self._slot_ev = [None] * ns
         self._slot = -1
@@ -136,9 +171,7 @@ class TrainEngine:
         # evaluation draws its eps / coins from streams of its own, so that eval_step never shifts the training streams
         self._eval_gen = torch.Generator().manual_seed(base + 0x5EED)
         self._eval_pyrand = random.Random(base + 0x5EED)
-        self._eval = None      # evaluation buffers and graphs, allocated on the first eval_step
         self.use_graph = use_graph and not self.aux
-        self._graphs = None
         self._buckets = None
         self._comm = None
         self._xchg_in_capture = False      # one-graph data parallel: the step being captured exchanges inside the graph
@@ -151,6 +184,61 @@ class TrainEngine:
         self._wplanes, self._plane_token = [], object()
         if os.environ.get("DVAE_WEIGHT_PLANES", "1") != "0" and not d.bow:
             self._alloc_weight_planes()
+
+    # ---- the per-shape state of the most recent step ------------------------------------------------------------
+    # After a step on a full (B, T) batch these are the full shape's: what they have always been.
+    plan = property(lambda self: self._sh.plan, doc="StepPlan of the most recent step (utils.LatentLog.append(engine.plan, "
+                                                    "ids) logs its rows: B' of them after a short batch)")
+    inputs = property(lambda self: self._sh.inputs, doc="[B', T] device token ids of the most recent step (PAD beyond T')")
+    lengths = property(lambda self: self._sh.lengths, doc="[B'] device lengths of the most recent step")
+    labels = property(lambda self: self._sh.labels, doc="[n_dsc, B'] device labels of the most recent step")
+    coins = property(lambda self: self._sh.coins, doc="[T - 1] int32 device teacher-forcing coins (1 = forced)")
+    preds = property(lambda self: self._sh.preds, doc="[B', T] device decoder inputs of a sampled-decode step, or None")
+    d_scal = property(lambda self: self._sh.d_scal)
+    _eval = property(lambda self: self._sh.eval)
+
+    def _shape(self, B):
+        """Make the shape of B rows current: the full shape, or a cached / new short one (evicting the least recently
+        used beyond MAX_EXTRA_SHAPES)."""
+        if B == self.B:
+            sh = self._full
+        else:
+            sh = self._extra.pop(B, None)
+            if sh is None:
+                if len(self._extra) >= self.MAX_EXTRA_SHAPES:
+                    torch.cuda.synchronize(self.device)      # enqueued steps may still read its graphs and blocks
+                    self._extra.popitem(last=False)
+                sh = _Shape(self, B)
+            self._extra[B] = sh
+        self._sh = sh
+        return sh
+
+    def _check_shape(self, B, T, where):
+        if not (1 <= B <= self.B and 2 <= T <= self.T):
+            raise ValueError(f"{where}: a batch of shape ({B}, {T}); this engine was built for ({self.B}, {self.T}) and "
+                             f"takes [B', T'] batches with 1 <= B' <= {self.B} and 2 <= T' <= {self.T}")
+
+    def _host_batch(self, inputs, lengths, labels, where):
+        """Checks a HOST batch against the engine's shape; returns (inputs, lengths, per-label rows) as numpy arrays."""
+        X = inputs.numpy() if torch.is_tensor(inputs) else np.asarray(inputs)
+        L = lengths.numpy() if torch.is_tensor(lengths) else np.asarray(lengths)
+        if X.ndim != 2:
+            raise ValueError(f"{where}: inputs must be [B', T'], got shape {tuple(X.shape)}")
+        B, T = X.shape
+        self._check_shape(B, T, where)
+        if L.shape != (B,):
+            raise ValueError(f"{where}: lengths has shape {tuple(L.shape)}, expected ({B},) for inputs of shape ({B}, {T})")
+        if int(L.max()) > T:
+            raise ValueError(f"{where}: a length of {int(L.max())} exceeds the batch's padded length T' = {T} "
+                             f"(engine shape ({self.B}, {self.T}))")
+        Ys = []
+        for n in self.label_names:
+            y = labels[n]
+            y = (y.numpy() if torch.is_tensor(y) else np.asarray(y)).reshape(-1)
+            if y.shape != (B,):
+                raise ValueError(f"{where}: labels['{n}'] has {y.size} elements, expected {B} (inputs of shape ({B}, {T}))")
+            Ys.append(y)
+        return X, L, Ys
 
     # ---- weight planes: fp16 (hi, lo) operand tiles of the LSTM input weights and of W_out^T, refreshed once per step ------
     def _alloc_weight_planes(self):
@@ -190,7 +278,7 @@ class TrainEngine:
         self.hyper[:5].copy_(self.d_scal[:5])
         self.kl_w.copy_(self.d_scal[8:8 + self.kl_w.numel()])
         if self.fixed_eps is not None:      # replay given reparameterisation noise (tests; forward(eps=...) of the drop-in path)
-            pl.eps.copy_(self.fixed_eps)
+            pl.eps.copy_(self.fixed_eps[:pl.B])      # a B' < B step reads the first B' rows
         else:
             pl.randn_eps()
         # the decoder's input embeddings, its layer-0 input projection and the W_out operand planes do not depend on
@@ -499,25 +587,25 @@ class TrainEngine:
                 self._fwd_bwd()
                 self._optim()
                 return
-            if self._graphs is None:
+            if self._sh.graphs is None:
                 self._capture()
-            self._graphs[0].replay()          # one graph: forward, backward, clip + Adam
+            self._sh.graphs[0].replay()          # one graph: forward, backward, clip + Adam
             return
         # data parallel: gradients are all-reduced in the order the backward pass finishes them, on a communication stream,
         # under the rest of the backward pass: W_out | decoder embedding + LSTM | upper encoder layers + heads | encoder
         # embedding + layer 0 (four stages); bag-of-words or one-layer encoders: decoder | everything else (two stages)
         self._ensure_buckets()
         cur = torch.cuda.current_stream()
-        if self.use_graph and self._graphs is None:
+        if self.use_graph and self._sh.graphs is None:
             self._capture()
         if self._one_graph_dp():      # the exchanges are nodes of the graph
-            self._graphs[0].replay()
+            self._sh.graphs[0].replay()
             return
         # NCCL on the communication stream between stage graphs (or eager stages); stage gi finishes bucket gi
         stages = (0, 1, 2, 3) if self._three_buckets() else (1, 2)
         for gi, part in enumerate(stages):
             if self.use_graph:
-                self._graphs[gi].replay()
+                self._sh.graphs[gi].replay()
             else:
                 self._fwd_bwd(part)
             if self._buckets[gi]:
@@ -527,12 +615,14 @@ class TrainEngine:
                         dist.all_reduce(v, op=dist.ReduceOp.SUM, group=self.pg)
         cur.wait_stream(self._comm)
         if self.use_graph:
-            self._graphs[-1].replay()
+            self._sh.graphs[-1].replay()
         else:
             self._optim()
 
     def _capture(self):
-        # warm up eagerly on a side stream (lazy module loading, cudaFuncSetAttribute, allocator), then capture
+        # warm up eagerly on a side stream (lazy module loading, cudaFuncSetAttribute, allocator), then capture the current
+        # shape's step.  The warm-up runs no gradient exchange (data parallel: the graph holds it, or NCCL runs between
+        # the stage graphs), so one rank capturing a new shape never waits on another
         snap = (self.flat.clone(), self.m.clone(), self.v.clone())
         s = torch.cuda.Stream(device=self.device)
         s.wait_stream(torch.cuda.current_stream())
@@ -573,7 +663,7 @@ class TrainEngine:
         # undo the warm-up updates so that capture leaves the training state untouched
         self.flat.copy_(snap[0]); self.m.copy_(snap[1]); self.v.copy_(snap[2])
         self.grad.zero_()
-        self._graphs = tuple(graphs)
+        self._sh.graphs = tuple(graphs)
 
     # ---- per-step host scalars -----------------------------------------------------------------
     def _acquire_slot(self):
@@ -583,10 +673,13 @@ class TrainEngine:
             ev.synchronize()
         return self._slot
 
-    def _fill_scalars(self, hv, eval_tf=None):
-        """Adam hyper-parameters and step count, KL weights (cyclic value of this global step), dropout / noise seed and the
-        teacher-forcing coins of this step, written into a pinned host block.  eval_tf (an evaluation's teacher-forcing
-        probability): "cyclic" KL weights are 1.0 (run.py:374-375), seed and coins come from the evaluation streams."""
+    def _fill_scalars(self, hv, eval_tf=None, T=None):
+        """Adam hyper-parameters and step count, KL weights (cyclic value of this global step), dropout / noise seed, the
+        batch's padded length T (default: the engine's) and the teacher-forcing coins of this step, written into a pinned
+        host block.  eval_tf (an evaluation's teacher-forcing probability): "cyclic" KL weights are 1.0 (run.py:374-375),
+        seed and coins come from the evaluation streams."""
+        T = self.T if T is None else T
+        hv["tlen"][0] = T
         train = eval_tf is None
         sc = hv["scal"]
         sc[0], sc[1], sc[2], sc[3], sc[4] = self.lr, 0.9, 0.999, 1e-8, float(self.adam_step + 1)
@@ -599,17 +692,19 @@ class TrainEngine:
         tf, rnd = (self.tf_prob, self._pyrand) if train else (eval_tf, self._eval_pyrand)
         if tf < 1.0:          # one coin per decoding step, shared by the batch (vae/model.py:463)
             c = hv["coins"]
-            for i in range(c.shape[0]):
+            for i in range(T - 1):      # T' - 1 draws, as the reference's loop: the stream of an engine built at T'
                 c[i] = 1 if rnd.random() < tf else 0
+            c[T - 1:] = 1               # steps past the batch's length read PAD inputs, forced
 
     def _upload(self, slot, names=None):
         """H2D of a pinned block: the whole block (one copy), or only the named fields (device-resident batches)."""
+        sh = self._sh
         if names is None:
-            self.d_stage.copy_(self.h_stage[slot], non_blocking=True)
+            sh.d_stage.copy_(sh.h_stage[slot], non_blocking=True)
         else:
             for k in names:
-                o, n = self._stage_lay[k]
-                self.d_stage[o:o + n].copy_(self.h_stage[slot, o:o + n], non_blocking=True)
+                o, n = sh.lay[k]
+                sh.d_stage[o:o + n].copy_(sh.h_stage[slot, o:o + n], non_blocking=True)
 
     def _release_slot(self, slot):
         ev = torch.cuda.Event()
@@ -618,41 +713,70 @@ class TrainEngine:
 
     # ---- public entry points -------------------------------------------------------------------
     def step_resident(self, inputs_dev, lengths_dev, labels_dev):
-        """One train step on a batch already in HBM; returns the device result block
-        (plan.out: [0] weighted KL, [1] KL, [2] dsc loss, [3..] per space, [27] reconstruction).
-        Asynchronous: may be called back to back without synchronising."""
+        """One train step on a batch already in HBM (inputs [B',T'] int64, lengths [B'], labels [n_dsc,B']); returns the
+        device result block (plan.out: [0] weighted KL, [1] KL, [2] dsc loss, [3..] per space, [27] reconstruction).
+        Asynchronous: may be called back to back without synchronising.  Lengths are checked against T' only when
+        T' < T (one device read); a full-width batch is taken without a host round trip."""
+        if inputs_dev.dim() != 2:
+            raise ValueError(f"step_resident: inputs must be [B', T'], got shape {tuple(inputs_dev.shape)}")
+        B, T = inputs_dev.shape
+        self._check_shape(B, T, "step_resident")
+        if tuple(lengths_dev.shape) != (B,):
+            raise ValueError(f"step_resident: lengths has shape {tuple(lengths_dev.shape)}, expected ({B},)")
+        if self.label_names and tuple(labels_dev.shape) != (self.n_dsc, B):
+            raise ValueError(f"step_resident: labels has shape {tuple(labels_dev.shape)}, expected ({self.n_dsc}, {B})")
+        if T < self.T and int(lengths_dev.max()) > T:
+            raise ValueError(f"step_resident: a length of {int(lengths_dev.max())} exceeds the batch's padded length "
+                             f"T' = {T} (engine shape ({self.B}, {self.T}))")
+        sh = self._shape(B)
         slot = self._acquire_slot()
-        self._fill_scalars(self._hv[slot])
+        self._fill_scalars(sh.hv[slot], T=T)
         self._upload(slot, ("seed", "scal", "coins") if self.sampled else ("seed", "scal"))
-        self.inputs.copy_(inputs_dev, non_blocking=True)
+        if T == self.T:
+            self.inputs.copy_(inputs_dev, non_blocking=True)
+        else:
+            self.inputs[:, :T].copy_(inputs_dev, non_blocking=True)
+            self.inputs[:, T:].zero_()
         self.lengths.copy_(lengths_dev, non_blocking=True)
         self.labels.copy_(labels_dev, non_blocking=True)
+        self._last_T = T
         self._run()
         self._release_slot(slot)
         self.step_idx += 1
         self.adam_step += 1
         return self.plan.out
 
-    def _enqueue_host_step(self, inputs, lengths, labels, eval_tf=None):
-        """Stage one HOST batch into the next pinned block, enqueue its single H2D copy, the step and the D2H copy of the
-        result block; returns the slot (its event completes when the losses are in h_outs[slot]).  eval_tf: an
-        evaluation step at that teacher-forcing probability instead (result block in the evaluation ring)."""
+    def _enqueue_host_step(self, inputs, lengths, labels, eval_tf=None, where="step_host"):
+        """Stage one HOST batch [B', T'] into the next pinned block of its shape (padded to T with PAD columns), enqueue its
+        single H2D copy, the step and the D2H copy of the result block; returns the slot (its event completes when the
+        losses are in h_outs[slot]).  eval_tf: an evaluation step at that teacher-forcing probability instead (result
+        block in the evaluation ring)."""
+        X, L, Ys = self._host_batch(inputs, lengths, labels, where)
+        B, T = X.shape
+        sh = self._shape(B)
+        if eval_tf is not None:
+            self._eval_setup()
         slot = self._acquire_slot()
-        hv = self._hv[slot]
-        hv["inputs"][...] = inputs.numpy() if torch.is_tensor(inputs) else inputs
-        hv["lengths"][...] = lengths.numpy() if torch.is_tensor(lengths) else lengths
-        for i, n in enumerate(self.label_names):
-            y = labels[n]
-            hv["labels"][i] = (y.numpy() if torch.is_tensor(y) else y).reshape(-1)
-        self._fill_scalars(hv, eval_tf)
+        hv = sh.hv[slot]
+        if T == self.T:
+            hv["inputs"][...] = X
+        else:
+            hv["inputs"][:, :T] = X
+            hv["inputs"][:, T:] = 0
+        hv["lengths"][...] = L
+        for i, y in enumerate(Ys):
+            hv["labels"][i] = y
+        self._fill_scalars(hv, eval_tf, T)
         self._upload(slot)
         if eval_tf is not None:
+            self._eval_last = (sh, T)
             ev = self._eval
             self._run(lambda: self._eval_run(eval_tf < 1.0))
             ev["h_out"][slot].copy_(ev["out"], non_blocking=True)
             ev["aux"][slot] = self._eval_aux() if self.aux else None
             self._release_slot(slot)
             return slot
+        self._last_T = T
         self._run()
         self.h_outs[slot].copy_(self.plan.out, non_blocking=True)
         self._release_slot(slot)
@@ -661,8 +785,9 @@ class TrainEngine:
         return slot
 
     def step_host(self, inputs, lengths, labels):
-        """End-to-end step: HOST tensors in (inputs [B,T] int64, lengths [B] int64, labels {name: [B,1]}),
-        python floats out.  One H2D copy of the staged block, the step, one D2H read of the loss block, then a wait."""
+        """End-to-end step: HOST tensors in (inputs [B',T'] int64, lengths [B'] int64, labels {name: [B',1]}; B' <= B,
+        2 <= T' <= T, lengths <= T', else ValueError), python floats out.  One H2D copy of the staged block, the step, one
+        D2H read of the loss block, then a wait."""
         slot = self._enqueue_host_step(inputs, lengths, labels)
         self._slot_ev[slot].synchronize()
         self.h_out = self.h_outs[slot]
@@ -672,11 +797,13 @@ class TrainEngine:
         """Pipelined training loop over an iterable of HOST batches (inputs, lengths, labels): yields the loss dict of every
         step, in order, `lag` steps behind the step being enqueued -- batch k + 1 is staged and uploaded while the GPU runs
         step k, and nothing waits for the device except the read of a result that is `lag` steps old.  Same arithmetic as
-        calling step_host() per batch (run.py:217-262); `lag` must be smaller than NSLOT."""
+        calling step_host() per batch (run.py:217-262), with the same batch shapes; `lag` must be smaller than NSLOT.
+        Data parallel: every rank's batches have the same shapes step by step (RatioSampler's default drop_uneven=True
+        gives equal shards of a short last batch); unequal shards are not supported."""
         assert 0 <= lag < self.NSLOT
         pending = []
         for inputs, lengths, labels in batches:
-            pending.append(self._enqueue_host_step(inputs, lengths, labels))
+            pending.append(self._enqueue_host_step(inputs, lengths, labels, where="train_steps"))
             if len(pending) > lag:
                 slot = pending.pop(0)
                 self._slot_ev[slot].synchronize()
@@ -708,14 +835,17 @@ class TrainEngine:
     # Result block (float32): [0, NS + 5) the training block's layout (heads scalars, [NS] reconstruction loss),
     # [NS + 1] corpus BLEU, then the 10 int64 BLEU counts of dvae_bleu_counts (clipped 1-4, total 1-4, cand / ref length).
     def _eval_setup(self):
-        if self._eval is not None:
-            return self._eval
-        NB = self.plan.out.numel()
+        """The current shape's evaluation buffers; the result ring (h_out, aux) is the engine's, shared by the shapes."""
+        sh = self._sh
+        if sh.eval is not None:
+            return sh.eval
+        NB = sh.plan.out.numel()
         out = torch.zeros(NB + 20, device=self.device, dtype=torch.float32)
-        self._eval = ev = {"out": out, "counts": out[NB:].view(torch.int64), "nb": NB, "graphs": {},
-                           "preds": torch.zeros(self.B, self.T, device=self.device, dtype=torch.int64),
-                           "h_out": torch.zeros(self.NSLOT, out.numel(), dtype=torch.float32).pin_memory(),
-                           "aux": [None] * self.NSLOT}
+        if self._eval_ring is None:
+            self._eval_ring = (torch.zeros(self.NSLOT, out.numel(), dtype=torch.float32).pin_memory(), [None] * self.NSLOT)
+        sh.eval = ev = {"out": out, "counts": out[NB:].view(torch.int64), "nb": NB, "graphs": {},
+                        "preds": torch.zeros(sh.B, self.T, device=self.device, dtype=torch.int64),
+                        "h_out": self._eval_ring[0], "aux": self._eval_ring[1]}
         return ev
 
     def _eval_body(self, sampled):
@@ -731,11 +861,12 @@ class TrainEngine:
         NS, NB = _lib.HEADS_NSCALARS, ev["nb"]
         ev["out"][:NB].copy_(pl.out)
         ev["counts"].zero_()
-        bleu_counts_(ev["counts"], self.inputs, preds, m.eos_token_idx)
+        # rows end at the batch's own padded length T' (from the staging block): an EOS-less row loses its T'-th token
+        bleu_counts_(ev["counts"], self.inputs, preds, m.eos_token_idx, t_max=self._sh.tlen)
         bleu_score_(ev["out"][NS + 1:NS + 2], ev["counts"])
 
     def _eval_run(self, sampled):
-        ev = self._eval
+        ev = self._eval           # the current shape's: its graphs are keyed by decode regime
         if not self.use_graph:
             self._eval_body(sampled)
         else:
@@ -761,8 +892,8 @@ class TrainEngine:
         block over the ranks (one all-reduce, float64 -- exact for the counts) and divide by the global batch."""
         from .losses import bleu_score_
         ev, NB, NS = self._eval, self._eval["nb"], _lib.HEADS_NSCALARS
-        red = torch.cat([ev["out"][:NB].double() * self.B, ev["counts"].double(),
-                         torch.full((1,), float(self.B), device=self.device, dtype=torch.float64)])
+        red = torch.cat([ev["out"][:NB].double() * self._sh.B, ev["counts"].double(),
+                         torch.full((1,), float(self._sh.B), device=self.device, dtype=torch.float64)])
         dist.all_reduce(red, op=dist.ReduceOp.SUM, group=self.pg)
         ev["out"][:NB].copy_(red[:NB] / red[-1])
         ev["counts"].copy_(red[NB:NB + 10].round().long())
@@ -791,16 +922,17 @@ class TrainEngine:
         return L
 
     def eval_step(self, inputs, lengths, labels, teacher_forcing_prob):
-        """Validation step (run.py:evalstep, run.py:347-423) on HOST tensors (inputs [B,T] int64, lengths [B], labels
-        {name: [B,1]}): eval-mode forward (no dropout, one eps draw), the loss dict of compute_all_losses with "cyclic" KL
-        weights at 1.0 (run.py:374-375), plus "bleu" (compute_bleu of the predictions against the inputs) and
+        """Validation step (run.py:evalstep, run.py:347-423) on HOST tensors (inputs [B',T'] int64, lengths [B'], labels
+        {name: [B',1]}; the shapes step_host takes): eval-mode forward (no dropout, one eps draw), the loss dict of
+        compute_all_losses with "cyclic" KL weights at 1.0 (run.py:374-375), plus "bleu" (compute_bleu of the predictions against the inputs) and
         "bleu_counts" (its 10 corpus statistics, which add over batches).  One captured graph per decode regime
-        (teacher_forcing_prob == 1: forced decode; < 1: sampled decode, coins drawn per call), one H2D and one D2H copy.
+        (teacher_forcing_prob == 1: forced decode; < 1: sampled decode, coins drawn per call) and batch shape, one H2D and
+        one D2H copy.
         Parameters, optimizer state, step counters and the training random streams are not touched; plan.z / mu / logvar
         hold this batch afterwards (utils.LatentLog.append(engine.plan, ids) logs dev latents); eval_predictions holds
-        the predicted tokens.  Data parallel: every rank passes its shard and gets the losses of the global batch."""
-        self._eval_setup()
-        slot = self._enqueue_host_step(inputs, lengths, labels, eval_tf=float(teacher_forcing_prob))
+        the predicted tokens.  Data parallel: every rank passes its shard (equal shards) and gets the losses of the
+        global batch."""
+        slot = self._enqueue_host_step(inputs, lengths, labels, eval_tf=float(teacher_forcing_prob), where="eval_step")
         self._slot_ev[slot].synchronize()
         return self._eval_losses(slot)
 
@@ -809,11 +941,10 @@ class TrainEngine:
         batch's loss dict `lag` batches behind the one being enqueued.  Sum "bleu_counts" over the batches and pass them
         to losses.bleu_from_counts() for the BLEU of the whole dev set."""
         assert 0 <= lag < self.NSLOT
-        self._eval_setup()
         tf = float(teacher_forcing_prob)
         pending = []
         for inputs, lengths, labels in batches:
-            pending.append(self._enqueue_host_step(inputs, lengths, labels, eval_tf=tf))
+            pending.append(self._enqueue_host_step(inputs, lengths, labels, eval_tf=tf, where="eval_steps"))
             if len(pending) > lag:
                 slot = pending.pop(0)
                 self._slot_ev[slot].synchronize()
@@ -824,15 +955,19 @@ class TrainEngine:
 
     @property
     def eval_predictions(self):
-        """[B,T] token predictions of the last eval_step (device tensor; overwritten by the next one)."""
-        return self._eval["preds"] if self._eval is not None else None
+        """[B',T'] token predictions of the last eval_step's batch (device tensor; overwritten by the next one)."""
+        if self._eval_last is None:
+            return None
+        sh, T = self._eval_last
+        return sh.eval["preds"][:, :T]
 
     @property
     def token_predictions(self):
-        """[B,T] decoder inputs of the last step (vae/model.py:455-472): sampled where the coin said so."""
+        """[B',T'] decoder inputs of the last step's batch (vae/model.py:455-472): sampled where the coin said so."""
+        T = self._last_T
         if self.sampled:
-            return self.preds
-        p = self.inputs.clone()
+            return self.preds[:, :T]
+        p = self.inputs[:, :T].clone()
         p[:, 0] = self.model.sos_token_idx
         return p
 
@@ -899,7 +1034,7 @@ class TrainEngine:
 
     @property
     def h2d_bytes_per_step(self):
-        return self._stage_bytes
+        return self._sh.bytes
 
     @property
     def d2h_bytes_per_step(self):

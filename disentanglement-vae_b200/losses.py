@@ -162,12 +162,19 @@ def compute_mi_losses(model, latent_params, beta=1.0):
     return {"total_mi": total_mi, "idv_mi_estimates": idv_mi_estimates}
 
 
-def bleu_counts_(counts, refs, cands, eos_token_idx):
+def bleu_counts_(counts, refs, cands, eos_token_idx, t_max=None):
     """Adds the corpus-BLEU statistics of (refs [B,T_ref], cands [B,T_cand]), int64 device tensors, into `counts`
-    (int64 [10] device tensor, see dvae_bleu_counts) on the current stream."""
-    _lib.check(_lib.load().dvae_bleu_counts(refs.data_ptr(), refs.stride(0), refs.size(1), cands.data_ptr(), cands.stride(0),
-                                            cands.size(1), refs.size(0), int(eos_token_idx), counts.data_ptr(),
-                                            _lib.stream_ptr()), "dvae_bleu_counts")
+    (int64 [10] device tensor, see dvae_bleu_counts) on the current stream.  `t_max`: optional int32 device tensor [1]
+    that bounds both row lengths (dvae_bleu_counts_ex: rows padded beyond their batch's own length)."""
+    lib = _lib.load()
+    args = (refs.data_ptr(), refs.stride(0), refs.size(1), cands.data_ptr(), cands.stride(0), cands.size(1), refs.size(0),
+            int(eos_token_idx))
+    if t_max is None:
+        _lib.check(lib.dvae_bleu_counts(*args, counts.data_ptr(), _lib.stream_ptr()), "dvae_bleu_counts")
+    else:
+        assert t_max.dtype == torch.int32 and t_max.is_cuda
+        _lib.check(lib.dvae_bleu_counts_ex(*args, t_max.data_ptr(), counts.data_ptr(), _lib.stream_ptr()),
+                   "dvae_bleu_counts_ex")
     return counts
 
 

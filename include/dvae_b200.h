@@ -424,12 +424,18 @@ int dvae_recount_lengths(const int64_t* tokens, int64_t tok_stride_b, int64_t to
  *   dvae_bleu_counts: ADDS this batch's statistics into counts[10] = {clipped n-gram matches n = 1..4, candidate n-grams
  *                     n = 1..4, candidate length, reference length}, so a corpus accumulates over calls and ranks (zero the
  *                     counters first).  T_ref and T_cand may differ; each must be <= DVAE_BLEU_MAX_T (else DVAE_EINVAL).
+ *   dvae_bleu_counts_ex: dvae_bleu_counts with t_max (device memory, one int32; NULL = no bound): each row ends at
+ *                     min(T_ref, *t_max) resp. min(T_cand, *t_max) columns.  For rows padded beyond their batch's own
+ *                     length: a row without EOS is cut at the batch's length, as the unpadded row would be, so one
+ *                     captured call serves every padded length.
  *   dvae_bleu_score : score_out[0] = 0 if any clipped count is 0, else
  *                     exp(min(1 - ref_len / cand_len, 0)) * exp(sum_n 0.25 log(clipped_n / total_n)), in float64,
  *                     stored as float32 in device memory (one thread; capturable in a CUDA graph). */
 #define DVAE_BLEU_MAX_T 256
 int dvae_bleu_counts(const int64_t* ref, int64_t ref_stride, int T_ref, const int64_t* cand, int64_t cand_stride,
                      int T_cand, int B, int64_t eos, int64_t* counts, void* stream);
+int dvae_bleu_counts_ex(const int64_t* ref, int64_t ref_stride, int T_ref, const int64_t* cand, int64_t cand_stride,
+                        int T_cand, int B, int64_t eos, const int* t_max, int64_t* counts, void* stream);
 int dvae_bleu_score(const int64_t* counts, float* score_out, void* stream);
 
 /* Backward: d_h [N,H], d_w [V,H], d_bias [V] (all overwritten) for d(loss) = grad_scale_dev[0]
