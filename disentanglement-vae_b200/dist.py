@@ -106,3 +106,12 @@ def grad_buckets4(model, flat_grad):
     if hi != base + dec.numel() or lo <= base:          # decoder.linear.* must be the tail of the decoder range
         return [[], b[0], b[1], b[2]]
     return [[flat_grad[lo:hi]], [flat_grad[base:lo]], b[1], b[2]]
+
+
+def stage_buckets(model, flat_grad, n_stages):
+    """The gradient buckets of TrainEngine's train-step stages, one list of views per stage in stage order: grad_buckets4
+    for the four stages of a recurrent encoder of two or more layers, else decoder.* | everything else (two stages)."""
+    if n_stages == 4:
+        return grad_buckets4(model, flat_grad)
+    b3 = grad_buckets3(model, flat_grad)
+    return [b3[0], b3[1] + b3[2]]

@@ -1,9 +1,11 @@
 """Graph-captured data-parallel training engine: the reference's train-step body
 (`run.py:217-276`: forward -> compute_all_losses -> backward -> clip_grad_norm_(5.0) -> [adversary steps] ->
 Adam.step -> zero_grad -> [MI-estimator steps]) as one fixed sequence of C-ABI kernel launches over pre-allocated
-buffers, replayed as CUDA graphs.  When world_size > 1 the flat gradient buffer is summed over the ranks in four buckets
-by the repo's all-reduce kernel inside the one step graph (peer-to-peer at two ranks, NVSwitch multicast beyond), or,
-when its start-up self-test fails on any rank, by NCCL between stage graphs.
+buffers, replayed as CUDA graphs.  The forward + backward pass is one ordered list of stages (`TrainEngine._stage_list`),
+each ending where a bucket of the flat gradient buffer is final: four for a recurrent encoder of two or more layers, two
+otherwise.  One GPU runs the stages back to back.  When world_size > 1, bucket k is summed over the ranks from the end of
+stage k on: by the repo's all-reduce kernel inside the one step graph (four stages; peer-to-peer at two ranks, NVSwitch
+multicast beyond), or by NCCL between stage graphs (two stages, or when the kernel's start-up self-test fails on any rank).
 
 Same kernels and the same `StepPlan` as the drop-in autograd path (`functions.py`); what the engine removes is
 per-op host work (autograd bookkeeping, ctypes marshalling, allocator traffic).
@@ -27,6 +29,8 @@ on a `_Shape` of its own at (B', T) -- plan, staging block, graphs -- built on i
 gradients, Adam moments, weight planes, counters and random streams are shared.  A batch of the full shape (B, T) runs
 exactly the graph the engine had before any other shape was seen.
 """
+import functools
+import math
 import os
 import random
 from collections import OrderedDict
@@ -39,10 +43,7 @@ from . import _lib
 from ._lib import ptr, check
 from .plan import StepPlan, Dims
 from .losses import get_cyclic_kl_weight
-
-
-def d_bow(plan):
-    return bool(plan.d.bow)
+from .dist import stage_buckets
 
 
 class _Shape:
@@ -58,45 +59,55 @@ class _Shape:
         # on the device, so the captured step serves every length distribution); nothing the engine returns reads
         # vocabulary outputs at masked positions
         self.plan.live_rows = True
-        T1 = max(T - 1, 1)
         # Everything the host sends per step lives in ONE device block (typed views below) filled by ONE H2D copy from a ring
         # of pinned host blocks: token ids, lengths, Philox seed, labels, Adam / KL scalars, teacher-forcing coins.  An
         # asynchronous H2D copy reads host memory when it executes, so a slot is rewritten only after the event recorded
         # behind its last use has completed (ADVICE r1: un-synchronised step_resident calls saw a later step's scalars).
+        # One row per field: dtype and shape.  The fields follow each other at 16-byte boundaries, except the batch's own
+        # padded length T' (the BLEU kernel's row bound): word 5 of the scalar block, which the step does not read, so the
+        # block keeps its size.
+        fields = {"inputs": (torch.int64, (B, T)), "lengths": (torch.int64, (B,)), "seed": (torch.int64, (1,)),
+                  "labels": (torch.float32, (eng.n_dsc, B)), "scal": (torch.float32, (8 + max(d.S, 1),)),
+                  "coins": (torch.int32, (max(T - 1, 1),)),          # 1 = teacher-forced step
+                  "tlen": (torch.int32, (1,))}
         lay, off = {}, 0
-        for name, nbytes in (("inputs", B * T * 8), ("lengths", B * 8), ("seed", 8), ("labels", eng.n_dsc * B * 4),
-                             ("scal", (8 + max(d.S, 1)) * 4), ("coins", T1 * 4)):
-            lay[name] = (off, nbytes)
-            off = (off + nbytes + 15) // 16 * 16
-        # the batch's own padded length T' (int32; the BLEU kernel's row bound) in word 5 of the scalar block, which the
-        # step does not read: the block keeps its size
-        lay["tlen"] = (lay["scal"][0] + 5 * 4, 4)
+        for name, (dtype, shape) in fields.items():
+            nbytes = math.prod(shape) * dtype.itemsize
+            if name == "tlen":
+                lay[name] = (lay["scal"][0] + 5 * 4, nbytes)
+            else:
+                lay[name] = (off, nbytes)
+                off = (off + nbytes + 15) // 16 * 16
         self.bytes, self.lay = off, lay
-        self.d_stage = torch.zeros(off, device=dev, dtype=torch.uint8)
 
-        def view(buf, name, dtype, *shape):
-            o, n = lay[name]
-            return buf[o:o + n].view(dtype).view(*shape)
-        self.inputs = view(self.d_stage, "inputs", torch.int64, B, T)
-        self.lengths = view(self.d_stage, "lengths", torch.int64, B)
-        self.labels = view(self.d_stage, "labels", torch.float32, eng.n_dsc, B)
-        self.d_scal = view(self.d_stage, "scal", torch.float32, 8 + max(d.S, 1))
-        self.coins = view(self.d_stage, "coins", torch.int32, T1)          # 1 = teacher-forced step
+        def views(buf):
+            return {k: buf[o:o + n].view(fields[k][0]).view(fields[k][1]) for k, (o, n) in lay.items()}
+        self.d_stage = torch.zeros(off, device=dev, dtype=torch.uint8)
+        dv = views(self.d_stage)
+        self.inputs, self.lengths, self.labels, self.d_scal, self.coins, self.tlen = (
+            dv[k] for k in ("inputs", "lengths", "labels", "scal", "coins", "tlen"))
         self.coins.fill_(1)
-        self.tlen = view(self.d_stage, "tlen", torch.int32, 1)
-        self.plan.seed_dev = view(self.d_stage, "seed", torch.int64, 1)     # the plan's kernels read the seed from here
+        self.plan.seed_dev = dv["seed"]     # the plan's kernels read the seed from here
         self.preds = torch.zeros(B, T, device=dev, dtype=torch.int64) if eng.sampled else None
         self.h_stage = torch.zeros(eng.NSLOT, off, dtype=torch.uint8).pin_memory()
-        self.hv = [{k: view(self.h_stage[i], k, dt, *shp).numpy() for k, dt, shp in
-                    (("inputs", torch.int64, (B, T)), ("lengths", torch.int64, (B,)), ("seed", torch.int64, (1,)),
-                     ("labels", torch.float32, (eng.n_dsc, B)), ("scal", torch.float32, (8 + max(d.S, 1),)),
-                     ("coins", torch.int32, (T1,)), ("tlen", torch.int32, (1,)))} for i in range(eng.NSLOT)]
+        self.hv = [{k: v.numpy() for k, v in views(h).items()} for h in self.h_stage]
         for hv in self.hv:
             hv["coins"][:] = 1
             hv["lengths"][:] = 1
             hv["tlen"][:] = T
         self.graphs = None     # captured train step: one graph, or the data-parallel stage graphs
         self.eval = None       # evaluation buffers and graphs, allocated on this shape's first eval_step
+
+
+class _Carry:
+    """The values one stage of a train step hands to a later one (TrainEngine._stages)."""
+
+    def __init__(self, g_z=None):
+        # extra gradient on the sampled latents [B, Z] (adversarial / MI objectives), or a callable evaluated after the forward
+        self.g_z = g_z
+        self.g_top = None             # d(loss)/d(decoder top-layer states): vocabulary backward -> decoder backward
+        self.g_ctx = None             # d(loss)/d(encoder context): heads backward -> encoder backward
+        self.side_pending = False     # the decoder's embedding-gradient scatter still runs on the hoist side stream
 
 
 class TrainEngine:
@@ -131,10 +142,10 @@ class TrainEngine:
         self.n = model._flat_numel
         f32 = dict(device=self.device, dtype=torch.float32)
         self.flat = model._flat[:self.n]
-        self.use_graph = use_graph
+        self.use_graph = use_graph and not self.aux
         self._nvls = None
         # DVAE_DP_NVLS=0 skips the exchange kernel: the one way to run the NCCL fallback where the kernel works (tests)
-        if self.world > 1 and use_graph and not self.aux and os.environ.get("DVAE_DP_NVLS", "1") != "0":
+        if self.world > 1 and self.use_graph and os.environ.get("DVAE_DP_NVLS", "1") != "0":
             self._setup_nvls()          # gradient buffer in multicast memory (self.grad), or None: NCCL exchanges
         if self._nvls is None:
             self.grad = torch.zeros(self.n, **f32)
@@ -171,10 +182,10 @@ class TrainEngine:
         # evaluation draws its eps / coins from streams of its own, so that eval_step never shifts the training streams
         self._eval_gen = torch.Generator().manual_seed(base + 0x5EED)
         self._eval_pyrand = random.Random(base + 0x5EED)
-        self.use_graph = use_graph and not self.aux
-        self._buckets = None
-        self._comm = None
-        self._xchg_in_capture = False      # one-graph data parallel: the step being captured exchanges inside the graph
+        self._stages = self._stage_list()
+        if self.world > 1:          # bucket k: the gradients final once stage k has run, summed over the ranks from there
+            self._buckets = stage_buckets(model, self.grad, len(self._stages))
+            self._comm = torch.cuda.Stream(device=self.device)
         # step counter in device memory, from which the exchange kernels derive their barrier epochs
         self._dp_ctr = torch.zeros(1, dtype=torch.int32, device=self.device)
         self._side = None
@@ -264,7 +275,11 @@ class TrainEngine:
         _lib.planes_owner = self._plane_token
 
     # ---- the kernel sequences ------------------------------------------------------------------
-    def _forward(self, fork_ok=True, train=True, sampled=None, preds=None):
+    def _hoisted(self, sampled):
+        """Whether the decoder's encoder-independent work runs on the hoist side stream (self._side) in a step."""
+        return os.environ.get("DVAE_HOIST", "1") != "0" and not self.d.bow and not sampled
+
+    def _forward(self, train=True, sampled=None, preds=None):
         """Forward pass of one step up to the reconstruction loss.  The defaults are the training step; eval_step passes
         train=False (no dropout) and its own decode regime / prediction buffer."""
         pl, P, m = self.plan, self.model._P, self.model
@@ -284,7 +299,7 @@ class TrainEngine:
         # the decoder's input embeddings, its layer-0 input projection and the W_out operand planes do not depend on
         # the encoder (teacher forcing): they run on a side stream under the encoder's recurrences (64 of 148 SMs)
         cur = torch.cuda.current_stream()
-        hoist = fork_ok and os.environ.get("DVAE_HOIST", "1") != "0" and not d_bow(pl) and not sampled
+        hoist = self._hoisted(sampled)
         # W_out^T planes (10 MB at cfg 2) are read by the vocabulary backward only: not refreshed for an evaluation
         refresh_wt = n_pl > n_ih and train
         fork_prep = None
@@ -313,73 +328,74 @@ class TrainEngine:
         else:
             h_top = pl.decode_forced(P, self.inputs, m.sos_token_idx, train)
         pl.vocab_ce(P, h_top, self.inputs, self.lengths)
-        return h_top, hoist
+        return h_top
 
-    def _fwd_bwd(self, part=None, g_z=None):
-        """part = None: the whole forward + backward; 1: forward, vocabulary backward and decoder backward (every
-        decoder.* gradient final); 2: heads and encoder backward.  The split lets the all-reduce of the decoder
-        gradients (half of the parameters) run under part 2 when training data-parallel.  `g_z` [B,Z]: extra gradient
-        on the sampled latents (adversarial / MI objectives); a callable is evaluated after the forward pass."""
-        pl, P, G, m = self.plan, self.model._P, self.G, self.model
-        st = _lib.stream_ptr()
-        cur = torch.cuda.current_stream()
-        # part 0 (data parallel only): forward + vocabulary backward on their own, so that W_out's gradient is exchanged first
-        xchg = self._xchg_in_capture and part is None      # one-graph data parallel: the exchanges inside the graph
-        if xchg:
-            check(self.lib.dvae_counter_increment(ptr(self._dp_ctr), st), "dvae_counter_increment")
-        if part == 0 or part is None or (part == 1 and not self._three_buckets()):
-            h_top, hoist = self._forward()
-            if callable(g_z):
-                g_z = g_z()
-            self._g_z = g_z
-            self._g_top = pl.vocab_ce_bwd(P, G, h_top, self.inputs, self.lengths, None)
-            self._hoist = hoist
-            if part == 0:
-                check(self.lib.dvae_join_side_streams(st), "dvae_join_side_streams")      # d_w runs on a side stream
-                return
-            if xchg:
-                self._signal(0, True)
-        if part in (None, 1):
-            g_top, hoist = self._g_top, self._hoist
-            # weight-gradient GEMMs of each layer keep running on side streams while the next layer's recurrence starts
-            check(self.lib.dvae_defer_joins(1), "dvae_defer_joins")
-            try:
-                pl.decode_bwd(P, G, g_top, emb_grad="decoder.embedding.weight" in m._layout,
-                              aux_stream=self._side if hoist else None)
-            finally:
-                if part == 1:
-                    check(self.lib.dvae_join_side_streams(st), "dvae_join_side_streams")
-                    if hoist:
-                        cur.wait_stream(self._side)
-            self._aux_pending = hoist and part is None
-            if xchg:
-                self._signal(1, True, self._side if hoist else None)
-        emb_enc = "encoder.embedding.weight" in m._layout
-        if part in (None, 2):
-            check(self.lib.dvae_defer_joins(1), "dvae_defer_joins")
-            try:
-                g_ctx = pl.heads_bwd(P, G, pl.ctx, pl.eps, self.labels, self.kl_w, pl.g_hid, g_z=getattr(self, "_g_z", None))
-                if getattr(self, "_aux_pending", False):      # the decoder's embedding-gradient scatter still reads g_dx[0]
-                    torch.cuda.current_stream().wait_stream(self._side)
-                    self._aux_pending = False
-                self._g_ctx = g_ctx
-                # data parallel with a multi-layer encoder: stop after the upper layers (their gradients go out under layer 0)
-                split = part == 2 and self._three_buckets()
-                if xchg:
-                    pl.encode_bwd(P, G, self.inputs, self.lengths, g_ctx, emb_grad=emb_enc, layers=(pl.d.Le - 1, 1))
-                    self._signal(2, True)
-                    pl.encode_bwd(P, G, self.inputs, self.lengths, g_ctx, emb_grad=emb_enc, layers=(0, 0))
-                    self._signal(3, True)
-                else:
-                    pl.encode_bwd(P, G, self.inputs, self.lengths, g_ctx, emb_grad=emb_enc, layers=(pl.d.Le - 1, 1) if split else None)
-            finally:
-                check(self.lib.dvae_join_side_streams(st), "dvae_join_side_streams")
-        if part == 3:
-            check(self.lib.dvae_defer_joins(1), "dvae_defer_joins")
-            try:
-                pl.encode_bwd(P, G, self.inputs, self.lengths, self._g_ctx, emb_grad=emb_enc, layers=(0, 0))
-            finally:
-                check(self.lib.dvae_join_side_streams(st), "dvae_join_side_streams")
+    # The train step's forward + backward pass is a list of stages (_stage_list); stage k ends with gradient bucket k final
+    # (dist.stage_buckets), which data-parallel training sums over the ranks from there.  Stages pass values on in a _Carry.
+    def _stage_list(self):
+        """A recurrent encoder of two or more layers: forward + vocabulary backward (-> decoder.linear.*) | decoder
+        backward (-> decoder embedding + LSTM) | heads + encoder layers Le-1..1 (-> upper encoder + heads) | encoder layer
+        0 + embedding (-> the rest).  Bag-of-words or one-layer encoders: forward + vocabulary and decoder backward (->
+        decoder.*) | heads + encoder (-> the rest).  Each stage is a tuple of pieces run in order."""
+        d = self.d
+        if d.bow or d.Le < 2:
+            return ((self._fwd_vocab_bwd, self._decoder_bwd), (self._heads_encoder_bwd,))
+        upper = functools.partial(self._heads_encoder_bwd, layers=(d.Le - 1, 1))
+        return ((self._fwd_vocab_bwd,), (self._decoder_bwd,), (upper,), (self._encoder_l0_bwd,))
+
+    def _fwd_vocab_bwd(self, c):
+        h_top = self._forward()
+        if callable(c.g_z):
+            c.g_z = c.g_z()
+        c.g_top = self.plan.vocab_ce_bwd(self.model._P, self.G, h_top, self.inputs, self.lengths, None)
+
+    def _decoder_bwd(self, c):
+        # weight-gradient GEMMs of each layer keep running on side streams while the next layer's recurrence starts
+        check(self.lib.dvae_defer_joins(1), "dvae_defer_joins")
+        c.side_pending = self._hoisted(self.sampled)
+        self.plan.decode_bwd(self.model._P, self.G, c.g_top, emb_grad="decoder.embedding.weight" in self.model._layout,
+                             aux_stream=self._side if c.side_pending else None)
+
+    def _heads_encoder_bwd(self, c, layers=None):
+        pl = self.plan
+        check(self.lib.dvae_defer_joins(1), "dvae_defer_joins")
+        c.g_ctx = pl.heads_bwd(self.model._P, self.G, pl.ctx, pl.eps, self.labels, self.kl_w, pl.g_hid, g_z=c.g_z)
+        if c.side_pending:          # the decoder's embedding-gradient scatter still reads g_dx[0]
+            torch.cuda.current_stream().wait_stream(self._side)
+            c.side_pending = False
+        pl.encode_bwd(self.model._P, self.G, self.inputs, self.lengths, c.g_ctx,
+                      emb_grad="encoder.embedding.weight" in self.model._layout, layers=layers)
+
+    def _encoder_l0_bwd(self, c):
+        check(self.lib.dvae_defer_joins(1), "dvae_defer_joins")
+        self.plan.encode_bwd(self.model._P, self.G, self.inputs, self.lengths, c.g_ctx,
+                             emb_grad="encoder.embedding.weight" in self.model._layout, layers=(0, 0))
+
+    def _fwd_bwd(self, c, stages=None, after_stage=None):
+        """Runs `stages` (default: all of them, the whole forward + backward pass) back to back, passing values on in the
+        _Carry `c`: side-stream work stays detached until their end, where every side stream is joined.
+        `after_stage(k, c)` runs at the end of stage k."""
+        try:
+            for k, stage in enumerate(self._stages if stages is None else stages):
+                for piece in stage:
+                    piece(c)
+                if after_stage is not None:
+                    after_stage(k, c)
+        finally:
+            check(self.lib.dvae_join_side_streams(_lib.stream_ptr()), "dvae_join_side_streams")
+        if c.side_pending:          # the decoder's stage run on its own: its embedding-gradient scatter is joined too
+            torch.cuda.current_stream().wait_stream(self._side)
+            c.side_pending = False
+
+    def _step(self, exchange=False):
+        """forward + backward + clip + Adam.  exchange (one-graph data parallel): each bucket's exchange starts inside the
+        step, at the end of its stage."""
+        after_stage = None
+        if exchange:
+            check(self.lib.dvae_counter_increment(ptr(self._dp_ctr), _lib.stream_ptr()), "dvae_counter_increment")
+            after_stage = lambda k, c: self._signal(k, self._side if c.side_pending else None)      # noqa: E731
+        self._fwd_bwd(_Carry(), after_stage=after_stage)
+        self._optim()
 
     def _setup_nvls(self):
         """The flat gradient buffer as a symmetric allocation bound to an NVSwitch multicast object, plus a barrier block,
@@ -447,18 +463,18 @@ class TrainEngine:
         self.grad = st["buf"][:self.n]
         self._nvls = st
 
-    # CTAs of the exchange kernel per bucket: early buckets finish under hundreds of us of backward pass, the last one is
-    # (nearly) exposed
+    # CTAs of the exchange kernel per bucket of the four-stage step: early buckets finish under hundreds of us of backward
+    # pass, the last one is (nearly) exposed
     XCHG_CTAS = (16, 16, 32, 64)
 
-    def _signal(self, k, include_sides, extra=None):
-        """Bucket k's gradients are final once everything enqueued so far (and, include_sides, the detached side-stream
-        work and `extra`) has run: start its exchange there, beside the rest of the backward pass -- as graph nodes on the
-        library's signal stream, one all-reduce kernel per view."""
+    def _signal(self, k, extra=None):
+        """Bucket k's gradients are final once everything enqueued so far, the detached side-stream work and `extra` have
+        run: start its exchange there, beside the rest of the backward pass -- as graph nodes on the library's signal
+        stream, one all-reduce kernel per view."""
         import ctypes as C
         out = C.c_void_p()
-        check(self.lib.dvae_fork_after(1 if include_sides else 0, extra.cuda_stream if extra is not None else None,
-                                       _lib.stream_ptr(), C.byref(out)), "dvae_fork_after")
+        check(self.lib.dvae_fork_after(1, extra.cuda_stream if extra is not None else None, _lib.stream_ptr(), C.byref(out)),
+              "dvae_fork_after")
         nv = self._nvls
         ctas = self.XCHG_CTAS[k]
         for j, v in enumerate(self._buckets[k]):
@@ -476,7 +492,7 @@ class TrainEngine:
         """Data parallel as ONE graph per step, the exchanges being the repo's all-reduce kernels inside it (csrc/nvls.cu):
         needs the kernel set up, graphs on and the four-bucket split.  Otherwise: stage graphs (or eager stages) with NCCL
         between them, whose ends also end the overlap of the weight-gradient GEMMs with the next recurrence."""
-        return self._nvls is not None and self.use_graph and self._three_buckets()
+        return self._nvls is not None and self.use_graph and len(self._stages) == len(self.XCHG_CTAS)
 
     @property
     def exchange_mode(self):
@@ -485,19 +501,6 @@ class TrainEngine:
         if self.world == 1:
             return "none"
         return self._nvls["mode"] if self._one_graph_dp() else "nccl+stages"
-
-    def _ensure_buckets(self):
-        if self._buckets is None:
-            from .dist import grad_buckets4, grad_buckets3
-            if self._three_buckets():
-                self._buckets = grad_buckets4(self.model, self.grad)
-            else:
-                b3 = grad_buckets3(self.model, self.grad)
-                self._buckets = [b3[0], b3[1] + b3[2]]
-            self._comm = torch.cuda.Stream(device=self.device)
-
-    def _three_buckets(self):
-        return self.world > 1 and not self.plan.d.bow and self.plan.d.Le >= 2
 
     def _optim(self):
         st = _lib.stream_ptr()
@@ -533,7 +536,7 @@ class TrainEngine:
             box.update(A=A, M=M, z=z)
             return z.grad.contiguous() if z.grad is not None else None
 
-        self._fwd_bwd(None, g_z=aux_grad)
+        self._fwd_bwd(_Carry(g_z=aux_grad))
         A, M, z = box["A"], box["M"], box["z"]
         for name, dsc_loss in A["idv_adv_dsc_losses"].items():      # run.py:256-260
             m.adversaries[name].optimizer_step(dsc_loss)
@@ -582,36 +585,26 @@ class TrainEngine:
     def _run_inner(self):
         if self.aux:
             return self._run_aux()
-        if self.world == 1:
-            if not self.use_graph:
-                self._fwd_bwd()
-                self._optim()
-                return
-            if self._sh.graphs is None:
-                self._capture()
-            self._sh.graphs[0].replay()          # one graph: forward, backward, clip + Adam
-            return
-        # data parallel: gradients are all-reduced in the order the backward pass finishes them, on a communication stream,
-        # under the rest of the backward pass: W_out | decoder embedding + LSTM | upper encoder layers + heads | encoder
-        # embedding + layer 0 (four stages); bag-of-words or one-layer encoders: decoder | everything else (two stages)
-        self._ensure_buckets()
-        cur = torch.cuda.current_stream()
         if self.use_graph and self._sh.graphs is None:
             self._capture()
-        if self._one_graph_dp():      # the exchanges are nodes of the graph
-            self._sh.graphs[0].replay()
-            return
-        # NCCL on the communication stream between stage graphs (or eager stages); stage gi finishes bucket gi
-        stages = (0, 1, 2, 3) if self._three_buckets() else (1, 2)
-        for gi, part in enumerate(stages):
+        if self.world == 1 or self._one_graph_dp():
             if self.use_graph:
-                self._sh.graphs[gi].replay()
+                self._sh.graphs[0].replay()      # one graph: forward, backward (and the exchanges), clip + Adam
             else:
-                self._fwd_bwd(part)
-            if self._buckets[gi]:
+                self._step()
+            return
+        # NCCL on the communication stream between stage graphs (or eager stages), under the stages that follow
+        cur = torch.cuda.current_stream()
+        c = _Carry()
+        for k, bucket in enumerate(self._buckets):
+            if self.use_graph:
+                self._sh.graphs[k].replay()
+            else:
+                self._fwd_bwd(c, [self._stages[k]])
+            if bucket:
                 self._comm.wait_stream(cur)
                 with torch.cuda.stream(self._comm):
-                    for v in self._buckets[gi]:
+                    for v in bucket:
                         dist.all_reduce(v, op=dist.ReduceOp.SUM, group=self.pg)
         cur.wait_stream(self._comm)
         if self.use_graph:
@@ -619,51 +612,41 @@ class TrainEngine:
         else:
             self._optim()
 
-    def _capture(self):
-        # warm up eagerly on a side stream (lazy module loading, cudaFuncSetAttribute, allocator), then capture the current
-        # shape's step.  The warm-up runs no gradient exchange (data parallel: the graph holds it, or NCCL runs between
-        # the stage graphs), so one rank capturing a new shape never waits on another
-        snap = (self.flat.clone(), self.m.clone(), self.v.clone())
+    def _graphs(self, warm_up, bodies):
+        """Runs warm_up() eagerly on a side stream (lazy module loading, cudaFuncSetAttribute, allocator, workspaces),
+        synchronises, then captures each of `bodies` as a CUDA graph on that stream."""
         s = torch.cuda.Stream(device=self.device)
         s.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(s):
-            for _ in range(2):
-                self._fwd_bwd()
-                self._optim()
+            warm_up()
         torch.cuda.current_stream().wait_stream(s)
         torch.cuda.synchronize()
         graphs = []
-        if self.world == 1:
+        for body in bodies:
             g = torch.cuda.CUDAGraph()
             with torch.cuda.graph(g, stream=s):
-                self._fwd_bwd(None)
-                self._optim()
+                body()
             graphs.append(g)
-        elif self._one_graph_dp():
-            g = torch.cuda.CUDAGraph()
-            self._xchg_in_capture = True
-            try:
-                with torch.cuda.graph(g, stream=s):
-                    self._fwd_bwd(None)
-                    self._optim()
-            finally:
-                self._xchg_in_capture = False
-            graphs.append(g)
-        else:                 # the all-reduces sit between the graphs (NCCL on its own stream)
-            for part in ((0, 1, 2, 3) if self._three_buckets() else (1, 2)):
-                g = torch.cuda.CUDAGraph()
-                with torch.cuda.graph(g, stream=s):
-                    self._fwd_bwd(part)
-                graphs.append(g)
-            gb = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(gb, stream=s):
-                self._optim()
-            graphs.append(gb)
         torch.cuda.synchronize()
+        return tuple(graphs)
+
+    def _capture(self):
+        """Captures the current shape's train step.  The warm-up runs no gradient exchange (data parallel: the graph holds
+        it, or NCCL runs between the stage graphs), so one rank capturing a new shape never waits on another."""
+        def warm_up():
+            for _ in range(2):
+                self._step()
+        snap = (self.flat.clone(), self.m.clone(), self.v.clone())
+        if self.world == 1 or self._one_graph_dp():
+            bodies = [functools.partial(self._step, exchange=self.world > 1)]
+        else:                 # the all-reduces sit between the graphs (NCCL on its own stream)
+            c = _Carry()
+            bodies = [functools.partial(self._fwd_bwd, c, [stage]) for stage in self._stages] + [self._optim]
+        graphs = self._graphs(warm_up, bodies)
         # undo the warm-up updates so that capture leaves the training state untouched
         self.flat.copy_(snap[0]); self.m.copy_(snap[1]); self.v.copy_(snap[2])
         self.grad.zero_()
-        self._sh.graphs = tuple(graphs)
+        self._sh.graphs = graphs
 
     # ---- per-step host scalars -----------------------------------------------------------------
     def _acquire_slot(self):
@@ -711,6 +694,32 @@ class TrainEngine:
         ev.record()
         self._slot_ev[slot] = ev
 
+    def _train_step(self, slot, T, h_out=None):
+        """Runs the train step on the staged batch of padded length T (and copies its result block into h_out), releases
+        `slot` behind it and advances the step counters."""
+        self._last_T = T
+        self._run()
+        if h_out is not None:
+            h_out.copy_(self.plan.out, non_blocking=True)
+        self._release_slot(slot)
+        self.step_idx += 1
+        self.adam_step += 1
+
+    def _pipelined(self, batches, lag, enqueue, result):
+        """enqueue(inputs, lengths, labels) -> slot for every batch; yields result(slot) of each, in order, `lag` batches
+        behind the one being enqueued: nothing waits for the device but the read of a result `lag` steps old."""
+        assert 0 <= lag < self.NSLOT
+        pending = []
+        for inputs, lengths, labels in batches:
+            pending.append(enqueue(inputs, lengths, labels))
+            if len(pending) > lag:
+                slot = pending.pop(0)
+                self._slot_ev[slot].synchronize()
+                yield result(slot)
+        for slot in pending:
+            self._slot_ev[slot].synchronize()
+            yield result(slot)
+
     # ---- public entry points -------------------------------------------------------------------
     def step_resident(self, inputs_dev, lengths_dev, labels_dev):
         """One train step on a batch already in HBM (inputs [B',T'] int64, lengths [B'], labels [n_dsc,B']); returns the
@@ -739,11 +748,7 @@ class TrainEngine:
             self.inputs[:, T:].zero_()
         self.lengths.copy_(lengths_dev, non_blocking=True)
         self.labels.copy_(labels_dev, non_blocking=True)
-        self._last_T = T
-        self._run()
-        self._release_slot(slot)
-        self.step_idx += 1
-        self.adam_step += 1
+        self._train_step(slot, T)
         return self.plan.out
 
     def _enqueue_host_step(self, inputs, lengths, labels, eval_tf=None, where="step_host"):
@@ -776,12 +781,7 @@ class TrainEngine:
             ev["aux"][slot] = self._eval_aux() if self.aux else None
             self._release_slot(slot)
             return slot
-        self._last_T = T
-        self._run()
-        self.h_outs[slot].copy_(self.plan.out, non_blocking=True)
-        self._release_slot(slot)
-        self.step_idx += 1
-        self.adam_step += 1
+        self._train_step(slot, T, self.h_outs[slot])
         return slot
 
     def step_host(self, inputs, lengths, labels):
@@ -800,17 +800,8 @@ class TrainEngine:
         calling step_host() per batch (run.py:217-262), with the same batch shapes; `lag` must be smaller than NSLOT.
         Data parallel: every rank's batches have the same shapes step by step (RatioSampler's default drop_uneven=True
         gives equal shards of a short last batch); unequal shards are not supported."""
-        assert 0 <= lag < self.NSLOT
-        pending = []
-        for inputs, lengths, labels in batches:
-            pending.append(self._enqueue_host_step(inputs, lengths, labels, where="train_steps"))
-            if len(pending) > lag:
-                slot = pending.pop(0)
-                self._slot_ev[slot].synchronize()
-                yield self.losses_from(self.h_outs[slot])
-        for slot in pending:
-            self._slot_ev[slot].synchronize()
-            yield self.losses_from(self.h_outs[slot])
+        return self._pipelined(batches, lag, functools.partial(self._enqueue_host_step, where="train_steps"),
+                               lambda slot: self.losses_from(self.h_outs[slot]))
 
     def losses_from(self, out, aux=None):
         """The loss dict of `compute_all_losses` from a result block; `aux`: the adversarial / MI values to add (default:
@@ -866,24 +857,14 @@ class TrainEngine:
         bleu_score_(ev["out"][NS + 1:NS + 2], ev["counts"])
 
     def _eval_run(self, sampled):
-        ev = self._eval           # the current shape's: its graphs are keyed by decode regime
+        graphs = self._eval["graphs"]      # the current shape's, keyed by decode regime
+        body = functools.partial(self._eval_body, sampled)
         if not self.use_graph:
-            self._eval_body(sampled)
+            body()
         else:
-            g = ev["graphs"].get(sampled)
-            if g is None:      # warm up eagerly (lazy module loading, workspaces), then capture; nothing to undo
-                s = torch.cuda.Stream(device=self.device)
-                s.wait_stream(torch.cuda.current_stream())
-                with torch.cuda.stream(s):
-                    self._eval_body(sampled)
-                torch.cuda.current_stream().wait_stream(s)
-                torch.cuda.synchronize()
-                g = torch.cuda.CUDAGraph()
-                with torch.cuda.graph(g, stream=s):
-                    self._eval_body(sampled)
-                torch.cuda.synchronize()
-                ev["graphs"][sampled] = g
-            g.replay()
+            if sampled not in graphs:      # nothing to undo after the warm-up
+                graphs[sampled], = self._graphs(body, [body])
+            graphs[sampled].replay()
         if self.world > 1:
             self._eval_all_reduce()
 
@@ -940,18 +921,8 @@ class TrainEngine:
         """eval_step over an iterable of HOST batches (inputs, lengths, labels), pipelined as train_steps: yields each
         batch's loss dict `lag` batches behind the one being enqueued.  Sum "bleu_counts" over the batches and pass them
         to losses.bleu_from_counts() for the BLEU of the whole dev set."""
-        assert 0 <= lag < self.NSLOT
-        tf = float(teacher_forcing_prob)
-        pending = []
-        for inputs, lengths, labels in batches:
-            pending.append(self._enqueue_host_step(inputs, lengths, labels, eval_tf=tf, where="eval_steps"))
-            if len(pending) > lag:
-                slot = pending.pop(0)
-                self._slot_ev[slot].synchronize()
-                yield self._eval_losses(slot)
-        for slot in pending:
-            self._slot_ev[slot].synchronize()
-            yield self._eval_losses(slot)
+        enqueue = functools.partial(self._enqueue_host_step, eval_tf=float(teacher_forcing_prob), where="eval_steps")
+        return self._pipelined(batches, lag, enqueue, self._eval_losses)
 
     @property
     def eval_predictions(self):

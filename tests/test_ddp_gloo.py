@@ -160,3 +160,27 @@ def test_four_stage_split_puts_the_output_layer_first(dvae):
     assert sum(v.numel() for v in b[0]) >= n_lin and sum(v.numel() for v in b[0]) <= n_lin + 8
     off = vae._layout["decoder.linear.weight"]
     assert b[0][0].data_ptr() == flat.data_ptr() + 4 * off
+
+
+def test_two_stage_split_covers_flat_gradient_exactly_once(dvae):
+    """stage_buckets of a two-stage step (bag-of-words and one-layer encoders): decoder.* | everything else."""
+    import importlib
+    dvae_dist = importlib.import_module("disentanglement-vae_b200.dist")
+    for bow, layers in ((True, 1), (False, 1)):
+        p = dict(bow_encoder=bow, embedding_dim=12, hidden_dim=16, num_rnn_layers=layers, encoder_dropout=0.0,
+                 decoder_dropout=0.0, bidirectional_encoder=True, latent_dims={"total": 7, "polarity": 1, "uncertainty": 2},
+                 adversarial_loss=False, mi_loss=False)
+        vae = dvae.build_vae(p, 29, None, {"uncertainty": 3, "polarity": 1}, torch.device("cpu"), 2, 3)
+        flat = torch.zeros(vae._flat_numel)
+        buckets = dvae_dist.stage_buckets(vae, flat, 2)
+        assert len(buckets) == 2
+        named = dict(vae.named_parameters())
+        for i, views in enumerate(buckets):
+            for v in views:
+                v += 1.0
+                off = (v.data_ptr() - flat.data_ptr()) // 4
+                for name, o in vae._layout.items():
+                    if off <= o < off + v.numel():
+                        assert name.startswith("decoder.") == (i == 0), (bow, name, i)
+        assert torch.equal(flat, torch.ones_like(flat))              # every element in exactly one bucket
+        assert sum(v.numel() for v in buckets[0]) >= sum(q.numel() for k, q in named.items() if k.startswith("decoder."))
