@@ -67,6 +67,7 @@ SIGNATURES = {
     "dvae_lstm_seq_bwd": (_i, [_p, _l, _i, _i, _i, _i, _i, _pp, _pp, _p, _p, _l, _l, _p, _p, _l, _p, _p, _p, _l,
                                _p, _p, _l, _l, _p, _l, _pp, _pp, _pp, _pp, _p, _p, _l, _l, _p, _p]),
     "dvae_lstm_bwd_planes_ws_floats": (_l, [_i, _i, _i, _i, _i]),
+    "dvae_lstm_bwd_dx_stream": (_i, [_p]),
     "dvae_lstm_seq_bwd_ex": (_i, [_p, _l, _i, _i, _i, _i, _i, _pp, _pp, _p, _p, _l, _l, _p, _p, _l, _p, _p, _p, _l,
                                   _p, _p, _l, _l, _p, _l, _pp, _pp, _pp, _pp, _p, _p, _l, _l, _p, _p, _p]),
     "dvae_counter_increment": (_i, [_p, _p]),

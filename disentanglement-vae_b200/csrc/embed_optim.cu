@@ -108,6 +108,9 @@ __global__ void bow_max_bwd_kernel(const float* __restrict__ d_ctx, int64_t ldd,
 
 __global__ void dropout_kernel(const float* __restrict__ x, int64_t ldx, int64_t rows, int width, float p,
                                const uint64_t* seed_dev, uint32_t salt, float* __restrict__ y, int64_t ldy, int64_t row0) {
+  // the recurrence that follows a layer's dropout is launched programmatically: it may start its prologue now and waits
+  // for this grid to complete before it reads y
+  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
   const int w4n = (width + 3) / 4;
   const int64_t total4 = rows * w4n;
   const uint64_t seed = (p > 0.f && seed_dev) ? *seed_dev : 0;

@@ -337,6 +337,9 @@ int lstm_seq_fwd_impl(const float* x, int64_t ldx, int T, int B, int I, int H, i
   return DVAE_OK;
 }
 
+// dvae_lstm_bwd_dx_stream: where the d_x GEMM of a unidirectional layer's backward runs (nullptr: the call's stream)
+static thread_local cudaStream_t g_dx_stream = nullptr;
+
 int lstm_seq_bwd_impl(const float* x, int64_t ldx, int T, int B, int I, int H, int D, const float* const* w_ih,
                       const float* const* w_hh, const float* h0, const float* c0, int64_t ld0, int64_t dir0,
                       const int64_t* lengths, const float* hs, int64_t ldhs, float* gates, const float* cs,
@@ -427,7 +430,8 @@ int lstm_seq_bwd_impl(const float* x, int64_t ldx, int T, int B, int I, int H, i
   gh.a_amax_n = amax_n;
   // the weight-gradient GEMMs below run on side streams beside the NEXT layer's recurrence (deferred joins): sized to leave
   // that recurrence its SMs (64 at cfg 2).  Two machine-filling split-K grids (2 x 144 CTAs) kept the recurrence kernel
-  // from being scheduled for 25-40 us at every layer boundary.
+  // from being scheduled for 25-40 us at every layer boundary.  (Caps derived from the SMs the recurrence leaves, 42 per
+  // GEMM or 28 with d_x beside them, measured slower at cfg 2: 1.064 against 1.042 ms per step.)
   GemmHints gh_bg = gh;
   {
     static const int cap = [] { const char* e = getenv("DVAE_DW_MAX_CTAS"); return e ? atoi(e) : 48; }();
@@ -436,6 +440,9 @@ int lstm_seq_bwd_impl(const float* x, int64_t ldx, int T, int B, int I, int H, i
     // 2.3 % there (cfg 4: 25.70 ms capped, 25.10 ms uncapped).
     gh_bg.max_ctas = (defer_joins_enabled() && tc_lstm_supported(H)) ? cap : 0;
   }
+  // a unidirectional layer's d_x on the caller-named stream (dvae_lstm_bwd_dx_stream), ordered after the recurrence: a
+  // background GEMM there, sized like the weight gradients
+  const bool dx_bg = d_x && D == 1 && g_dx_stream && g_dx_stream != st;
   // d_x accumulates over the directions (main stream, in order); the weight / bias gradients of each direction are
   // independent of it and of each other: parallel branches
   Fork fork(st);
@@ -480,14 +487,25 @@ int lstm_seq_bwd_impl(const float* x, int64_t ldx, int T, int B, int I, int H, i
     if (rc) return rc;
     if ((rc = fork.chain(0, 1))) return rc;
   }
+  cudaStream_t dx_st = st;
+  if (dx_bg) {
+    static thread_local cudaEvent_t ev[64] = {};
+    int dev = 0;
+    DVAE_CUDA(cudaGetDevice(&dev));
+    DVAE_REQUIRE(dev >= 0 && dev < 64, "dvae_lstm_seq_bwd: device %d", dev);
+    if (!ev[dev]) DVAE_CUDA(cudaEventCreateWithFlags(&ev[dev], cudaEventDisableTiming));
+    DVAE_CUDA(cudaEventRecord(ev[dev], st));
+    DVAE_CUDA(cudaStreamWaitEvent(g_dx_stream, ev[dev], 0));
+    dx_st = g_dx_stream;
+  }
   for (int d = 0; d < D; ++d) {
     const float* dG = gates + d * slab;
     int rc;
     if (d_x && !(dx_pair && d == 1)) {
-      GemmHints ghx = gh;
+      GemmHints ghx = dx_st == st ? gh : gh_bg;
       ghx.c_zeroed = dx_zeroed;
       if (dx_pair) { ghx.atomic_out = true; ghx.concurrency = 2; }
-      rc = linear_impl_ex(dG, 4 * H, 0, w_ih[d], I, 1, d_x, lddx, T * B, I, 4 * H, nullptr, nullptr, (d == 0 && !dx_pair) ? 0.f : 1.f, 0, ghx, st);
+      rc = linear_impl_ex(dG, 4 * H, 0, w_ih[d], I, 1, d_x, lddx, T * B, I, 4 * H, nullptr, nullptr, (d == 0 && !dx_pair) ? 0.f : 1.f, 0, ghx, dx_st);
       if (rc) return rc;
       if (dx_pair && (rc = fork.wait_mark())) return rc;
     }
@@ -665,6 +683,11 @@ extern "C" int dvae_lstm_seq_bwd(const float* x, int64_t ldx, int T, int B, int 
   return dvae::lstm_seq_bwd_impl(x, ldx, T, B, I, H, D, w_ih, w_hh, h0, c0, ld0, dir0, lengths, hs, ldhs, gates, cs,
                                  d_hs, lddhs, d_hn, d_cn, ldn, dirn, d_x, lddx, d_w_ih, d_w_hh, d_b_ih, d_b_hh,
                                  d_h0, d_c0, ldd0, dird0, state_ws, nullptr, (cudaStream_t)stream);
+}
+
+extern "C" int dvae_lstm_bwd_dx_stream(void* stream) {
+  dvae::g_dx_stream = (cudaStream_t)stream;
+  return DVAE_OK;
 }
 
 extern "C" int64_t dvae_lstm_bwd_planes_ws_floats(int T, int B, int I, int H, int D) {

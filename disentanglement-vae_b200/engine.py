@@ -107,7 +107,7 @@ class _Carry:
         self.g_z = g_z
         self.g_top = None             # d(loss)/d(decoder top-layer states): vocabulary backward -> decoder backward
         self.g_ctx = None             # d(loss)/d(encoder context): heads backward -> encoder backward
-        self.side_pending = False     # the decoder's embedding-gradient scatter still runs on the hoist side stream
+        self.side_pending = False     # the decoder's layer-0 d_x and embedding-gradient scatter still run on the hoist side stream
 
 
 class TrainEngine:
@@ -360,9 +360,6 @@ class TrainEngine:
         pl = self.plan
         check(self.lib.dvae_defer_joins(1), "dvae_defer_joins")
         c.g_ctx = pl.heads_bwd(self.model._P, self.G, pl.ctx, pl.eps, self.labels, self.kl_w, pl.g_hid, g_z=c.g_z)
-        if c.side_pending:          # the decoder's embedding-gradient scatter still reads g_dx[0]
-            torch.cuda.current_stream().wait_stream(self._side)
-            c.side_pending = False
         pl.encode_bwd(self.model._P, self.G, self.inputs, self.lengths, c.g_ctx,
                       emb_grad="encoder.embedding.weight" in self.model._layout, layers=layers)
 
@@ -383,7 +380,7 @@ class TrainEngine:
                     after_stage(k, c)
         finally:
             check(self.lib.dvae_join_side_streams(_lib.stream_ptr()), "dvae_join_side_streams")
-        if c.side_pending:          # the decoder's stage run on its own: its embedding-gradient scatter is joined too
+        if c.side_pending:          # the decoder's layer-0 d_x and embedding-gradient scatter are joined too
             torch.cuda.current_stream().wait_stream(self._side)
             c.side_pending = False
 

@@ -111,6 +111,7 @@ class StepPlan:
         w = max(d.E, d.H * d.D, d.Hd)
         self.g_top = torch.empty(T1, B, d.Hd, **f32)
         self.g_dx = [torch.empty(max(T, T1), B, w, **f32) for _ in range(2)]
+        self.g_dx_dec0 = torch.empty(T1, B, d.E, **f32)       # decoder layer 0's d_x, written on decode_bwd's aux_stream
         self.g_hid = torch.empty(B, d.H2L, **f32)
         self.g_ctx = torch.empty(B, d.C, **f32)
         self.heads_bwd_ws = torch.empty(self.lib.dvae_heads_bwd_ws_floats(B, d.Z, d.H2L), **f32)
@@ -336,9 +337,10 @@ class StepPlan:
         return self.g_top
 
     def decode_bwd(self, P, G, g_top, emb_grad=True, aux_stream=None):
-        """BPTT through the decoder stack; leaves d(hid) in self.g_hid.  With `aux_stream` the embedding-gradient
-        scatter (nothing downstream reads it before the optimizer) is enqueued there; the caller makes its stream wait
-        for `aux_stream` before anything overwrites g_dx[0] (encode_bwd) or reads the embedding gradient."""
+        """BPTT through the decoder stack; leaves d(hid) in self.g_hid.  With `aux_stream` layer 0's d_x GEMM (into its
+        own buffer) and the embedding-gradient scatter -- nothing downstream reads either before the optimizer -- are
+        enqueued there, beside the heads' and the encoder's backward; the caller makes its stream wait for `aux_stream`
+        before anything reads the embedding gradient."""
         self._alloc_bwd()
         lib, d, st = self.lib, self.d, _lib.stream_ptr()
         B, T1 = self.B, self.T1
@@ -347,26 +349,32 @@ class StepPlan:
         for l in range(d.Ld - 1, -1, -1):
             I = d.E if l == 0 else d.Hd
             x = self.x_dec if l == 0 else (self.d_xin[l] if p > 0.0 else self.d_hs[l - 1])
-            g_out = self.g_dx[l % 2]
+            dx_aside = l == 0 and aux_stream is not None
+            g_out = self.g_dx_dec0 if dx_aside else self.g_dx[l % 2]
             w_ih, w_hh, _, _ = self._dec_w(P, l)
             gw_ih, gw_hh, gb_ih, gb_hh = self._dec_w(G, l)
             need_dx = l > 0 or emb_grad
-            check(lib.dvae_lstm_seq_bwd_ex(ptr(x), I, T1, B, I, d.Hd, 1, ptr_array(w_ih), ptr_array(w_hh),
-                                        hid.data_ptr() + 4 * l * d.Hd, hid.data_ptr() + 4 * (d.Ld + l) * d.Hd,
-                                        d.H2L, 0, None, ptr(self.d_hs[l]), d.Hd, ptr(self.d_gates[l]),
-                                        ptr(self.d_cs[l]), ptr(g_in), d.Hd, None, None, 0, 0,
-                                        ptr(g_out) if need_dx else None, I, ptr_array(gw_ih), ptr_array(gw_hh),
-                                        ptr_array(gb_ih), ptr_array(gb_hh), self.g_hid.data_ptr() + 4 * l * d.Hd,
-                                        self.g_hid.data_ptr() + 4 * (d.Ld + l) * d.Hd, d.H2L, 0,
-                                        ptr(self.state_ws), ptr(self.lstm_bwd_planes), st), "dvae_lstm_seq_bwd(dec)")
+            if dx_aside:
+                check(lib.dvae_lstm_bwd_dx_stream(aux_stream.cuda_stream), "dvae_lstm_bwd_dx_stream")
+            try:
+                check(lib.dvae_lstm_seq_bwd_ex(ptr(x), I, T1, B, I, d.Hd, 1, ptr_array(w_ih), ptr_array(w_hh),
+                                            hid.data_ptr() + 4 * l * d.Hd, hid.data_ptr() + 4 * (d.Ld + l) * d.Hd,
+                                            d.H2L, 0, None, ptr(self.d_hs[l]), d.Hd, ptr(self.d_gates[l]),
+                                            ptr(self.d_cs[l]), ptr(g_in), d.Hd, None, None, 0, 0,
+                                            ptr(g_out) if need_dx else None, I, ptr_array(gw_ih), ptr_array(gw_hh),
+                                            ptr_array(gb_ih), ptr_array(gb_hh), self.g_hid.data_ptr() + 4 * l * d.Hd,
+                                            self.g_hid.data_ptr() + 4 * (d.Ld + l) * d.Hd, d.H2L, 0,
+                                            ptr(self.state_ws), ptr(self.lstm_bwd_planes), st), "dvae_lstm_seq_bwd(dec)")
+            finally:
+                if dx_aside:
+                    check(lib.dvae_lstm_bwd_dx_stream(None), "dvae_lstm_bwd_dx_stream")
             if l > 0 and p > 0.0:
                 check(lib.dvae_dropout(ptr(g_out), I, T1 * B, I, p, ptr(self.seed_dev), SALT_DEC_LAYER + l,
                                        ptr(g_out), I, 0, st), "dvae_dropout(bwd)")
             g_in = g_out
         if emb_grad:
             tok = self._dec_tokens
-            if aux_stream is not None:
-                aux_stream.wait_stream(torch.cuda.current_stream())
+            if aux_stream is not None:      # behind layer 0's d_x GEMM, which the library ordered after the recurrence
                 st = aux_stream.cuda_stream
             check(lib.dvae_embedding_bwd(ptr(g_in), d.E, ptr(tok), tok.stride(0), tok.stride(1), T1, B, p,
                                          ptr(self.seed_dev), SALT_DEC_EMB, self._dec_first, 0,

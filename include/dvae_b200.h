@@ -264,6 +264,10 @@ int dvae_lstm_seq_bwd(const float* x, int64_t ldx, int T, int B, int I, int H, i
  * transposed.  With the workspace x, dG and hs are transposed once into fp16 operand planes (one launch; dG scaled by the
  * max |dG| the recurrence kernel measured) and those GEMMs are bulk-copy fed on both operands. */
 int64_t dvae_lstm_bwd_planes_ws_floats(int T, int B, int I, int H, int D);
+/* Per host thread: the d_x GEMM of the following unidirectional (D = 1) dvae_lstm_seq_bwd / _ex calls runs on `stream`,
+ * ordered after the call's recurrence, as background work beside what the caller's stream does next (NULL: the call's own
+ * stream, the default).  The caller orders its reads of d_x after `stream`.  Scheduling only: d_x is the same. */
+int dvae_lstm_bwd_dx_stream(void* stream);
 int dvae_lstm_seq_bwd_ex(const float* x, int64_t ldx, int T, int B, int I, int H, int D,
                          const float* const* w_ih_host, const float* const* w_hh_host,
                          const float* h0, const float* c0, int64_t ld0, int64_t dir0,
